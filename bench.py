@@ -12,13 +12,14 @@ configs[4] the 3-variable stress model, N = 1), ``eager_gpu_baseline`` (the refe
     python bench.py --impl reference --ref-device cuda [--ref-batch 16] [--ref-autocast]     # optional extra: the same algorithm run
                                                              # op by op by eager PyTorch on cuda:0 (never the default arm)
     python bench.py --workload train [--profile-ops]         # configs[2]: the training step
+    python bench.py --gpus N --steps K --warmup W --dump-outputs DIR   # also writes DIR/x.npy, the image after the last timed step
 
 A "step" is ONE reverse (p_sample) step of the loop over the whole local batch: level-projection select, FD gate,
 stem assembly, the UNet (~270 kernel launches, replayed as one CUDA graph), the fused sampler update.  Every one of the
 1000 steps of a chain is the same work, so
     value = samples/s = global_batch / (T * seconds_per_step + once-per-batch precompute seconds),  T = 1000,
-with K timed steps (K = 1000 times the whole chain).  The activations of one step (GBs at batch 64) far exceed the
-126 MB L2, so no L2 flush is needed between timed steps.
+with K timed steps (K = 1000 times the whole chain; past the end of the chain its step counter restarts).  The activations
+of one step (GBs at batch 64) far exceed the 126 MB L2, so no L2 flush is needed between timed steps.
 """
 import argparse
 import json
@@ -203,7 +204,7 @@ def cpu_reference_steps(n_steps, warmup, seed=0):
             dt = time.perf_counter() - t0
             if i >= warmup:
                 times.append(dt)
-            t -= 1
+            t = (t - 1) % T_FULL                      # past the end of the chain, restart it
     return times, cores
 
 
@@ -245,7 +246,7 @@ def gpu_eager_reference_steps(n_steps, warmup, batch, autocast, seed=0):
             torch.cuda.synchronize()
             if i >= warmup:
                 times.append(e0.elapsed_time(e1) * 1e-3)
-            t -= 1
+            t = (t - 1) % T_FULL                      # past the end of the chain, restart it
     return times
 
 
@@ -374,7 +375,7 @@ def _time_loop(ctx, diff, plan, set_condition, shape, K, warmup, sample_clocks=F
         loop.step()
     loop.capture()
     loop.replay()                                   # one graph warm-up replay
-    K = min(K, T_FULL - warmup - 2)
+    left = T_FULL - 2 - max(0, warmup - 1)          # steps left in the chain after the warm-up steps and replay
     sampler = ClockSampler(ctx.local) if sample_clocks else None
     ctx.barrier()
     if sampler:
@@ -382,12 +383,45 @@ def _time_loop(ctx, diff, plan, set_condition, shape, K, warmup, sample_clocks=F
     e0, e1 = ev(), ev()
     e0.record()
     for _ in range(K):
+        if left == 0:                               # chain finished: restart its step counter on the current x, same work per step
+            loop.reset_counter()
+            left = T_FULL
         loop.replay()
+        left -= 1
     e1.record()
     ctx.barrier()
+    if left < 2:                                    # the roofline pass and --profile-ops step the loop twice more: keep t >= 0
+        loop.reset_counter()
     clocks = sampler.stop() if sampler else None
     ms_total, pre = ctx.max_over_ranks(e0.elapsed_time(e1), pre_ms)
     return dict(ms_per_step=ms_total / K, pre_ms=pre, launches_per_step=launches_per_step, clocks=clocks, loop=loop, K=K)
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def _dump_outputs(ctx, out_dir, arrays):
+    """--dump-outputs: each (B, ...) array, the shards of all ranks concatenated in rank order, is written by rank 0 as
+    <out_dir>/<name>.npy in float32.  Above DUMP_LIMIT_BYTES in all, a fixed seeded subset of the batch rows is kept (sorted)."""
+    import numpy as np
+    torch = ctx.torch
+    full = {}
+    for name, t in arrays.items():
+        t = t.detach().float().contiguous()
+        if ctx.world > 1:
+            parts = [torch.empty_like(t) for _ in range(ctx.world)]
+            ctx.dist.all_gather(parts, t)
+            t = torch.cat(parts)
+        full[name] = t.cpu().numpy()
+    if ctx.rank != 0:
+        return
+    total = sum(a.nbytes for a in full.values())
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in full.items():
+        if total > DUMP_LIMIT_BYTES:
+            keep = max(1, int(a.shape[0] * DUMP_LIMIT_BYTES // total))
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], keep, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def _synthetic_sr(ctx, B, c=1, lr_hw=(32, 64), scale=4, pinned=True):
@@ -481,6 +515,9 @@ def measure_sampling(ctx, net, diff, B, args, full):
     cond = sr_host.to(ctx.dev, non_blocking=True)
     torch.cuda.synchronize(ctx.dev)
     r = _time_loop(ctx, diff, plan, lambda: plan.set_condition(cond), tuple(cond.shape), args.steps, args.warmup, sample_clocks=full)
+    if full and args.dump_outputs:
+        # the image of the reverse loop after the last timed step, before the roofline pass steps it again
+        _dump_outputs(ctx, args.dump_outputs, {"x": r["loop"].x})
     ms, pre = r["ms_per_step"], r["pre_ms"]
     rec = {"batch_per_gpu": B, "global_batch": B * ctx.world, "ms_per_step": ms, "precompute_ms_per_batch": pre,
            "value": B * ctx.world / (T_FULL * ms * 1e-3 + pre * 1e-3), "unit": "samples/s", "steps": r["K"],
@@ -773,7 +810,17 @@ def main():
     ap.add_argument("--workload", default="sample", choices=["sample", "train"], help="sample = headline metric; train = configs[2]")
     ap.add_argument("--train-batch", type=int, default=4)
     ap.add_argument("--train-precision", default="bf16", choices=["bf16", "fp32"])
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="sampling workload of --impl ours only: after the timed steps of the headline record, write the reverse loop's "
+                         "image after its last timed step (all ranks' shards, float32) as DIR/x.npy; the inputs depend only on the "
+                         "arguments, so two builds can be compared")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.impl == "ours" and args.workload == "sample" and args.warmup > T_FULL - 1:
+        ap.error("--warmup must leave the warm-up steps inside the %d-step chain" % T_FULL)
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "sample"):
+        ap.error("--dump-outputs applies to the sampling workload of --impl ours")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     if args.impl == "reference":

@@ -28,6 +28,21 @@ def fields(tag, batch, c_img, height, width, seed, scale=4):
     return lr, sr, hr
 
 
+def grad_inputs(name, g):
+    """The fixture ``g`` of training-step case ``name`` with its inputs (lr, sr, hr, noise) in place.  A case marked
+    ``regenerate_inputs`` stores only their heads: the fields are regenerated from the seed as make_golden.run_grad_case drew
+    them, and the heads pin the generator streams."""
+    spec = CASES[name]
+    if not spec.get("regenerate_inputs"):
+        return g
+    cfg, seed = spec["cfg"], spec["seed"]
+    lr, sr, hr = fields(name, spec["batch"], cfg["image_channels"], cfg["image_height"], cfg["image_width"], seed)
+    out = dict(g, lr=lr, sr=sr, hr=hr, noise=seeded_randn(name + ".noise", sr.shape, seed))
+    for k in ("lr", "sr", "hr", "noise"):
+        assert torch.equal(out[k][:, :, :2, :8], g[k + "_head"]), k
+    return out
+
+
 def short_schedule(T):
     return {"schedule": "linear", "n_timestep": T, "linear_start": 1e-6, "linear_end": 1e-2}
 
@@ -50,8 +65,9 @@ CASES = {
     "resdiff_loss_small": dict(kind="resdiff_loss", cfg=unet_cfg(32, 64, attn_res=(4,)), batch=2, seed=31, t=400),
     # one training step: loss / numel -> backward (model.py:61-69); fixture = per-parameter gradient summaries
     "resdiff_grad_small": dict(kind="resdiff_grad", cfg=unet_cfg(32, 64, attn_res=(4,)), batch=2, seed=61, t=400),
-    # the BASELINE configs[2] training step itself: Cfg-A UNet at 128x256, batch 4 (HF_guided_CA at level 0 over 8192 keys)
-    "resdiff_grad_full_b4": dict(kind="resdiff_grad", cfg=unet_cfg(128, 256), batch=4, seed=66, t=400),
+    # the BASELINE configs[2] training step itself: Cfg-A UNet at 128x256, batch 4 (HF_guided_CA at level 0 over 8192 keys); its
+    # inputs are regenerated from the seed (grad_inputs), the fixture keeps only their heads
+    "resdiff_grad_full_b4": dict(kind="resdiff_grad", cfg=unet_cfg(128, 256), batch=4, seed=66, t=400, regenerate_inputs=True),
     "phydiff_grad_small": dict(kind="phydiff_grad", cfg=unet_cfg(32, 64, attn_res=(4,)), batch=2, seed=62, t=350),
     "sr3_grad_small": dict(kind="sr3_grad", cfg=unet_cfg(32, 64, attn_res=(4,), in_channel=2), batch=2, seed=63, t=500),
     "srdiff_chain_small": dict(kind="srdiff_chain", cfg=unet_cfg(32, 64, attn_res=(4,), in_channel=1), batch=2, seed=63, T=4),

@@ -100,7 +100,12 @@ def run_grad_case(ref, name, spec):
         np.random.randint, np.random.uniform = _ri, _un
     l_pix = loss.sum() / int(hr.numel())
     l_pix.backward()
-    out = dict(hr=hr, sr=sr, lr=lr, noise=noise, level=torch.FloatTensor(u), loss=loss.detach().reshape(1), wsum=_checksum(net))
+    out = dict(level=torch.FloatTensor(u), loss=loss.detach().reshape(1), wsum=_checksum(net))
+    inputs = dict(hr=hr, sr=sr, lr=lr, noise=noise)
+    if spec.get("regenerate_inputs"):
+        # 128x256 fields: the tests regenerate them from the seed (cases.grad_inputs); the heads detect RNG drift
+        inputs = {k + "_head": v[:, :, :2, :8].clone() for k, v in inputs.items()}
+    out.update(inputs)
     named = [(n, p.grad) for n, p in net.named_parameters() if p.grad is not None]
     if spec.get("joint"):
         named += [("rrdb_encoder." + n, p.grad) for n, p in diff.rrdb_encoder.named_parameters() if p.grad is not None]

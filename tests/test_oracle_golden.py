@@ -143,8 +143,8 @@ def test_phy_stencils_known_answer():
 def test_resdiff_param_grads_match_reference(name):
     """Oracle autograd vs the gradient summaries of the real reference's training step (model.py:61-68); the second case is the
     BASELINE configs[2] shape itself (Cfg-A at 128x256, batch 4)."""
-    from oracle.cases import grad_summary
-    g, spec = load_golden(name), CASES[name]
+    from oracle.cases import grad_inputs, grad_summary
+    g, spec = grad_inputs(name, load_golden(name)), CASES[name]
     sd = _sd("resdiff", spec["seed"], spec["cfg"])
     np.testing.assert_allclose(_wsum(sd), g["wsum"].numpy(), rtol=1e-9)
     loss, grads = process.resdiff_param_grads(sd, spec["cfg"], g["hr"], g["sr"], g["level"], g["noise"])

@@ -446,8 +446,8 @@ def test_training_step_at_benchmark_shape_vs_reference(precision):
     tile choices of the backward kernels (row-tile shapes, split of the weight-gradient K loop, images per tile) depend on the batch and
     the resolution, so the 32x64 fixtures do not cover what bench.py --workload train launches.  Tolerances: fp32 check mode 2e-4 per
     tensor, bf16 1.6e-1 per tensor and 1e-1 on the projected whole-gradient error."""
-    from oracle.cases import grad_summary
-    g, spec = load_golden("resdiff_grad_full_b4"), CASES["resdiff_grad_full_b4"]
+    from oracle.cases import grad_inputs, grad_summary
+    g, spec = grad_inputs("resdiff_grad_full_b4", load_golden("resdiff_grad_full_b4")), CASES["resdiff_grad_full_b4"]
     cfg = spec["cfg"]
     net, diff = _build(cfg, spec["seed"], precision, "resdiff")
     loss = _train_backward(diff, g, spec)
