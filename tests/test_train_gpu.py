@@ -163,7 +163,8 @@ def test_conv_wgrad_tc_vs_simt(case):
 
 
 @pytest.mark.parametrize("a_mn,b_mn", [(False, True), (True, False), (True, True)])
-@pytest.mark.parametrize("M,N,K,batch", [(128, 128, 64, 2), (256, 64, 128, 3), (64, 192, 256, 1), (512, 512, 64, 2)])
+@pytest.mark.parametrize("M,N,K,batch", [(128, 128, 64, 2), (256, 64, 128, 3), (64, 192, 256, 1), (512, 512, 64, 2),
+                                     (64, 128, 8192, 2)])
 def test_gemm_tc_transposed_operands(a_mn, b_mn, M, N, K, batch):
     """Attention backward needs A^T / B^T operands: the tcgen05 GEMM consumes MN-major (transposed) operands directly."""
     dev = _dev()
