@@ -85,9 +85,6 @@ typedef struct {
    * pixels): [kx][3 * 64 rows][Cin], row block b of slice kx = the 64 (zero-padded) output channels of tap (ky = 2 - b, kx),
    * dtype = x_dtype (wsr_pack_conv_weight_vmerge).  NULL = not available. */
   const void* w_vmerge;
-  /* reserved (round 1 exchanged split-K partial tiles through this caller-owned buffer; the split-K kernels now form a thread-block
-   * cluster per tile and exchange the partials through distributed shared memory, so nothing is read or written here).  Pass NULL / 0. */
-  void* splitk_ws; long long splitk_ws_bytes;
 } WsrConvDesc;
 
 /* fp32-accumulate SIMT implicit GEMM; any dtype, any channel count.  This is the "fp32 check mode" kernel. */
@@ -96,21 +93,17 @@ int wsr_conv_simt(const WsrConvDesc* d, void* stream);
  * Cin2 % 64 == 0, Cout % 16 == 0, W a power of two (>= 2), pitches % 8 == 0, 16-byte aligned bases. */
 int wsr_conv_tc(const WsrConvDesc* d, void* stream);
 int wsr_conv_tc_can_fuse_gn(const WsrConvDesc* d);
-/* test introspection: (CTA pairs << 20) | (column-tile width << 8) | K splits chosen by the most recent wsr_conv_tc / wsr_conv_taps_tc call */
+/* test introspection: (CTA pairs << 20) | (column-tile width << 8) | K splits chosen by the most recent wsr_conv_tc / wsr_conv_taps_tc call.
+ * Classic-mode launches whose 3x3 K loop is long (>= 36 K blocks) and whose 64-column tiles fill at most half of the SMs are split
+ * over a 2-CTA cluster (each CTA accumulates half of the K blocks; partial tiles are exchanged through distributed shared memory). */
 int wsr_debug_last_tc_config(void);
-/* split-K of the classic-mode tcgen05 convolution (a cluster of 2 / 4 / 8 CTAs per tile, each accumulating a range of the K blocks; partial
- * tiles exchanged through distributed shared memory): mode 0 = never, 1 = the one measured-faster cut (default: 2-CTA clusters for 3x3
- * convolutions whose tiles fill at most half of the SMs; env WSR_SPLITK), 2 = cost-model search over (column tile, 2 / 4 / 8 splits), measured
- * slower for the whole step on B200 (DESIGN.md 8) and kept for the kernel tests.  Returns the previous mode. */
-int wsr_debug_set_splitk(int on);
 /* CTA pairs (tcgen05 cta_group::2: two SMs of a TPC share one 256 x 256 tile, each staging half of the weight columns) for the classic-mode
- * 256-column convolution tiles: 0 = never, 1 = launches of more than one wave (default; env WSR_PAIR), 2 = every eligible launch (an even
- * number of row tiles).  Returns the previous mode.  wsr_debug_last_tc_config() reports the choice in bit 20. */
+ * 256-column convolution tiles: 0 = never, 1 = launches of more than one wave (default), 2 = every eligible launch (an even number of row
+ * tiles).  Returns the previous mode.  wsr_debug_last_tc_config() reports the choice in bit 20. */
 int wsr_debug_set_pair(int mode);
 /* Programmatic dependent launch for the kernels launched after this call (convolutions, GroupNorm apply, small attention, head): a kernel
- * may start its prologue while its predecessor drains.  Off by default (no gain at 64 images per GPU, where the device runs under its power
- * cap; env WSR_PDL=1 switches it on); the sampling loop switches it on around the graph capture of small batches.  Returns the previous
- * setting (-1 = undecided). */
+ * may start its prologue while its predecessor drains.  Off until wsr_set_pdl(1) (no gain at 64 images per GPU, where the device runs under
+ * its power cap); the sampling loop switches it on around the graph capture of small batches.  Returns the previous setting (0 or 1). */
 int wsr_set_pdl(int on);
 
 /* ---------------------------------------------------------------------------------------------------------------

@@ -46,7 +46,6 @@ class ConvDesc(C.Structure):
         ("gn_stats", C.c_void_p), ("gn_stats_ld", C.c_int),
         ("gn_table", C.c_void_p), ("gn_table_ld", C.c_int), ("gn_act", C.c_int),
         ("w_vmerge", C.c_void_p),
-        ("splitk_ws", C.c_void_p), ("splitk_ws_bytes", C.c_int64),
     ]
 
 
@@ -97,7 +96,6 @@ SIGNATURES = {
     "wsr_conv_tc": [C.POINTER(ConvDesc), _P],
     "wsr_conv_tc_can_fuse_gn": [C.POINTER(ConvDesc)],
     "wsr_debug_last_tc_config": [],
-    "wsr_debug_set_splitk": [_I],
     "wsr_debug_set_pair": [_I],
     "wsr_set_pdl": [_I],
     "wsr_gn_finalize": [_P, _I, _I, _I, _I, _I, _F, _P, _P, _P, _I, _P],
@@ -167,7 +165,7 @@ SIGNATURES = {
 }
 _RESTYPE = {"wsr_fd_precompute_workspace_bytes": C.c_int64, "wsr_fd_backward_workspace_bytes": C.c_int64}
 # functions whose return value is data, not a status
-_NO_STATUS = {"wsr_version", "wsr_device_is_sm100", "wsr_conv_tc_can_fuse_gn", "wsr_debug_last_tc_config", "wsr_debug_set_splitk", "wsr_debug_set_pair", "wsr_set_pdl", "wsr_attention_small_tc_supported", "wsr_head_sampler_supported", "wsr_fd_precompute_workspace_bytes", "wsr_fd_backward_workspace_bytes"}
+_NO_STATUS = {"wsr_version", "wsr_device_is_sm100", "wsr_conv_tc_can_fuse_gn", "wsr_debug_last_tc_config", "wsr_debug_set_pair", "wsr_set_pdl", "wsr_attention_small_tc_supported", "wsr_head_sampler_supported", "wsr_fd_precompute_workspace_bytes", "wsr_fd_backward_workspace_bytes"}
 
 _lib = None
 launches = 0          # number of status-returning calls made (bench.py's gpu_launches bookkeeping is done there)

@@ -11,13 +11,13 @@ void set_error(const char* fmt, ...) {
   vsnprintf(g_err, sizeof(g_err), fmt, ap);
   va_end(ap);
 }
-int g_pdl_mode = -1;
+int g_pdl_mode = 0;
 }  // namespace wsr
 
 extern "C" const char* wsr_last_error(void) { return wsr::g_err; }
 extern "C" int wsr_version(void) { return 100; }
 
-// programmatic dependent launch on / off for the launches that follow (common.cuh); returns the previous setting (-1 = was undecided)
+// programmatic dependent launch on / off for the launches that follow (common.cuh); returns the previous setting
 extern "C" int wsr_set_pdl(int on) {
   const int prev = wsr::g_pdl_mode;
   wsr::g_pdl_mode = on ? 1 : 0;

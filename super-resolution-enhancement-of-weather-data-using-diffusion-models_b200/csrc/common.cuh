@@ -39,18 +39,15 @@ void set_error(const char* fmt, ...);
 // input-independent prologue, then block in pdl_wait() until the predecessor grid has completed and its memory is visible.
 // EVERY global-memory access that may depend on (or be overwritten under) earlier work must come after pdl_wait().
 // Measured on B200 (bench.py, CUDA-graph replay of the step, A/B on one box): 17.39 ms with the attribute vs 17.17 ms without -- the
-// graph already keeps launch gaps short and the device runs under its power cap -- so the attribute is OFF unless WSR_PDL=1 or
+// graph already keeps launch gaps short and the device runs under its power cap -- so the attribute is OFF unless
 // wsr_set_pdl(1) (pdl_wait() is then a no-op).
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 
-// process-wide switch (common.cu): -1 = not decided yet -> WSR_PDL, default off; wsr_set_pdl() overrides (the sampling loop switches it on
+// process-wide switch (common.cu), off by default; wsr_set_pdl() sets it (the sampling loop switches it on
 // while it captures the step graph of a SMALL batch, where launch gaps are a visible share of the step: 3.39 -> 3.31 ms at 8 images)
 extern int g_pdl_mode;
-static inline bool pdl_enabled() {
-  if (g_pdl_mode < 0) g_pdl_mode = getenv("WSR_PDL") ? (atoi(getenv("WSR_PDL")) != 0 ? 1 : 0) : 0;
-  return g_pdl_mode != 0;
-}
+static inline bool pdl_enabled() { return g_pdl_mode != 0; }
 
 template <typename... KArgs, typename... Args>
 static inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args&&... args) {

@@ -228,23 +228,14 @@ template <typename TI, typename TO, int VEC, bool DROP>
 __global__ void gn_apply_kernel(const TI* __restrict__ x, int HW, int C, int ld, int CV, int PL, int chunk,
                                 const double* __restrict__ stats, int stats_ld, const float* __restrict__ gamma,
                                 const float* __restrict__ beta, int groups, float eps, int act, TO* __restrict__ y, int y_ld,
-                                float drop_p, uint64_t drop_seed, uint32_t drop_tag, int cpi, int nr, int nimg) {
+                                float drop_p, uint64_t drop_seed, uint32_t drop_tag) {
   extern __shared__ float sm[];   // scale[C], shift[C], then (mean, rstd) per group
-  // Block -> (image, pixel chunk).  nr == 0: natural order (blockIdx.x = image * cpi + chunk).  nr > 0: "range-reversed" order.  The
-  // producing convolution is a persistent kernel whose CTA r wrote the r-th of nr contiguous ranges of this tensor front to back, so
-  // when it ends the 126 MB L2 holds the TAIL of every range; walking every range back to front (pass k visits the k-th chunk from the
-  // end of all ranges) reads those tails while they are still cached, and leaves the HEADS of the ranges of the output in L2, which is
-  // where the consuming convolution's CTAs start.  In natural order a tensor larger than the cache streams through it with no hits.
-  int gc = blockIdx.x;
-  if (nr > 0) {
-    const long long T = (long long)cpi * nimg;
-    const int k = blockIdx.x / nr, r = blockIdx.x - k * nr;
-    const long long start = (long long)r * T / nr, end = (long long)(r + 1) * T / nr;
-    if (k >= end - start) return;
-    gc = (int)(end - 1 - k);
-  }
-  const int n = nr > 0 ? gc / cpi : blockIdx.y;
-  const int chunk_idx = nr > 0 ? gc - n * cpi : blockIdx.x;
+  // Block -> (image, pixel chunk) in natural order.  Walking the ranges the producing convolution's CTAs wrote back to front, to
+  // read their L2-resident tails first, MEASURED no faster on B200 (profiles/r02_gn_order_ab.txt): the 65 gn_apply launches of a B = 64
+  // step take 3.09 ms that way vs 3.03 ms in natural order, the whole step 16.64 vs 16.56 ms (3.53 vs 3.51 ms at B = 8) -- the
+  // write-back L2 does not keep the producer's tail lines resident the way an LRU read cache would.
+  const int n = blockIdx.y;
+  const int chunk_idx = blockIdx.x;
   const int cpg = C / groups;
   float* gm = sm + 2 * C;
   pdl_launch_dependents();        // programmatic dependent launch (common.cuh): the statistics come from the preceding convolution
@@ -713,27 +704,10 @@ static int gn_apply_impl(const void* x, int x_dtype, int N, int HW, int C, int x
     if (chunk < 4 * g.PL) chunk = 4 * g.PL;
     if (chunk < g.chunk) g.chunk = chunk;
   }
-  const int cpi = (HW + g.chunk - 1) / g.chunk;
-  dim3 grid(cpi, N);
-  // range-reversed block order (see the kernel).  MEASURED on B200 (A/B in one job, profiles/r02_gn_order_ab.txt): no effect -- the 65
-  // gn_apply launches of a B = 64 step take 3.09 ms reversed vs 3.03 ms in natural order, the whole step 16.64 vs 16.56 ms (3.53 vs 3.51
-  // ms at B = 8): the write-back L2 does not keep the producer's tail lines resident the way an LRU read cache would.  OFF unless
-  // WSR_GN_ORDER=1.
-  static const int order_on = getenv("WSR_GN_ORDER") ? atoi(getenv("WSR_GN_ORDER")) : 0;
-  int nr = 0;
-  if (order_on) {
-    int sms = 0, dev = 0;
-    cudaGetDevice(&dev);
-    static int cached_sms = 0;
-    if (!cached_sms) { cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev); cached_sms = sms > 0 ? sms : 148; }
-    nr = cached_sms;
-    const long long T = (long long)cpi * N;
-    const long long maxlen = (T + nr - 1) / nr;
-    grid = dim3((unsigned)(maxlen * nr), 1);
-  }
+  const dim3 grid((HW + g.chunk - 1) / g.chunk, N);
   size_t smem = ((size_t)C * 2 + 2 * groups) * sizeof(float);
   cudaStream_t st = (cudaStream_t)stream;
-#define GN_APPLY(T, V, D) WSR_CUDA_OK(launch_pdl(gn_apply_kernel<T, T, V, D>, grid, dim3(g.threads), smem, st, (const T*)x, HW, C, x_ld, g.CV, g.PL, g.chunk, stats, stats_ld, gamma, beta, groups, eps, act, (T*)y, y_ld, drop_p, drop_seed, drop_tag, cpi, nr, N))
+#define GN_APPLY(T, V, D) WSR_CUDA_OK(launch_pdl(gn_apply_kernel<T, T, V, D>, grid, dim3(g.threads), smem, st, (const T*)x, HW, C, x_ld, g.CV, g.PL, g.chunk, stats, stats_ld, gamma, beta, groups, eps, act, (T*)y, y_ld, drop_p, drop_seed, drop_tag))
   if (drop_p > 0.f) {
     if (x_dtype == WSR_BF16) { if (g.vec == 8) GN_APPLY(__nv_bfloat16, 8, true); else GN_APPLY(__nv_bfloat16, 1, true); }
     else { if (g.vec == 4) GN_APPLY(float, 4, true); else GN_APPLY(float, 1, true); }

@@ -62,8 +62,6 @@ struct TcParams {
   int a_mn, b_mn;               // operand is MN-major (contiguous along rows / columns, strided along K): loaded as
                                 // [64 MN][64 K] boxes 8 KB apart and consumed through the MN-major UMMA descriptor
   int a_blk, b_blk;             // number of such 64-wide boxes per tile
-  int dbg;                      // debugging switches (env WSR_TC_DBG): 1 skip epilogue work, 2 skip MMA issue, 4 skip stores only
-  int halo_bo;                  // debugging switch: put (start row & 7) into the descriptor base-offset field
   int halo_rows;                // halo mode: output rows per tile (1 or 2; 2 = two accumulators share every weight tile)
   int n_taps, halo_bytes;       // halo mode: e[0..n_taps) are filter taps served from one (t1+2) x 3 halo tile per chunk
   int M1, M2, M3;               // valid row extents (masking)
@@ -86,7 +84,6 @@ struct TcParams {
   // the partial tiles are exchanged through distributed shared memory: CTA s finishes the 32-column chunks ch with ch % ksplit == s and
   // receives the other CTAs' partials of those chunks in its (by then idle) operand ring.
   int ksplit, kb_split;
-  int prefetch;                 // halo mode: L2-prefetch the halo box two loads ahead (see the producer)
   int pair;                     // classic mode, N = 256: run as CTA pairs (PAIR kernels); the weight map's box is then 128 rows
   const void* xg; int xg_ld, xg_H, xg_W;
   const void* x2g; int x2g_ld;
@@ -318,7 +315,7 @@ __global__ void __launch_bounds__(FUSE ? kTcThreadsFused : kTcThreads, 1) gemm_t
                 mbar_expect_tx(&full_a[sa], (uint32_t)p.halo_bytes);
                 tma_load_4d(smem + sa * kHaloStage, &p.amap[p.e[0].amap], &full_a[sa], c * kBlockK, c1 - 1, c2 - 1, c3);
               }
-              if (p.prefetch) {
+              if constexpr (FUSE) {
                 // the box that will land in this stage the NEXT time round (two halo loads ahead) goes to L2 now: with the transform
                 // between load and MMA a stage is refilled only after load + transform + MMA of its previous content, so the refill
                 // latency is on the critical path and should be an L2 hit, not an HBM round trip
@@ -395,21 +392,17 @@ __global__ void __launch_bounds__(FUSE ? kTcThreadsFused : kTcThreads, 1) gemm_t
             const uint32_t a_lo = s_lo | a_lbo;
             const uint32_t b_lo = (s_lo + (uint32_t)(kABytes >> 4)) | b_lbo;
             if constexpr (PAIR) {
-              if (!(p.dbg & 2)) {
-                umma_bf16_lo_pair(d_tmem, a_lo, b_lo, idesc, kb != kb0 ? 1u : 0u);
-                umma_bf16_lo_pair(d_tmem, a_lo + 2u, b_lo + 2u, idesc, 1u);
-                umma_bf16_lo_pair(d_tmem, a_lo + 4u, b_lo + 4u, idesc, 1u);
-                umma_bf16_lo_pair(d_tmem, a_lo + 6u, b_lo + 6u, idesc, 1u);
-              }
+              umma_bf16_lo_pair(d_tmem, a_lo, b_lo, idesc, kb != kb0 ? 1u : 0u);
+              umma_bf16_lo_pair(d_tmem, a_lo + 2u, b_lo + 2u, idesc, 1u);
+              umma_bf16_lo_pair(d_tmem, a_lo + 4u, b_lo + 4u, idesc, 1u);
+              umma_bf16_lo_pair(d_tmem, a_lo + 6u, b_lo + 6u, idesc, 1u);
               umma_commit_pair(&empty_a[sa]);                           // frees the stage in both CTAs
               if (kb == kb1 - 1) umma_commit_pair(&tfull_bar[acc]);     // both epilogues
             } else {
-            if (!(p.dbg & 2)) {
-              umma_bf16_lo(d_tmem, a_lo, b_lo, idesc, kb != kb0 ? 1u : 0u);
-              umma_bf16_lo(d_tmem, a_lo + a_st, b_lo + b_st, idesc, 1u);
-              umma_bf16_lo(d_tmem, a_lo + 2 * a_st, b_lo + 2 * b_st, idesc, 1u);
-              umma_bf16_lo(d_tmem, a_lo + 3 * a_st, b_lo + 3 * b_st, idesc, 1u);
-            }
+            umma_bf16_lo(d_tmem, a_lo, b_lo, idesc, kb != kb0 ? 1u : 0u);
+            umma_bf16_lo(d_tmem, a_lo + a_st, b_lo + b_st, idesc, 1u);
+            umma_bf16_lo(d_tmem, a_lo + 2 * a_st, b_lo + 2 * b_st, idesc, 1u);
+            umma_bf16_lo(d_tmem, a_lo + 3 * a_st, b_lo + 3 * b_st, idesc, 1u);
             umma_commit(&empty_a[sa]);
             if (kb == kb1 - 1) umma_commit(&tfull_bar[acc]);
             }
@@ -440,35 +433,33 @@ __global__ void __launch_bounds__(FUSE ? kTcThreadsFused : kTcThreads, 1) gemm_t
                 tc_fence_after();
                 const uint32_t v_lo = a_lo0 + (uint32_t)dxi * 8u;                 // halo column offset dx + 1 = dxi
                 const uint32_t b_lo = desc_lo(smem_u32(smem_b + sb * Cfg::kBBytes));
-                if (!(p.dbg & 2)) {
 #pragma unroll
-                  for (int k = 0; k < kBlockK / 16; ++k) {
-                    if (kb == 0 && k == 0) {
-                      // very first K step of the tile: every accumulator block starts from zero, which a merged MMA cannot
-                      // express (one accumulate flag per instruction) -> nine plain N = 64 MMAs, first touch overwrites
-                      // (issued in halo-row order so that the fused-GroupNorm kernels can start as soon as row 0 is transformed; output
-                      // row rr is still first touched by its dy = -1 tap, halo row rr)
+                for (int k = 0; k < kBlockK / 16; ++k) {
+                  if (kb == 0 && k == 0) {
+                    // very first K step of the tile: every accumulator block starts from zero, which a merged MMA cannot
+                    // express (one accumulate flag per instruction) -> nine plain N = 64 MMAs, first touch overwrites
+                    // (issued in halo-row order so that the fused-GroupNorm kernels can start as soon as row 0 is transformed; output
+                    // row rr is still first touched by its dy = -1 tap, halo row rr)
 #pragma unroll
-                      for (int hr = 0; hr < ROWS + 2; ++hr) {
-                        need_rows(hr + 1);
+                    for (int hr = 0; hr < ROWS + 2; ++hr) {
+                      need_rows(hr + 1);
 #pragma unroll
-                        for (int dyi = 0; dyi < 3; ++dyi) {      // dy = dyi - 1 reads halo row rr + dyi; weights block 2 - dyi
-                          const int rr = hr - dyi;
-                          if (rr >= 0 && rr < ROWS)
-                            umma_bf16_lo(d_tmem + (uint32_t)(rr * 64), v_lo + (uint32_t)hr * pitch8, b_lo + (uint32_t)(2 - dyi) * 512u,
-                                         kIdBase | (8u << 17), dyi != 0 ? 1u : 0u);
-                        }
+                      for (int dyi = 0; dyi < 3; ++dyi) {      // dy = dyi - 1 reads halo row rr + dyi; weights block 2 - dyi
+                        const int rr = hr - dyi;
+                        if (rr >= 0 && rr < ROWS)
+                          umma_bf16_lo(d_tmem + (uint32_t)(rr * 64), v_lo + (uint32_t)hr * pitch8, b_lo + (uint32_t)(2 - dyi) * 512u,
+                                       kIdBase | (8u << 17), dyi != 0 ? 1u : 0u);
                       }
-                    } else {
+                    }
+                  } else {
 #pragma unroll
-                      for (int hr = 0; hr < ROWS + 2; ++hr) {
-                        need_rows(hr + 1);
-                        // halo row hr feeds output rows hr-2 (dy=+1, block 0), hr-1 (dy=0, block 1), hr (dy=-1, block 2)
-                        const int r_lo = hr - 2 < 0 ? 0 : hr - 2, r_hi = hr < ROWS - 1 ? hr : ROWS - 1;
-                        const int nblk = r_hi - r_lo + 1, blk0 = r_lo - (hr - 2);
-                        umma_bf16_lo(d_tmem + (uint32_t)(r_lo * 64), v_lo + (uint32_t)hr * pitch8 + (uint32_t)(2 * k),
-                                     b_lo + (uint32_t)blk0 * 512u + (uint32_t)(2 * k), kIdBase | ((uint32_t)(nblk * 8) << 17), 1u);
-                      }
+                    for (int hr = 0; hr < ROWS + 2; ++hr) {
+                      need_rows(hr + 1);
+                      // halo row hr feeds output rows hr-2 (dy=+1, block 0), hr-1 (dy=0, block 1), hr (dy=-1, block 2)
+                      const int r_lo = hr - 2 < 0 ? 0 : hr - 2, r_hi = hr < ROWS - 1 ? hr : ROWS - 1;
+                      const int nblk = r_hi - r_lo + 1, blk0 = r_lo - (hr - 2);
+                      umma_bf16_lo(d_tmem + (uint32_t)(r_lo * 64), v_lo + (uint32_t)hr * pitch8 + (uint32_t)(2 * k),
+                                   b_lo + (uint32_t)blk0 * 512u + (uint32_t)(2 * k), kIdBase | ((uint32_t)(nblk * 8) << 17), 1u);
                     }
                   }
                 }
@@ -486,15 +477,13 @@ __global__ void __launch_bounds__(FUSE ? kTcThreadsFused : kTcThreads, 1) gemm_t
               const uint32_t t_lo = a_lo0 + (uint32_t)((e.d2 + 1) * pitch + (e.d1 + 1)) * 8u;    // 128-byte rows = 8 address units
               const uint32_t b_lo = desc_lo(smem_u32(smem_b + sb * Cfg::kBBytes));
               need_rows(e.d2 + 1 + ROWS);                  // this tap reads halo rows dy + 1 .. dy + ROWS
-              if (!(p.dbg & 2)) {
-                // k outer, row inner: consecutive MMAs accumulate into different TMEM tiles
+              // k outer, row inner: consecutive MMAs accumulate into different TMEM tiles
 #pragma unroll
-                for (int k = 0; k < kBlockK / 16; ++k) {
+              for (int k = 0; k < kBlockK / 16; ++k) {
 #pragma unroll
-                  for (int rr = 0; rr < ROWS; ++rr)       // output row rr of the tile reads halo rows rr .. rr+2
-                    umma_bf16_lo(d_tmem + (uint32_t)(rr * BLOCK_N), t_lo + (uint32_t)rr * pitch8 + (uint32_t)(2 * k), b_lo + (uint32_t)(2 * k),
-                                 Cfg::kIdesc, k != 0 ? 1u : (kb != 0 ? 1u : 0u));
-                }
+                for (int rr = 0; rr < ROWS; ++rr)       // output row rr of the tile reads halo rows rr .. rr+2
+                  umma_bf16_lo(d_tmem + (uint32_t)(rr * BLOCK_N), t_lo + (uint32_t)rr * pitch8 + (uint32_t)(2 * k), b_lo + (uint32_t)(2 * k),
+                               Cfg::kIdesc, k != 0 ? 1u : (kb != 0 ? 1u : 0u));
               }
               umma_commit(&empty_b[sb]);
               if (++sb == kRingB) { sb = 0; pb ^= 1; }
@@ -772,10 +761,8 @@ __global__ void __launch_bounds__(FUSE ? kTcThreadsFused : kTcThreads, 1) gemm_t
           const uint32_t src_idx = (uint32_t)split_s < owner ? (uint32_t)split_s : (uint32_t)split_s - 1u;
           const uint32_t slot = ((uint32_t)(ch / (int)S) * (S - 1u) + src_idx) * (uint32_t)(kBlockM * 128) + (uint32_t)row * 128u;
           const uint32_t dst = dsmem_addr(ring + slot, owner);
-          if (!(p.dbg & 16)) {
 #pragma unroll
-            for (int q = 0; q < 8; ++q) dsmem_st4(dst + (uint32_t)((q ^ (row & 7)) << 4), v[4 * q], v[4 * q + 1], v[4 * q + 2], v[4 * q + 3]);
-          }
+          for (int q = 0; q < 8; ++q) dsmem_st4(dst + (uint32_t)((q ^ (row & 7)) << 4), v[4 * q], v[4 * q + 1], v[4 * q + 2], v[4 * q + 3]);
         }
         fence_acq_rel_cluster();
         __syncwarp();
@@ -796,7 +783,7 @@ __global__ void __launch_bounds__(FUSE ? kTcThreadsFused : kTcThreads, 1) gemm_t
       const long long qbase = o1 * p.q_s1 + o2 * p.q_s2 + (long long)r3 * p.q_s3 + (long long)zb * p.q_sb;
       const float* rowvec = p.rowvec ? p.rowvec + (long long)r3 * p.rowvec_ld : nullptr;
 #pragma unroll 1
-      for (int ci = 0; ci < ((p.dbg & 1) ? 0 : kChunksPerWarp); ++ci) {
+      for (int ci = 0; ci < kChunksPerWarp; ++ci) {
         const int ch = ch_begin + ci;
         if constexpr (SPLIT) { if (ch % p.ksplit != split_s) continue; }
         uint32_t v[32];
@@ -804,7 +791,7 @@ __global__ void __launch_bounds__(FUSE ? kTcThreadsFused : kTcThreads, 1) gemm_t
         if constexpr (SPLIT) {
           // phase B: this CTA owns the chunk -- add the other CTAs' partials out of the ring
           const int S = p.ksplit;
-          for (int si = 0; si < ((p.dbg & 32) ? 0 : S - 1); ++si) {
+          for (int si = 0; si < S - 1; ++si) {
             const uint8_t* src = smem + ((size_t)((ch / S) * (S - 1) + si) * kBlockM + row) * 128;
 #pragma unroll
             for (int q = 0; q < 8; ++q) {
@@ -928,7 +915,7 @@ __global__ void __launch_bounds__(FUSE ? kTcThreadsFused : kTcThreads, 1) gemm_t
               }
               const int r16 = 8 * j + sr;
               const uint4 u = *(const uint4*)(stg + r16 * 64 + ((sq ^ ((r16 >> 1) & 3)) << 4));
-              if (ok && !(p.dbg & 4)) *(uint4*)((__nv_bfloat16*)p.out + ob + n0 + sq * 8) = u;
+              if (ok) *(uint4*)((__nv_bfloat16*)p.out + ob + n0 + sq * 8) = u;
             }
             __syncwarp();
           }
@@ -1000,8 +987,7 @@ __global__ void __launch_bounds__(FUSE ? kTcThreadsFused : kTcThreads, 1) gemm_t
               for (int j = 0; j < 32; ++j)
                 if (n0 + j < p.Ncols) f[j] += p.res2_scale * ld_dt(p.res2, qbase + (long long)(n0 + j) * p.q_sc, p.res2_dtype);
             }
-            if (p.dbg & 4) {
-            } else if (vec_ok && p.out_dtype == WSR_BF16) {
+            if (vec_ok && p.out_dtype == WSR_BF16) {
               uint4* op = (uint4*)((__nv_bfloat16*)p.out + obase + n0);
   #pragma unroll
               for (int q = 0; q < 4; ++q) {
@@ -1211,12 +1197,6 @@ static bool stage_preconditions(const TcParams& p, int block_n) {
   return true;
 }
 
-// WSR_STAGE_MASK (debugging / measurement): bit 0 = vertical-tap-merge kernels, bit 1 = other halo kernels, bit 2 = classic
-static int stage_mask() {
-  static const int m = getenv("WSR_NO_STAGE") ? 0 : (getenv("WSR_STAGE_MASK") ? atoi(getenv("WSR_STAGE_MASK")) : 7);
-  return m;
-}
-
 template <int BLOCK_N>
 static int launch_tc(const TcParams& p, cudaStream_t st) {
   const bool sok = stage_preconditions(p, BLOCK_N);
@@ -1234,99 +1214,49 @@ static int launch_tc(const TcParams& p, cudaStream_t st) {
   }
   if (p.n_taps > 0) {
     if constexpr (BLOCK_N == 64) {
-      if (p.halo_rows == 3) {
-        if (sok && (stage_mask() & 1)) return launch_tc_impl<BLOCK_N, true, 3, false, true, true>(p, st);
-        return launch_tc_impl<BLOCK_N, true, 3, false, true>(p, st);
-      }
+      if (p.halo_rows == 3) return sok ? launch_tc_impl<BLOCK_N, true, 3, false, true, true>(p, st) : launch_tc_impl<BLOCK_N, true, 3, false, true>(p, st);
     }
     if constexpr (BLOCK_N <= 64) {
       if (p.halo_rows == 4) return launch_tc_impl<BLOCK_N, true, 4>(p, st);
     }
-    const bool stg = sok && (stage_mask() & 2);
     if constexpr (BLOCK_N <= 128) {
-      if (p.halo_rows == 2) return stg ? launch_tc_impl<BLOCK_N, true, 2, false, false, true>(p, st) : launch_tc_impl<BLOCK_N, true, 2>(p, st);
+      if (p.halo_rows == 2) return sok ? launch_tc_impl<BLOCK_N, true, 2, false, false, true>(p, st) : launch_tc_impl<BLOCK_N, true, 2>(p, st);
     }
-    return stg ? launch_tc_impl<BLOCK_N, true, 1, false, false, true>(p, st) : launch_tc_impl<BLOCK_N, true, 1>(p, st);
+    return sok ? launch_tc_impl<BLOCK_N, true, 1, false, false, true>(p, st) : launch_tc_impl<BLOCK_N, true, 1>(p, st);
   }
   if (p.ksplit > 1) {
-    WSR_REQUIRE(sok, WSR_E_INVALID, "gemm_tc: split-K chosen without the staged-epilogue preconditions");
-    return launch_tc_impl<BLOCK_N, false, 1, false, false, true, true>(p, st);
+    // pick_split only cuts launches whose tiles fit in half a wave, and pick_block_n gives those 64-column tiles
+    WSR_REQUIRE(BLOCK_N == 64 && p.ksplit == 2 && sok, WSR_E_INVALID, "gemm_tc: split-K chosen with BN=%d S=%d or without the staged-epilogue preconditions",
+                BLOCK_N, p.ksplit);
+    if constexpr (BLOCK_N == 64) return launch_tc_impl<BLOCK_N, false, 1, false, false, true, true>(p, st);
   }
   if constexpr (BLOCK_N == 256) {
-    if (p.pair) return (sok && (stage_mask() & 4)) ? launch_tc_pair<true>(p, st) : launch_tc_pair<false>(p, st);
+    if (p.pair) return sok ? launch_tc_pair<true>(p, st) : launch_tc_pair<false>(p, st);
   }
-  if (sok && (stage_mask() & 4)) return launch_tc_impl<BLOCK_N, false, 1, false, false, true>(p, st);
+  if (sok) return launch_tc_impl<BLOCK_N, false, 1, false, false, true>(p, st);
   return launch_tc_impl<BLOCK_N, false, 1>(p, st);
 }
 
-// Split-K plan for a classic-mode launch whose tiles do not fill the machine (deep UNet levels at small batch: 8 .. 64 row tiles for
-// 148 SMs).  What bounds such a launch is the operand fetch of each CTA -- one SM receives at most ~65 bytes per clock from L2
-// (tools/tma_probe.cu, profiles/r02_tma_probe.txt), and a 128 x BN x 64 K block needs 16 KB + BN * 128 B -- or its MMAs, 4 * (69 + 0.28 BN)
-// cycles; cutting the K loop over the S CTAs of a cluster divides both, at the price of the partial-tile exchange through distributed
-// shared memory (~1500 cycles of barriers + (S-1)/S * BN * 512 B at ~32 B per clock).  Returns the chosen BN and sets *ksplit (1 = no
-// split).  S is a power of two that divides the BN / 32 column chunks; at least 4 K blocks per split; tiles * S <= SMs.
+// Split-K for a classic-mode launch whose tiles do not fill the machine (deep UNet levels at small batch: 8 .. 64 row tiles for 148 SMs).
+// What bounds such a launch is the operand fetch of each CTA -- one SM receives at most ~65 bytes per clock from L2 (tools/tma_probe.cu,
+// profiles/r02_tma_probe.txt) -- or its MMAs; cutting the K loop over the CTAs of a cluster divides both, at the price of the
+// partial-tile exchange through distributed shared memory.
 // MEASURED on B200 (tools/prof_conv.py, profiles/r02_splitk_cluster_sweep.txt; 512->512 3x3 @8x16, 8 images, unsplit BN = 64: 24.7 us):
 // BN 64 / S 2: 21.1 us, BN 128 / S 2 and S 4: 22.9 / 22.7 us, BN 256 / S 2 and S 4: 27.3 us, BN 256 / S 8: 56 us.  The launch is
 // t = 5.3 us + 0.27 us per K block; halving the K loop saves 9.7 us and the cluster launch + two cluster-wide barrier rounds + the
 // exchange give 6 us of it back, and clusters of 8 do not even fit one wave.  Whole step at 8 images per GPU: 3.38 ms without, 3.90 ms
-// with the model's choice.  So the cost-model search is for tests only (WSR_SPLITK=2 / wsr_debug_set_splitk(2)); the default (1) applies the
-// single cut that measured faster, below; 0 = never.  (The round-1 global-memory exchange was worse still: 30 us.)
+// with a cost-model search over (BN, S) and S up to 8.  So the rule is the single cut that measured faster: keep the unsplit tile shape and
+// halve its K loop over a 2-CTA cluster, when that still fits one wave and the K loop is long enough to pay for the exchange (3x3
+// convolutions with >= 256 input channels: 24.7 -> 21.1 us, 43.7 -> 33.8 us, 28.8 -> 24.0 us on the 8x16 level at 8 images; 1x1
+// convolutions get SLOWER, 7.5 -> 9.6 us).  (The round-1 global-memory exchange was worse still: 30 us.)
+// Tiles that fit in half a wave always get BN = 64 from pick_block_n, so a split launch has BN = 64 and S = 2.  Returns S (1 = no split).
+static int pick_split(int ncols, int m_tiles, int total_kb, int bn) {
+  const int tiles = m_tiles * ((ncols + bn - 1) / bn);
+  return (total_kb >= 36 && 2 * tiles <= sm_count() && ncols % bn == 0) ? 2 : 1;
+}
+
 static int g_last_ksplit = 1, g_last_bn = 0, g_last_pair = 0;      // introspection for the tests (wsr_debug_last_tc_config)
-static int g_pair_mode = -1;                      // -1 = read WSR_PAIR on first use; wsr_debug_set_pair overrides
-static int g_splitk_on = -1;                      // -1 = read WSR_SPLITK on first use; 0 off, 1 the measured rule (default), 2 cost-model search (tests)
-
-static double kblock_cycles(int bn) {
-  const double fetch = (16384.0 + bn * 128.0) / 65.0, mma = 4.0 * (69.0 + 0.28 * bn);
-  return fetch > mma ? fetch : mma;
-}
-
-static int pick_split(int ncols, int m_tiles, int total_kb, int bn_nosplit, int* ksplit) {
-  *ksplit = 1;
-  if (g_splitk_on < 0) g_splitk_on = getenv("WSR_SPLITK") ? atoi(getenv("WSR_SPLITK")) : 1;
-  static const bool forced = getenv("WSR_SPLITK_FORCE") != nullptr;
-  if (!g_splitk_on && !forced) return bn_nosplit;
-  const int sms = sm_count();
-  // WSR_SPLITK_FORCE="bn,S": measurement override (tools/prof_conv.py); ignored when the plan is not feasible
-  static const char* force = getenv("WSR_SPLITK_FORCE");
-  if (force) {
-    int fbn = 0, fs = 0;
-    if (sscanf(force, "%d,%d", &fbn, &fs) == 2 && (fbn == 64 || fbn == 128 || fbn == 256) && ncols % fbn == 0) {
-      const int tiles = m_tiles * (ncols / fbn);
-      const int per = fs > 0 ? (total_kb + fs - 1) / fs : 0;
-      if ((fs == 2 || fs == 4 || fs == 8) && fs <= fbn / 32 && tiles * fs <= sms && per >= 1 && (fs - 1) * per < total_kb) { *ksplit = fs; return fbn; }
-      if (fs == 1) return fbn;
-    }
-    return bn_nosplit;
-  }
-  if (g_splitk_on == 1) {
-    // the one cut that measured faster (see above): keep the unsplit tile shape and halve its K loop over a 2-CTA cluster, when that
-    // still fits one wave and the K loop is long enough to pay for the exchange (3x3 convolutions with >= 256 input channels: 24.7 ->
-    // 21.1 us, 43.7 -> 33.8 us, 28.8 -> 24.0 us on the 8x16 level at 8 images; 1x1 convolutions get SLOWER, 7.5 -> 9.6 us)
-    const int tiles = m_tiles * ((ncols + bn_nosplit - 1) / bn_nosplit);
-    if (total_kb >= 36 && 2 * tiles <= sms && ncols % bn_nosplit == 0 && (bn_nosplit / 32) % 2 == 0) *ksplit = 2;
-    return bn_nosplit;
-  }
-  const double base_tiles = (double)m_tiles * ((ncols + bn_nosplit - 1) / bn_nosplit);
-  const double base = ceil(base_tiles / sms) * total_kb * kblock_cycles(bn_nosplit);
-  double best = base * 0.85;                       // split only for a clear win
-  int best_bn = bn_nosplit;
-  const int cand_bn[3] = {256, 128, 64};
-  const int cand_s[3] = {2, 4, 8};
-  for (int i = 0; i < 3; ++i) {
-    const int bn = cand_bn[i];
-    if (ncols % bn != 0) continue;
-    const int tiles = m_tiles * (ncols / bn);
-    for (int j = 0; j < 3; ++j) {
-      const int S = cand_s[j];
-      if (S > bn / 32 || tiles * S > sms) continue;
-      const int per = (total_kb + S - 1) / S;
-      if (per < 4 || (S - 1) * per >= total_kb) continue;
-      const double cost = per * kblock_cycles(bn) + 1500.0 + 16.0 * bn * (S - 1) / S;
-      if (cost < best) { best = cost; best_bn = bn; *ksplit = S; }
-    }
-  }
-  return best_bn;
-}
+static int g_pair_mode = 1;                       // CTA-pair policy, see wsr_debug_set_pair
 
 static int pick_block_n(int ncols, int m_tiles) {
   // Column-tile width by a small cost model measured on B200: one 128 x BN x 16 MMA costs about (69 + 0.28 * BN) cycles
@@ -1366,15 +1296,9 @@ static inline int cdiv(int a, int b) { return (a + b - 1) / b; }
 
 /* (column-tile width << 8) | K splits of the most recent wsr_conv_tc / wsr_conv_taps_tc launch of this process (tests only) */
 extern "C" int wsr_debug_last_tc_config(void) { return (g_last_pair << 20) | (g_last_bn << 8) | g_last_ksplit; }
-/* enable (1) / disable (0) the split-K plan of wsr_conv_tc / wsr_conv_taps_tc for this process; returns the previous setting */
 // CTA-pair policy of the classic 256-column convolution tiles: 0 never, 1 launches of more than one wave (default), 2 every eligible launch
 extern "C" int wsr_debug_set_pair(int mode) {
-  if (g_pair_mode < 0) g_pair_mode = getenv("WSR_PAIR") ? atoi(getenv("WSR_PAIR")) : 1;
   const int prev = g_pair_mode; g_pair_mode = mode < 0 ? 0 : (mode > 2 ? 2 : mode); return prev;
-}
-extern "C" int wsr_debug_set_splitk(int on) {
-  if (g_splitk_on < 0) g_splitk_on = getenv("WSR_SPLITK") ? atoi(getenv("WSR_SPLITK")) : 1;
-  const int prev = g_splitk_on; g_splitk_on = on < 0 ? 0 : (on > 2 ? 2 : on); return prev;
 }
 
 extern "C" int wsr_conv_tc(const WsrConvDesc* d, void* stream) {
@@ -1421,29 +1345,22 @@ extern "C" int wsr_conv_tc(const WsrConvDesc* d, void* stream) {
   p.q_s1 = d->res2_ld; p.q_s2 = (long long)OW * d->res2_ld; p.q_s3 = (long long)OH * OW * d->res2_ld; p.q_sc = 1;
 
   const int m_tiles = p.g1 * p.g2 * p.g3;
-  int bn = pick_block_n(d->Cout, m_tiles);
+  const int bn = pick_block_n(d->Cout, m_tiles);
   // halo mode: when a tile is a segment of ONE image row, the 9 taps are 9 shifted views of a single halo tile, so the
   // activation operand is fetched once per 64-channel chunk instead of once per tap; with two output rows per tile
   // (two accumulators) every weight tile is used twice as well.  Both cut the L2 -> SM traffic that bounds these layers.
-  static const bool no_halo = getenv("WSR_NO_HALO") != nullptr;
-  static const int max_rows = getenv("WSR_HALO_ROWS") ? atoi(getenv("WSR_HALO_ROWS")) : 4;
-  const bool halo = !no_halo && d->ksize == 3 && d->stride == 1 && p.t2 == 1 && p.t3 == 1 && p.t1 + 2 <= 130;
-  // split-K (classic tiles that do not fill the machine; needs the caller's workspace and the staged-epilogue preconditions)
+  const bool halo = d->ksize == 3 && d->stride == 1 && p.t2 == 1 && p.t3 == 1 && p.t1 + 2 <= 130;
+  // split-K (classic tiles that do not fill the machine; needs the staged-epilogue preconditions)
   p.ksplit = 1;
-  if (!halo && d->gn_table == nullptr && stage_preconditions(p, 64)) {
+  if (!halo && d->gn_table == nullptr && stage_preconditions(p, bn)) {
     const int kb_est = (merged ? 4 : taps) * (d->Cin / 64) + (d->x2 ? d->Cin2 / 64 : 0);
-    int ks = 1;
-    const int bn2 = pick_split(d->Cout, m_tiles, kb_est, bn, &ks);
-    if (ks == 1 || stage_preconditions(p, bn2)) {
-      bn = bn2;
-      if (ks > 1) { p.ksplit = ks; p.kb_split = (kb_est + ks - 1) / ks; }
-    }
+    p.ksplit = pick_split(d->Cout, m_tiles, kb_est, bn);
+    p.kb_split = cdiv(kb_est, p.ksplit);
   }
   // vertical tap merge (N = 64, plain 3x3): three output rows per tile, needs the vmerge weight pack (w_vmerge)
-  static const bool no_vm = getenv("WSR_NO_VMERGE") != nullptr;
-  const bool vmerge = halo && bn == 64 && taps == 9 && !d->upsample && d->w_vmerge != nullptr && !no_vm;
+  const bool vmerge = halo && bn == 64 && taps == 9 && !d->upsample && d->w_vmerge != nullptr;
   // (the 4-row tiles have no shared memory left for the staged epilogue and are not built with the fused GroupNorm input)
-  const int hrows = vmerge ? 3 : (halo && bn <= 64 && GH % 4 == 0 && max_rows >= 4 && d->gn_table == nullptr) ? 4 : (halo && bn <= 128 && GH % 2 == 0 && max_rows >= 2) ? 2 : 1;
+  const int hrows = vmerge ? 3 : (halo && bn <= 64 && GH % 4 == 0 && d->gn_table == nullptr) ? 4 : (halo && bn <= 128 && GH % 2 == 0) ? 2 : 1;
   WSR_REQUIRE(d->gn_table == nullptr || halo, WSR_E_UNSUPPORTED,
               "conv_tc: the fused GroupNorm input needs a stride-1 3x3 convolution on rows of >= 128 pixels (see wsr_conv_tc_can_fuse_gn)");
   if (d->gn_table) {
@@ -1455,22 +1372,14 @@ extern "C" int wsr_conv_tc(const WsrConvDesc* d, void* stream) {
   }
   p.n_taps = halo ? taps : 0;
   p.halo_rows = hrows;
-  {
-    // WSR_HALO_PREFETCH: 0 = never, 1 = fused-GroupNorm kernels only (default), 2 = every halo kernel
-    static const int pf = getenv("WSR_HALO_PREFETCH") ? atoi(getenv("WSR_HALO_PREFETCH")) : 1;
-    p.prefetch = halo && (pf >= 2 || (pf == 1 && d->gn_table != nullptr)) ? 1 : 0;
-  }
   p.halo_bytes = (p.t1 + 2) * (hrows + 2) * 128;
   if (halo) { p.g2 = cdiv(GH, hrows); p.a_bytes = p.t1 * hrows * 128; }
   const bool fuse_stats = d->gn_stats != nullptr && (halo ? p.t1 % 32 == 0 : (p.t1 * p.t2) % 32 == 0);
   p.stats = fuse_stats ? d->gn_stats : nullptr;
   p.stats_ld = d->gn_stats_ld;
-  static const int dbg_flags = getenv("WSR_TC_DBG") ? atoi(getenv("WSR_TC_DBG")) : 0;
-  p.dbg = dbg_flags;
 
-  // CTA pairs (cta_group::2) for the classic 256-column tiles: needs an even number of row tiles; WSR_PAIR=0 switches it off, WSR_PAIR=2
-  // takes every eligible launch (tests)
-  if (g_pair_mode < 0) g_pair_mode = getenv("WSR_PAIR") ? atoi(getenv("WSR_PAIR")) : 1;
+  // CTA pairs (cta_group::2) for the classic 256-column tiles: needs an even number of row tiles; wsr_debug_set_pair(2) takes every
+  // eligible launch (tests)
   const int pair_mode = g_pair_mode;
   const bool pair_on = pair_mode != 0;
   // (measured on B200, tools/prof_conv.py: +6..7 % on the launches of more than one wave -- 1348 -> 1437, 1416 -> 1496, 1454 -> 1552 TFLOP/s
@@ -1601,7 +1510,7 @@ extern "C" int wsr_conv_tc_can_fuse_gn(const WsrConvDesc* d) {
   if (d->Cin % 64 != 0 || (d->x2 && d->Cin2 % 64 != 0)) return 0;
   int t1, t2, t3;
   choose_tile(d->W, d->H, d->N, t1, t2, t3);
-  return (t2 == 1 && t3 == 1 && t1 + 2 <= 130 && getenv("WSR_NO_HALO") == nullptr) ? 1 : 0;
+  return (t2 == 1 && t3 == 1 && t1 + 2 <= 130) ? 1 : 0;
 }
 
 // Tap-table variant (data gradients of the stride-2 / upsample convolutions; see wsr.h).  Classic (non-halo) tiles only.
@@ -1641,17 +1550,13 @@ extern "C" int wsr_conv_taps_tc(const WsrConvDesc* d, const WsrTapTable* t, void
   p.res2 = d->res2; p.res2_dtype = d->res2_dtype; p.res2_scale = d->res2_scale;
   p.q_s1 = d->res2_ld; p.q_s2 = (long long)OW * d->res2_ld; p.q_s3 = (long long)OH * OW * d->res2_ld; p.q_sc = 1;
   const int m_tiles = p.g1 * p.g2 * p.g3;
-  int bn = pick_block_n(d->Cout, m_tiles);
+  const int bn = pick_block_n(d->Cout, m_tiles);
   p.n_taps = 0; p.halo_rows = 1;
   p.ksplit = 1;
-  if (stage_preconditions(p, 64)) {
+  if (stage_preconditions(p, bn)) {
     const int kb_est = t->ntaps * (d->Cin / 64);
-    int ks = 1;
-    const int bn2 = pick_split(d->Cout, m_tiles, kb_est, bn, &ks);
-    if (ks == 1 || stage_preconditions(p, bn2)) {
-      bn = bn2;
-      if (ks > 1) { p.ksplit = ks; p.kb_split = (kb_est + ks - 1) / ks; }
-    }
+    p.ksplit = pick_split(d->Cout, m_tiles, kb_est, bn);
+    p.kb_split = cdiv(kb_est, p.ksplit);
   }
   const bool fuse_stats = d->gn_stats != nullptr && (p.t1 * p.t2) % 32 == 0;
   p.stats = fuse_stats ? d->gn_stats : nullptr;

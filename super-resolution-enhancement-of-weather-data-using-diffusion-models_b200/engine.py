@@ -105,7 +105,6 @@ class Engine:
         self.prof = None         # list of (name, flops, bytes, start_event, end_event) when profiling
         self.prof_detail = False
         self.no_fused_attention = False
-        self.splitk_ws = None          # WsrConvDesc.splitk_ws is reserved: split-K partials travel through distributed shared memory
 
     # ---- plumbing -------------------------------------------------------------------------------------------------
     def call(self, name, *args, flops=0, nbytes=0, tag=None, xflops=None):
@@ -334,8 +333,6 @@ class Engine:
         if res2 is not None:
             d.res2, d.res2_dtype, d.res2_ld, d.res2_scale = res2.ptr, res2.dt, res2.ld, res2_scale
         d.y, d.y_dtype, d.y_ld = y.ptr, y.dt, y.ld
-        if self.splitk_ws is not None:
-            d.splitk_ws, d.splitk_ws_bytes = self.splitk_ws.data_ptr(), self.splitk_ws.numel()
         if y.st is not None:
             d.gn_stats, d.gn_stats_ld = y.stats_ptr, y.st_ld       # GroupNorm statistics of y come out of the epilogue
         if gn is not None:

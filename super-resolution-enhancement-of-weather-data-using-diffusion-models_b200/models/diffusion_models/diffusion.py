@@ -9,7 +9,6 @@ instead of ~610 eager launches plus a host->device copy (reference diffusion.py:
 from abc import abstractmethod
 
 import numpy as np
-import os
 import torch
 from torch import nn
 
@@ -249,15 +248,15 @@ class ReverseLoop:
         torch.cuda.synchronize(self.plan.eng.device)
         self.graph = torch.cuda.CUDAGraph()
         # small batches (<= 8 images of 128x256 per GPU -- the sharded benchmark): the ~190 launches of a step are short enough for the
-        # gaps between them to show, so the graph is captured with programmatic dependent launch (wsr.h: wsr_set_pdl); WSR_PDL overrides
+        # gaps between them to show, so the graph is captured with programmatic dependent launch (wsr.h: wsr_set_pdl)
         small = self.x.shape[0] * self.x.shape[-2] * self.x.shape[-1] <= 8 * 128 * 256
-        prev = nat.call("wsr_set_pdl", 1) if (small and "WSR_PDL" not in os.environ) else None
+        prev = nat.call("wsr_set_pdl", 1) if small else None
         try:
             with torch.cuda.graph(self.graph):
                 self.step()
         finally:
             if prev is not None:
-                nat.call("wsr_set_pdl", max(prev, 0))
+                nat.call("wsr_set_pdl", prev)
         return self.graph
 
     def replay(self):

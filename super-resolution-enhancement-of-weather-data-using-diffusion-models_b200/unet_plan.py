@@ -52,11 +52,9 @@ class UNetPlan:
         # (profiles/r02_fused_gn_decomposition.txt):  128->128 @64x128: 0.166 ms fused vs 0.141 conv + 0.061 gn_apply;
         # 384->128: 0.441 vs 0.358 + 0.138;  but 64->64 @128x256: 0.326 vs 0.163 + 0.094 and 192->64: 0.719 vs 0.364 + 0.260 --
         # the N = 64 layers are bound by the tensor core's own shared-memory operand fetch, and the transform's traffic on the same
-        # banks slows both.  Policy (WSR_FUSE_GN): 1 (default) = fuse where the convolution's column tile is >= 128 wide, 2 = fuse
-        # every eligible layer, 0 = never.
-        import os
-        self.fuse_gn_mode = int(os.environ.get("WSR_FUSE_GN", "1")) if (getattr(self, "fuse_gn", True) and self.eng.mode == "bf16") else 0
-        self.fuse_gn = self.fuse_gn_mode > 0
+        # banks slows both.  So only layers with at least 128 output channels fuse (_res_block); fusing every eligible layer measured
+        # slower at every batch size (DESIGN.md section 8).
+        self.fuse_gn = getattr(self, "fuse_gn", True) and self.eng.mode == "bf16"
         self._structure()
         self._buffers()
         self.refresh_weights()
@@ -463,7 +461,7 @@ class UNetPlan:
         e, B, G = self.eng, self.B, self.groups
         SW = nat.ACT_SWISH
         if not hasattr(r, "fuse1"):
-            wide = self.fuse_gn_mode >= 2 or r.cout >= 128
+            wide = r.cout >= 128
             r.fuse1 = self.fuse_gn and wide and e.conv_can_fuse_gn(x, r.conv1)
             r.fuse2 = self.fuse_gn and wide and e.conv_can_fuse_gn(r.hbuf, r.conv2, x2=x if r.has_res_conv else None)
             r.tab1 = e.empty((B, r.cin, 2), torch.float32) if r.fuse1 else None
@@ -513,8 +511,7 @@ class UNetPlan:
 
     def _plain_plan(self):
         """The sampling / inference plan (not the train plan, whose backward pass reads q | k and V^T separately)."""
-        import os
-        return type(self) is UNetPlan and os.environ.get("WSR_NO_NHWC_V") is None
+        return type(self) is UNetPlan
 
     def _side_stream(self):
         """The HF-guided cross-attention branches (resdiff/unet.py:156-163: they only produce the SKIP tensors; the main path continues
@@ -526,9 +523,8 @@ class UNetPlan:
             return None
         ok = getattr(self, "_side_ok", None)
         if ok is None:
-            import os
             e = self.eng
-            ok = e.use_tc and e.mode == "bf16" and not e.no_fused_attention and os.environ.get("WSR_NO_SIDE_STREAM") is None
+            ok = e.use_tc and e.mode == "bf16" and not e.no_fused_attention
             for ca in self.hfca:
                 n = ca.h * ca.w
                 fused_long = ca.c in (64, 128) and n % 128 == 0
@@ -573,9 +569,7 @@ class UNetPlan:
         (wsr_final_conv_sampler_step): bf16 sampling plan, head input produced by a convolution that emitted its statistics."""
         ok = getattr(self, "_fuse_head", None)
         if ok is None:
-            import os
             ok = self._fuse_head = (type(self) is UNetPlan and self.eng.mode == "bf16" and self.eng.use_tc
-                                    and os.environ.get("WSR_NO_FUSED_HEAD") is None
                                     and bool(nat.call("wsr_head_sampler_supported", self.final_cin, self.C_img, self.groups)))
         return ok
 
@@ -640,12 +634,5 @@ class UNetPlan:
     def _head(self, x):
         """final_conv = GroupNorm -> Swish -> conv3x3 (resdiff/unet.py:119, nn_modules/resnet.py:19-28)."""
         e = self.eng
-        if not hasattr(self, "fuse_final"):
-            self.fuse_final = self.fuse_gn_mode >= 2 and e.conv_can_fuse_gn(x, self.final)
-            self.tab_final = e.empty((self.B, self.final_cin, 2), torch.float32) if self.fuse_final else None
-        if self.fuse_final:
-            e.gn_finalize(x, self.gf, self.bf_, self.groups, self.tab_final)
-            e.conv(x, self.final, self.eps_nhwc, gn=(self.tab_final, nat.ACT_SWISH))
-        else:
-            e.gn_apply(x, self.gf, self.bf_, self.groups, nat.ACT_SWISH, self.final_a)
-            e.conv(self.final_a, self.final, self.eps_nhwc)
+        e.gn_apply(x, self.gf, self.bf_, self.groups, nat.ACT_SWISH, self.final_a)
+        e.conv(self.final_a, self.final, self.eps_nhwc)

@@ -20,7 +20,6 @@ them, so a data-parallel trainer can all-reduce contiguous buckets while the res
 import ctypes
 import functools
 import math
-import os
 
 import torch
 
@@ -44,9 +43,9 @@ class UNetTrainPlan(UNetPlan):
         self._seed = ctypes.c_uint64(0)
         self._lists = {}
         self._n_bwd = 0
-        self.replay_enabled = os.environ.get("WSR_NO_REPLAY") is None
+        self.replay_enabled = True
         self._jobtab = None            # (device WsrPackJob table, njobs, total units, parameter-address signature)
-        self.batched_refresh = os.environ.get("WSR_NO_BATCHED_REFRESH") is None
+        self.batched_refresh = True     # False: re-pack weights tensor by tensor (the reference the tests compare with)
         self.fuse_gn = False           # the backward pass reads the normalised activations (a1, a2): keep them materialised
         super().__init__(net, batch, device, precision, strict_tc)
         self.eng.no_fused_attention = False
@@ -312,10 +311,10 @@ class UNetTrainPlan(UNetPlan):
     # step's kernel time) go to a second stream and run BESIDE the chain: fork = the side stream waits for everything the main
     # stream has issued so far (x and dy of the layer are final by then and are not written again during this backward), join =
     # the main stream waits for the side stream before a gradient range is handed to the all-reduce / optimizer.  Both are host
-    # callbacks in the recorded launch list, so replays fork and join exactly like the recording run.  WSR_WGRAD_STREAM=0: off.
+    # callbacks in the recorded launch list, so replays fork and join exactly like the recording run.
     def _wstream(self):
         if not hasattr(self, "_wside"):
-            on = os.environ.get("WSR_WGRAD_STREAM", "1") != "0" and self.eng.device.type == "cuda"
+            on = self.eng.device.type == "cuda"
             self._wside = torch.cuda.Stream(device=self.eng.device) if on else None
             self._wev_fork = torch.cuda.Event() if on else None
             self._wev_join = torch.cuda.Event() if on else None
@@ -365,11 +364,10 @@ class UNetTrainPlan(UNetPlan):
     # that Downsample again -- half a pass later.  In between sits the most expensive single piece of the step, the N = 8192 attention
     # backward through four (B, 8192, 8192) matrices.  The branches therefore run on their own stream from the end of the up path on
     # (deepest level first, the order in which the chain will ask for them), each into a private dx buffer and private attention
-    # scratch; the chain joins a branch where it used to compute it and adds the private dx.  WSR_HFCA_STREAM=0: off.
+    # scratch; the chain joins a branch where it used to compute it and adds the private dx.
     def _hstream(self):
         if not hasattr(self, "_hside"):
-            on = (os.environ.get("WSR_HFCA_STREAM", "1") != "0" and self.eng.device.type == "cuda" and self.has_hfca
-                  and self.scores is not None)
+            on = self.eng.device.type == "cuda" and self.has_hfca and self.scores is not None
             if on:
                 # the branch needs its own (B, N, N) scratch set (3.2 GB at batch 4): beyond 8 GB the batch is large enough to fill the
                 # machine without the overlap, and the memory is better left to the activations

@@ -19,6 +19,7 @@ torch.backends.cuda.matmul.allow_tf32 = False
 nat = wsr.pkg.native
 engine_mod = wsr.sub("engine")
 Engine, Act = engine_mod.Engine, engine_mod.Act
+T = wsr.sub("taps")
 
 
 def _dev():
@@ -126,30 +127,29 @@ def test_conv_tc_vs_simt(case):
 
 
 SPLITK_CASES = [
-    # N, Cin, Cout, H, W, k, stride, up, Cin2 (fused 1x1 segment), expect a split
-    (8, 512, 512, 8, 16, 3, 1, False, 0, True),        # the 8x16 level at 8 samples per GPU: 8 row tiles for 148 SMs
-    (8, 512, 512, 8, 16, 3, 1, False, 1024, True),     # ... with the ResnetBlock's 1x1 res_conv as a second K segment
-    (8, 1024, 512, 16, 32, 3, 1, False, 0, True),      # the 16x32 level: 32 row tiles
-    (8, 512, 512, 8, 16, 3, 1, True, 0, True),         # nearest-x2 + 3x3 (phase-merged taps, 4 launches)
-    (8, 512, 512, 16, 32, 3, 2, False, 0, True),       # stride 2 (phase-subsampled tensor maps)
-    (3, 192, 256, 4, 8, 3, 1, False, 0, True),         # uneven split of 27 K blocks, partial row tile
-    (64, 512, 512, 8, 16, 3, 1, False, 0, False),      # enough tiles: no split
+    # N, Cin, Cout, H, W, k, stride, up, Cin2 (fused 1x1 segment), expect a split.  Every split case has 64-column tiles.
+    pytest.param(8, 512, 512, 8, 16, 3, 1, False, 0, True, id="3x3-8x16"),           # 64 tiles, 72 K blocks: halved over 2-CTA clusters
+    pytest.param(8, 512, 512, 8, 16, 3, 1, False, 1024, True, id="3x3-res_conv"),    # ... + the 1x1 res_conv as a second K segment (88)
+    pytest.param(8, 640, 512, 8, 16, 3, 1, True, 0, True, id="merged-upsample"),     # phase-merged nearest-x2 + 3x3, 4 launches of 40
+    pytest.param(8, 512, 512, 16, 32, 3, 2, False, 0, True, id="stride2"),           # phase-subsampled tensor maps
+    pytest.param(3, 576, 256, 4, 8, 3, 1, False, 0, True, id="uneven-partial"),      # 81 K blocks split 41 / 40, partial 96-row tile
+    pytest.param(4, 256, 512, 8, 16, 4, 1, "dgrad", 0, True, id="taps-dgrad"),       # tap table: dgrad of nearest-x2 + 3x3, 16 taps, 64 K blocks
+    pytest.param(64, 256, 512, 8, 16, 4, 1, "dgrad", 0, False, id="taps-dgrad-b64"), # ... at 64 images: 128 tiles of 256 columns
+    pytest.param(8, 512, 512, 8, 16, 1, 1, False, 0, False, id="1x1"),               # 1x1: the K loop is too short to pay for the exchange
+    pytest.param(8, 512, 512, 16, 32, 3, 1, False, 0, False, id="3x3-16x32"),        # 128 tiles of 128 columns: no room for a second CTA
+    pytest.param(8, 1024, 512, 16, 32, 3, 1, False, 0, False, id="3x3-16x32-1024"),  # ... with a longer K loop
+    pytest.param(64, 512, 512, 8, 16, 3, 1, False, 0, False, id="3x3-8x16-b64"),     # enough tiles: no split
 ]
 
 
-@pytest.mark.parametrize("case", SPLITK_CASES)
-def test_conv_tc_split_k_vs_simt(case):
-    """Split-K of the classic-mode tcgen05 convolution (tiles that do not fill the SMs): the CTAs of a thread-block cluster each
-    accumulate a range of the K blocks and exchange fp32 partial tiles through distributed shared memory; distributed fix-up with
-    bias / time-embedding row / residual / GroupNorm statistics in the epilogue; compared with the SIMT kernel on the same bf16
-    operands, run twice.  The path is correct but measured not worth it on B200 (DESIGN.md section 8), so it is off by default; the
-    test switches it on (wsr_debug_set_splitk) for its own launches only."""
-    N, Cin, Cout, H, W, k, stride, up, Cin2, expect = case
-    prev = nat.call("wsr_debug_set_splitk", 2)
-    try:
-        _split_k_case(N, Cin, Cout, H, W, k, stride, up, Cin2, expect)
-    finally:
-        nat.call("wsr_debug_set_splitk", prev)
+@pytest.mark.parametrize("N, Cin, Cout, H, W, k, stride, up, Cin2, expect", SPLITK_CASES)
+def test_conv_tc_split_k_vs_simt(N, Cin, Cout, H, W, k, stride, up, Cin2, expect):
+    """Split-K of the classic-mode tcgen05 convolution: only the cut that measured faster on B200 -- the unsplit tile shape with its K
+    loop halved over a 2-CTA cluster, for 3x3 convolutions whose tiles fill at most half of the SMs.  The two CTAs each accumulate half
+    of the K blocks and exchange fp32 partial tiles through distributed shared memory; distributed fix-up with bias / time-embedding
+    row / residual / GroupNorm statistics in the epilogue; compared with the SIMT kernel on the same bf16 operands, run twice, and the
+    split (or its absence) checked through wsr_debug_last_tc_config."""
+    _split_k_case(N, Cin, Cout, H, W, k, stride, up, Cin2, expect)
 
 
 PAIR_CASES = [
@@ -177,28 +177,17 @@ def test_conv_tc_cta_pair_vs_simt(case):
         nat.call("wsr_debug_set_pair", prev)
 
 
-@pytest.mark.parametrize("case", [
-    (8, 512, 512, 8, 16, 3, 1, False, 0, True),        # 64 tiles of 64 columns, 72 K blocks: halved over 2-CTA clusters
-    (8, 512, 512, 8, 16, 3, 1, False, 1024, True),     # ... with the fused 1x1 segment
-    (8, 512, 512, 8, 16, 1, 1, False, 0, False),       # 1x1: the K loop is too short to pay for the exchange
-    (8, 512, 512, 16, 32, 3, 1, False, 0, False),      # 128 tiles: no room for a second CTA per tile
-])
-def test_conv_tc_split_k_default_rule(case):
-    """The default split-K policy (mode 1): only the cut that measured faster on B200 -- the unsplit tile shape with its K loop halved over
-    a 2-CTA cluster, for 3x3 convolutions whose tiles fill at most half of the SMs."""
-    prev = nat.call("wsr_debug_set_splitk", 1)
-    try:
-        _split_k_case(*case)
-    finally:
-        nat.call("wsr_debug_set_splitk", prev)
-
-
 def _split_k_case(N, Cin, Cout, H, W, k, stride, up, Cin2, expect, expect_pair=None):
+    # up == "dgrad": the tap-table data gradient of nearest-x2 + 3x3 with input (H, W) -- a 4x4 convolution reading dY at (2H, 2W)
+    dgrad, up = up == "dgrad", up is True
     torch.manual_seed(12)
     dev = _dev()
     eng = Engine(dev, "bf16")
-    x = torch.randn(N, Cin, H, W, device=dev)
-    w = torch.randn(Cout, Cin, k, k, device=dev) / math.sqrt(Cin * k * k)
+    x = torch.randn(N, Cin, 2 * H, 2 * W, device=dev) if dgrad else torch.randn(N, Cin, H, W, device=dev)
+    if dgrad:
+        w = T.upsample_dgrad_weight(torch.randn(Cin, Cout, 3, 3, device=dev) / math.sqrt(Cout * 9))
+    else:
+        w = torch.randn(Cout, Cin, k, k, device=dev) / math.sqrt(Cin * k * k)
     b = torch.randn(Cout, device=dev)
     rv = torch.randn(N, Cout, device=dev)
     OH, OW = (H * (2 if up else 1)) // stride, (W * (2 if up else 1)) // stride
@@ -207,6 +196,8 @@ def _split_k_case(N, Cin, Cout, H, W, k, stride, up, Cin2, expect, expect_pair=N
     pc_ref = eng.pack_conv(w, b)
     xa, ra = _nhwc(x, eng), _nhwc(res, eng)
     kw = dict(stride=stride, upsample=up, rowvec=rv.data_ptr(), rowvec_ld=Cout, res=ra)
+    if dgrad:
+        kw["taps"] = T.dgrad_upsample_taps(H, W)
     kw_ref = dict(kw)
     if Cin2:
         x2 = torch.randn(N, Cin2, H, W, device=dev)

@@ -1,6 +1,6 @@
 """Times single tcgen05 convolution shapes as CUDA-graph replays (no host overhead in the timed region), for calibrating the
 column-tile / split-K cost model of csrc/gemm_tc.cu.
-usage: python tools/prof_conv.py [B]          env: WSR_NO_SPLITK=1, WSR_SPLITK_FORCE="bn,S" """
+usage: python tools/prof_conv.py [B]"""
 import math
 import os
 import sys

@@ -1,5 +1,5 @@
-"""Profiling helper: one 3x3 conv with and without the fused GroupNorm input, under the WSR_TC_DBG switches
-(1 = skip epilogue work, 2 = skip MMA issue).  usage: python tools/prof_fuse.py N Cin Cout H W [reps]"""
+"""Profiling helper: one 3x3 conv with and without the fused GroupNorm input.
+usage: python tools/prof_fuse.py N Cin Cout H W [reps]"""
 import math
 import os
 import sys
@@ -47,8 +47,8 @@ def main():
     t_gn = timed(lambda: eng.gn_apply(x, gamma, beta, 32, nat.ACT_SWISH, a))
     t_fused = timed(lambda: eng.conv(x, pc, y, gn=(tab, nat.ACT_SWISH)))
     fl = 2.0 * N * H * W * Cout * Cin * 9
-    print("dbg=%s conv %d->%d %dx%d N=%d: plain %.3f ms (%.0f TF/s), gn_apply %.3f ms, fused %.3f ms (%.0f TF/s)" % (
-        os.environ.get("WSR_TC_DBG", "0"), Cin, Cout, H, W, N, t_plain, fl / t_plain / 1e9, t_gn, t_fused, fl / t_fused / 1e9))
+    print("conv %d->%d %dx%d N=%d: plain %.3f ms (%.0f TF/s), gn_apply %.3f ms, fused %.3f ms (%.0f TF/s)" % (
+        Cin, Cout, H, W, N, t_plain, fl / t_plain / 1e9, t_gn, t_fused, fl / t_fused / 1e9))
 
 
 if __name__ == "__main__":
