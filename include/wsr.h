@@ -358,6 +358,17 @@ int wsr_standard_scale(const float* x, int planes, int64_t hw, const float* mean
 /* One pass for MAE / MSE / RMSE / MR (training/metrics.py:75-201): acc[0] += sum |d|, acc[1] += sum d^2, acc[2] += sum d (doubles),
  * d = scale[plane] * (pred - target); scale = per-plane std folds the inverse transform in (the means cancel), or NULL. */
 int wsr_error_sums(const float* pred, const float* target, int planes, int64_t hw, const float* scale, double* acc, void* stream);
+/* Probabilistic scores of an ensemble, one pass.  ens: N members (2 <= N <= 256), member-major, member i's planes at
+ * ens + i * member_stride (fp32, planes * hw each: the layout of an N x B reverse-loop batch).  Per pixel, over the members x_i:
+ *   mean[p*hw + j] = (1/N) sum_i x_i,  spread[p*hw + j] = sqrt(sum_i (x_i - mean)^2 / (N - 1))      (input units; either may be NULL)
+ * and ACCUMULATED per plane p into acc[p*5 + k] (doubles, zeroed by the caller), with s = scale[p] (or 1 when scale is NULL):
+ *   k = 0: s * (1/N) sum_i |x_i - y|       k = 1: s * sum_i sum_j |x_i - x_j|  (= 2 sum_k (2k - N + 1) x_(k), x_(k) sorted ascending)
+ *   k = 2: s^2 * (mean - y)^2              k = 3: s^2 * sum_i (x_i - mean)^2 / (N - 1)              k = 4: s * (mean - y)
+ * so CRPS = acc0/n - acc1/(2 N^2 n) (standard) or acc0/n - acc1/(2 N (N-1) n) (fair) over n pixels.  Without target (NULL) only k = 3
+ * is accumulated.  rank_hist (or NULL; needs target): rank_hist[p*(N+1) + r] += 1 for every pixel whose target has r members STRICTLY
+ * below it -- members equal to the target count as not below.  scale folds the inverse StandardScaling in, as in wsr_error_sums. */
+int wsr_ensemble_stats(const float* ens, int N, int64_t member_stride, const float* target, int planes, int64_t hw, const float* scale,
+                       float* mean, float* spread, double* acc, unsigned long long* rank_hist, void* stream);
 
 /* Prior pre-training (SURVEY.md 8f N4).  image_compare_loss of models/simple_cnn/loss.py:60-76: alpha * fft_mse_loss +
  * beta * dwt_mse_loss (4 Haar levels) between x and y, fp32 NCHW planes with H, W multiples of 16.  *loss += value (double);
@@ -396,6 +407,19 @@ int wsr_final_conv_sampler_step(const void* x, int x_ld, int B, int H, int W, in
                                 const float* bias, int Cout, float* eps_out, float* x_state, const float* z,
                                 int64_t z_step_stride, uint64_t seed, const float* tables, int T, const int* t_dev, int clip,
                                 void* stream);
+/* Member-keyed (ensemble) variants of wsr_sampler_step, wsr_final_conv_sampler_step and wsr_randn: the batch is a stack of members of
+ * member_elems elements each (C*H*W*B_cond), and element i draws from Philox key member_keys[i / member_elems] (device array) at the
+ * member-local element i % member_elems instead of key `seed` at element i.  So the slice of member m is bit-identical to the plain entry
+ * point run on that slice alone with seed = member_keys[m], however the members are batched.  member_elems must be a positive multiple
+ * of 4 (a Philox group of 4 elements never straddles two members); other values return WSR_E_INVALID.  Injected noise (z) ignores the keys. */
+int wsr_sampler_step_members(const float* x, const void* eps, int eps_dtype, const float* z, int64_t z_step_stride,
+                             const uint64_t* member_keys, int64_t member_elems, const float* tables, int T, const int* t_dev, int clip,
+                             float* x_out, int64_t n, void* stream);
+int wsr_final_conv_sampler_step_members(const void* x, int x_ld, int B, int H, int W, int Cin, const double* stats, int stats_ld,
+                                        const float* gamma, const float* beta, int groups, float gn_eps, const void* w,
+                                        const float* bias, int Cout, float* eps_out, float* x_state, const float* z,
+                                        int64_t z_step_stride, const uint64_t* member_keys, int64_t member_elems, const float* tables,
+                                        int T, const int* t_dev, int clip, void* stream);
 int wsr_head_sampler_supported(int Cin, int Cout, int groups);
 int wsr_pack_head_weight(const float* w_tap_cout_cin, int Cout, int Cin, void* dst, void* stream);
 /* out[b][:] = table[r][:] for b < B, r = *row_index (one row of the per-time-step projection table broadcast to the
@@ -405,6 +429,7 @@ int wsr_broadcast_row(const float* table, int P, const int* row_index, int B, fl
 int wsr_step_counter_add(int* t_dev, int delta, void* stream);
 /* Standard normal fill with the same Philox stream layout as wsr_sampler_step (counter word = `tag`). */
 int wsr_randn(float* out, int64_t n, uint64_t seed, uint32_t tag, void* stream);
+int wsr_randn_members(float* out, int64_t n, const uint64_t* member_keys, int64_t member_elems, uint32_t tag, void* stream);
 /* q_sample (diffusion.py:209-228): x_noisy = a[b]*(hr-sr) + sqrt(1-a[b]^2)*noise, per-sample a; fp32 NCHW. */
 int wsr_q_sample(const float* hr, const float* sr, const float* noise, const float* a, int B, int64_t per_sample,
                  float* x_noisy, void* stream);

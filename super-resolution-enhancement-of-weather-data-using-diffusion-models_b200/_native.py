@@ -132,16 +132,21 @@ SIGNATURES = {
     "wsr_bicubic_upsample": [_P, _I, _I, _I, _I, _P, _P],
     "wsr_standard_scale": [_P, _I, _L, _P, _P, _I, _P, _P],
     "wsr_error_sums": [_P, _P, _I, _L, _P, _P, _P],
+    "wsr_ensemble_stats": [_P, _I, _L, _P, _I, _L, _P, _P, _P, _P, _P, _P],
     "wsr_image_compare_loss": [_P, _P, _I, _I, _I, _F, _F, _P, _P, _P],
     "wsr_relu_mask": [_P, _P, _L, _P],
     "wsr_lrelu_mask": [_P, _I, _I, _P, _I, _I, _L, _I, _F, _P],
     "wsr_sampler_step": [_P, _P, _I, _P, _L, _U64, _P, _I, _P, _I, _P, _L, _P],
     "wsr_final_conv_sampler_step": [_P, _I, _I, _I, _I, _I, _P, _I, _P, _P, _I, _F, _P, _P, _I, _P, _P, _P, _L, _U64, _P, _I, _P, _I, _P],
+    "wsr_sampler_step_members": [_P, _P, _I, _P, _L, _P, _L, _P, _I, _P, _I, _P, _L, _P],
+    "wsr_final_conv_sampler_step_members": [_P, _I, _I, _I, _I, _I, _P, _I, _P, _P, _I, _F, _P, _P, _I, _P, _P, _P, _L, _P, _L, _P, _I, _P,
+                                            _I, _P],
     "wsr_head_sampler_supported": [_I, _I, _I],
     "wsr_pack_head_weight": [_P, _I, _I, _P, _P],
     "wsr_broadcast_row": [_P, _I, _P, _I, _P, _P],
     "wsr_step_counter_add": [_P, _I, _P],
     "wsr_randn": [_P, _L, _U64, _U32, _P],
+    "wsr_randn_members": [_P, _L, _P, _L, _U32, _P],
     "wsr_q_sample": [_P, _P, _P, _P, _I, _L, _P, _P],
     "wsr_noise_loss": [_P, _P, _L, _I, _P, _P, _F, _P],
     # training step (backward.cu, fd.cu)

@@ -500,9 +500,25 @@ __device__ __forceinline__ void randn4(uint64_t seed, uint32_t tag, uint64_t grp
   z[0] = r0 * c0; z[1] = r0 * s0; z[2] = r1 * c1; z[3] = r1 * s1;
 }
 
+// Philox key and member-local group of the 4-element group g: the plain stream (key = seed, group g), or the member-keyed stream of
+// an ensemble batch (member m = g / member_groups draws from key member_keys[m] at group g - m * member_groups), so that member m's
+// slice is exactly the plain stream of key member_keys[m] over that slice alone.
+template <bool MK>
+__device__ __forceinline__ uint64_t noise_key(uint64_t seed, const uint64_t* __restrict__ member_keys, int64_t member_groups, int64_t& g) {
+  if constexpr (MK) {
+    const int64_t m = g / member_groups;
+    g -= m * member_groups;
+    return __ldg((const unsigned long long*)member_keys + m);
+  } else {
+    (void)member_keys; (void)member_groups;
+    return seed;
+  }
+}
+
+template <bool MK>
 __global__ void sampler_step_kernel(const float* x, const void* eps, int edt, const float* __restrict__ z, int64_t z_stride,
-                                    uint64_t seed, const float* __restrict__ tab, int T, const int* __restrict__ t_dev,
-                                    int clip, float* xo, int64_t n) {
+                                    uint64_t seed, const uint64_t* __restrict__ member_keys, int64_t member_groups,
+                                    const float* __restrict__ tab, int T, const int* __restrict__ t_dev, int clip, float* xo, int64_t n) {
   const int t = *t_dev;
   if (z) z += (int64_t)(T - t) * z_stride;
   const float c_recip = tab[t], c_recipm1 = tab[T + t], coef1 = tab[2 * T + t], coef2 = tab[3 * T + t];
@@ -516,7 +532,9 @@ __global__ void sampler_step_kernel(const float* x, const void* eps, int edt, co
 #pragma unroll
       for (int j = 0; j < 4; ++j) if (i0 + j < n) zz[j] = z[i0 + j];
     } else {
-      randn4(seed, (uint32_t)t, (uint64_t)g, zz);
+      int64_t lg = g;
+      const uint64_t key = noise_key<MK>(seed, member_keys, member_groups, lg);
+      randn4(key, (uint32_t)t, (uint64_t)lg, zz);
     }
   }
 #pragma unroll
@@ -539,11 +557,15 @@ __global__ void broadcast_row_kernel(const float* __restrict__ table, int P, con
   if (i < P) dst[i] = src[i];
 }
 
-__global__ void randn_kernel(float* out, int64_t n, uint64_t seed, uint32_t tag) {
+template <bool MK>
+__global__ void randn_kernel(float* out, int64_t n, uint64_t seed, const uint64_t* __restrict__ member_keys, int64_t member_groups,
+                             uint32_t tag) {
   int64_t g = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (g * 4 >= n) return;
   float z[4];
-  randn4(seed, tag, (uint64_t)g, z);
+  int64_t lg = g;
+  const uint64_t key = noise_key<MK>(seed, member_keys, member_groups, lg);
+  randn4(key, tag, (uint64_t)lg, z);
 #pragma unroll
   for (int j = 0; j < 4; ++j) if (g * 4 + j < n) out[g * 4 + j] = z[j];
 }
@@ -817,7 +839,21 @@ extern "C" int wsr_sampler_step(const float* x, const void* eps, int eps_dtype, 
                                 uint64_t seed, const float* tables, int T, const int* t_dev, int clip, float* x_out,
                                 int64_t n, void* stream) {
   WSR_REQUIRE(x && eps && tables && t_dev && x_out && valid_dtype(eps_dtype) && T > 0 && n > 0, WSR_E_INVALID, "sampler_step: bad argument");
-  sampler_step_kernel<<<blocks_for((n + 3) / 4, 256), 256, 0, (cudaStream_t)stream>>>(x, eps, eps_dtype, z, z_step_stride, seed, tables, T, t_dev, clip, x_out, n);
+  sampler_step_kernel<false><<<blocks_for((n + 3) / 4, 256), 256, 0, (cudaStream_t)stream>>>(x, eps, eps_dtype, z, z_step_stride, seed, nullptr, 1,
+                                                                                              tables, T, t_dev, clip, x_out, n);
+  WSR_LAUNCH_OK();
+  return WSR_OK;
+}
+
+extern "C" int wsr_sampler_step_members(const float* x, const void* eps, int eps_dtype, const float* z, int64_t z_step_stride,
+                                        const uint64_t* member_keys, int64_t member_elems, const float* tables, int T, const int* t_dev,
+                                        int clip, float* x_out, int64_t n, void* stream) {
+  WSR_REQUIRE(x && eps && tables && t_dev && x_out && member_keys && valid_dtype(eps_dtype) && T > 0 && n > 0, WSR_E_INVALID,
+              "sampler_step_members: bad argument");
+  WSR_REQUIRE(member_elems > 0 && member_elems % 4 == 0, WSR_E_INVALID, "sampler_step_members: member_elems=%lld is not a positive multiple of 4",
+              (long long)member_elems);
+  sampler_step_kernel<true><<<blocks_for((n + 3) / 4, 256), 256, 0, (cudaStream_t)stream>>>(x, eps, eps_dtype, z, z_step_stride, 0, member_keys,
+                                                                                             member_elems / 4, tables, T, t_dev, clip, x_out, n);
   WSR_LAUNCH_OK();
   return WSR_OK;
 }
@@ -831,7 +867,16 @@ extern "C" int wsr_step_counter_add(int* t_dev, int delta, void* stream) {
 
 extern "C" int wsr_randn(float* out, int64_t n, uint64_t seed, uint32_t tag, void* stream) {
   WSR_REQUIRE(out && n > 0, WSR_E_INVALID, "randn: bad argument");
-  randn_kernel<<<blocks_for((n + 3) / 4, 256), 256, 0, (cudaStream_t)stream>>>(out, n, seed, tag);
+  randn_kernel<false><<<blocks_for((n + 3) / 4, 256), 256, 0, (cudaStream_t)stream>>>(out, n, seed, nullptr, 1, tag);
+  WSR_LAUNCH_OK();
+  return WSR_OK;
+}
+
+extern "C" int wsr_randn_members(float* out, int64_t n, const uint64_t* member_keys, int64_t member_elems, uint32_t tag, void* stream) {
+  WSR_REQUIRE(out && member_keys && n > 0, WSR_E_INVALID, "randn_members: bad argument");
+  WSR_REQUIRE(member_elems > 0 && member_elems % 4 == 0, WSR_E_INVALID, "randn_members: member_elems=%lld is not a positive multiple of 4",
+              (long long)member_elems);
+  randn_kernel<true><<<blocks_for((n + 3) / 4, 256), 256, 0, (cudaStream_t)stream>>>(out, n, 0, member_keys, member_elems / 4, tag);
   WSR_LAUNCH_OK();
   return WSR_OK;
 }

@@ -28,6 +28,7 @@ struct HeadParams {
   float* eps_out;                          // fp32 NCHW (B, Cout, H, W) or null
   float* xs;                               // fp32 NCHW state x_t -> x_{t-1} in place, or null (convolution only)
   const float* z; long long z_stride; unsigned long long seed; const float* tab; int T; const int* t_dev; int clip;
+  const unsigned long long* member_keys; long long member_groups;   // ensemble batch (MK): per-member Philox keys, member elements / 4
 };
 
 __device__ __forceinline__ void head_randn4(uint64_t seed, uint32_t tag, uint64_t grp, float (&z)[4]) {
@@ -46,7 +47,7 @@ __device__ __forceinline__ void head_randn4(uint64_t seed, uint32_t tag, uint64_
 
 // shared memory: tile [Cin/64 planes][6 rows][130 cols][64 ch] bf16 | weights bf16 as ldmatrix-ready 8x8 blocks
 // [plane][tap][16-channel step][k half][n = 8 output channels (zero above Cout)][8 channels] | scale[Cin] shift[Cin] | group moments
-template <int COUT>
+template <int COUT, bool MK>
 __global__ void __launch_bounds__(kHeadThreads) head_sampler_kernel(const HeadParams p) {
   extern __shared__ __align__(16) uint8_t hsm[];
   constexpr int TR = kHeadRows + 2, TC = kHeadCols + 2;
@@ -226,7 +227,17 @@ __global__ void __launch_bounds__(kHeadThreads) head_sampler_kernel(const HeadPa
         float zz = 0.f;
         if (t > 0) {
           if (zt) zz = zt[i];
-          else { float z4[4]; head_randn4(p.seed, (uint32_t)t, (uint64_t)(i >> 2), z4); const int wsel = (int)(i & 3); zz = wsel == 0 ? z4[0] : wsel == 1 ? z4[1] : wsel == 2 ? z4[2] : z4[3]; }
+          else {
+            // MK: member m = group / member_groups draws from its own key at the member-local group (wsr_sampler_step_members)
+            long long grp = i >> 2;
+            unsigned long long key = p.seed;
+            if constexpr (MK) {
+              const long long m = grp / p.member_groups;
+              grp -= m * p.member_groups;
+              key = __ldg(p.member_keys + m);
+            }
+            float z4[4]; head_randn4(key, (uint32_t)t, (uint64_t)grp, z4); const int wsel = (int)(i & 3); zz = wsel == 0 ? z4[0] : wsel == 1 ? z4[1] : wsel == 2 ? z4[2] : z4[3];
+          }
         }
         const float xv = p.xs[i];
         float x0v = c_recip * xv - c_recipm1 * e;
@@ -251,16 +262,16 @@ static size_t head_smem_bytes(int Cin, int Cout, int groups) {
   return (size_t)(Cin / 64) * (kHeadRows + 2) * (kHeadCols + 2) * 128 + (size_t)(Cin / 64) * 9 * 4 * 2 * 128 + (size_t)(2 * Cin + 2 * groups) * 4;
 }
 
-template <int COUT>
+template <int COUT, bool MK>
 static int launch_head(const HeadParams& p, cudaStream_t st) {
   const size_t smem = head_smem_bytes(p.Cin, COUT, p.groups);
   static size_t attr = 0;
   if (smem > attr) {
-    WSR_CUDA_OK(cudaFuncSetAttribute(head_sampler_kernel<COUT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    WSR_CUDA_OK(cudaFuncSetAttribute(head_sampler_kernel<COUT, MK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     attr = smem;
   }
   const int tiles = ((p.W + kHeadCols - 1) / kHeadCols) * ((p.H + kHeadRows - 1) / kHeadRows);
-  WSR_CUDA_OK(launch_pdl(head_sampler_kernel<COUT>, dim3(tiles, p.B), dim3(kHeadThreads), smem, st, p));
+  WSR_CUDA_OK(launch_pdl(head_sampler_kernel<COUT, MK>, dim3(tiles, p.B), dim3(kHeadThreads), smem, st, p));
   return WSR_OK;
 }
 
@@ -281,11 +292,11 @@ extern "C" int wsr_pack_head_weight(const float* w, int Cout, int Cin, void* dst
   return WSR_OK;
 }
 
-extern "C" int wsr_final_conv_sampler_step(const void* x, int x_ld, int B, int H, int W, int Cin, const double* stats, int stats_ld,
-                                           const float* gamma, const float* beta, int groups, float gn_eps, const void* w,
-                                           const float* bias, int Cout, float* eps_out, float* x_state, const float* z,
-                                           int64_t z_step_stride, uint64_t seed, const float* tables, int T, const int* t_dev,
-                                           int clip, void* stream) {
+static int head_sampler_step(const void* x, int x_ld, int B, int H, int W, int Cin, const double* stats, int stats_ld,
+                             const float* gamma, const float* beta, int groups, float gn_eps, const void* w, const float* bias, int Cout,
+                             float* eps_out, float* x_state, const float* z, int64_t z_step_stride, uint64_t seed,
+                             const uint64_t* member_keys, int64_t member_elems, const float* tables, int T, const int* t_dev, int clip,
+                             void* stream) {
   WSR_REQUIRE(x && stats && gamma && beta && w, WSR_E_INVALID, "final_conv_sampler_step: null pointer");
   WSR_REQUIRE(B > 0 && B <= 65535 && H > 0 && W > 0, WSR_E_INVALID, "final_conv_sampler_step: bad shape");
   WSR_REQUIRE(wsr_head_sampler_supported(Cin, Cout, groups), WSR_E_UNSUPPORTED,
@@ -299,11 +310,42 @@ extern "C" int wsr_final_conv_sampler_step(const void* x, int x_ld, int B, int H
   p.stats = stats; p.stats_ld = stats_ld; p.gamma = gamma; p.beta = beta; p.groups = groups; p.gn_eps = gn_eps;
   p.w = (const uint4*)w; p.bias = bias; p.eps_out = eps_out; p.xs = x_state; p.z = z; p.z_stride = z_step_stride; p.seed = seed;
   p.tab = tables; p.T = T; p.t_dev = t_dev; p.clip = clip;
+  p.member_keys = (const unsigned long long*)member_keys; p.member_groups = member_elems / 4;
   cudaStream_t st = (cudaStream_t)stream;
-  switch (Cout) {
-    case 1: return launch_head<1>(p, st);
-    case 2: return launch_head<2>(p, st);
-    case 3: return launch_head<3>(p, st);
-    default: return launch_head<4>(p, st);
+  if (member_keys) {
+    switch (Cout) {
+      case 1: return launch_head<1, true>(p, st);
+      case 2: return launch_head<2, true>(p, st);
+      case 3: return launch_head<3, true>(p, st);
+      default: return launch_head<4, true>(p, st);
+    }
   }
+  switch (Cout) {
+    case 1: return launch_head<1, false>(p, st);
+    case 2: return launch_head<2, false>(p, st);
+    case 3: return launch_head<3, false>(p, st);
+    default: return launch_head<4, false>(p, st);
+  }
+}
+
+extern "C" int wsr_final_conv_sampler_step(const void* x, int x_ld, int B, int H, int W, int Cin, const double* stats, int stats_ld,
+                                           const float* gamma, const float* beta, int groups, float gn_eps, const void* w,
+                                           const float* bias, int Cout, float* eps_out, float* x_state, const float* z,
+                                           int64_t z_step_stride, uint64_t seed, const float* tables, int T, const int* t_dev,
+                                           int clip, void* stream) {
+  return head_sampler_step(x, x_ld, B, H, W, Cin, stats, stats_ld, gamma, beta, groups, gn_eps, w, bias, Cout, eps_out, x_state, z,
+                           z_step_stride, seed, nullptr, 0, tables, T, t_dev, clip, stream);
+}
+
+extern "C" int wsr_final_conv_sampler_step_members(const void* x, int x_ld, int B, int H, int W, int Cin, const double* stats,
+                                                   int stats_ld, const float* gamma, const float* beta, int groups, float gn_eps,
+                                                   const void* w, const float* bias, int Cout, float* eps_out, float* x_state,
+                                                   const float* z, int64_t z_step_stride, const uint64_t* member_keys,
+                                                   int64_t member_elems, const float* tables, int T, const int* t_dev, int clip,
+                                                   void* stream) {
+  WSR_REQUIRE(member_keys, WSR_E_INVALID, "final_conv_sampler_step_members: null member_keys");
+  WSR_REQUIRE(member_elems > 0 && member_elems % 4 == 0, WSR_E_INVALID,
+              "final_conv_sampler_step_members: member_elems=%lld is not a positive multiple of 4", (long long)member_elems);
+  return head_sampler_step(x, x_ld, B, H, W, Cin, stats, stats_ld, gamma, beta, groups, gn_eps, w, bias, Cout, eps_out, x_state, z,
+                           z_step_stride, 0, member_keys, member_elems, tables, T, t_dev, clip, stream);
 }

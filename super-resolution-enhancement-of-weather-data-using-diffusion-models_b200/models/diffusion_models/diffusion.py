@@ -35,6 +35,19 @@ def rank_stream_seed(seed, rank=None):
     return (z ^ (z >> 31)) & ((1 << 62) - 1)
 
 
+def member_key(seed, m):
+    """Philox key of ensemble member m: the splitmix derivation of ``rank_stream_seed`` with the member index in place of the rank.
+    Member 0 keeps ``seed`` (it is the single-GPU ``super_resolution`` run with that seed), and the key never depends on the rank,
+    the chunking or the batch a member is sampled in."""
+    return rank_stream_seed(seed, int(m))
+
+
+def ensemble_chunks(n_members, batch, max_images=64, member_offset=0):
+    """Member ranges [(first member, count)] sampled together: whole members, R = max(1, max_images // batch) per chunk."""
+    per = max(1, int(max_images) // int(batch))
+    return [(member_offset + c, min(per, n_members - c)) for c in range(0, int(n_members), per)]
+
+
 class GaussianDiffusion(nn.Module):
     def __init__(self, denoise_fn, channels=1, loss_type='l1', conditional=True, schedule_opt=None, image_height=128,
                  image_width=256, pretrained_model_path=None, lock_weights=True):
@@ -128,32 +141,40 @@ class GaussianDiffusion(nn.Module):
         self._step(plan, xb, t_dev, tab, None, 0, self._next_seed(), clip_denoised)
         return xb
 
-    def _step(self, plan, x, t_dev, tab, z, z_stride, seed, clip=True):
+    def _step(self, plan, x, t_dev, tab, z, z_stride, seed, clip=True, members=None):
+        """members: None, or (device int64 key table, elements per member) -- an ensemble batch with member-keyed noise."""
         st = plan.eng.stream
         plan.select_level_row(t_dev)
         if plan.can_fuse_head():
             # head (GroupNorm + Swish + conv3x3) and the reverse-step update in one HBM-bound kernel
             feat = plan.run(x, head=False)
-            plan.head_sampler_step(feat, x, tab, self.num_timesteps, t_dev, z, z_stride, seed, clip)
+            plan.head_sampler_step(feat, x, tab, self.num_timesteps, t_dev, z, z_stride, seed, clip, members=members)
             plan.eng.call("wsr_step_counter_add", t_dev.data_ptr(), -1, st)
             return
         plan.run(x)
-        plan.eng.call("wsr_sampler_step", x.data_ptr(), plan.eps.data_ptr(), nat.F32, 0 if z is None else z.data_ptr(),
-                      z_stride, seed, tab.data_ptr(), self.num_timesteps, t_dev.data_ptr(), 1 if clip else 0, x.data_ptr(),
-                      x.numel(), st, nbytes=x.numel() * (16 if z is not None else 12))
+        zp = 0 if z is None else z.data_ptr()
+        if members is None:
+            plan.eng.call("wsr_sampler_step", x.data_ptr(), plan.eps.data_ptr(), nat.F32, zp, z_stride, seed, tab.data_ptr(),
+                          self.num_timesteps, t_dev.data_ptr(), 1 if clip else 0, x.data_ptr(), x.numel(), st,
+                          nbytes=x.numel() * (16 if z is not None else 12))
+        else:
+            plan.eng.call("wsr_sampler_step_members", x.data_ptr(), plan.eps.data_ptr(), nat.F32, zp, z_stride, members[0].data_ptr(),
+                          members[1], tab.data_ptr(), self.num_timesteps, t_dev.data_ptr(), 1 if clip else 0, x.data_ptr(), x.numel(),
+                          st, nbytes=x.numel() * (16 if z is not None else 12))
         plan.eng.call("wsr_step_counter_add", t_dev.data_ptr(), -1, st)
 
     @torch.no_grad()
-    def begin_loop(self, plan, shape, noise_chain=None, seed=None):
+    def begin_loop(self, plan, shape, noise_chain=None, seed=None, member_keys=None):
         """Set up a reverse loop on the plan's current condition and return its state object (see ReverseLoop)."""
-        return ReverseLoop(self, plan, shape, noise_chain, seed)
+        return ReverseLoop(self, plan, shape, noise_chain, seed, member_keys)
 
     @torch.no_grad()
-    def _reverse_loop(self, plan, shape, noise_chain=None, seed=None, steps=None, collect_eps=False):
+    def _reverse_loop(self, plan, shape, noise_chain=None, seed=None, steps=None, collect_eps=False, member_keys=None):
         """T reverse steps on the plan's current condition.  noise_chain: optional injected noise [T+1, *shape]
-        (index 0 = initial image, index T-t = noise of step t) for parity runs; otherwise Philox noise from ``seed``.
+        (index 0 = initial image, index T-t = noise of step t) for parity runs; otherwise Philox noise from ``seed``, or, with
+        ``member_keys`` (R Philox keys), from key member_keys[m] for the m-th of R equal member slices of the batch.
         Returns the final x_0 (fp32 NCHW)."""
-        loop = self.begin_loop(plan, shape, noise_chain, seed)
+        loop = self.begin_loop(plan, shape, noise_chain, seed, member_keys)
         n_steps = self.num_timesteps if steps is None else min(int(steps), self.num_timesteps)
         eps_log = []
         # first step eagerly (lazy initialisation of kernel attributes happens here), the rest as graph replays
@@ -173,6 +194,43 @@ class GaussianDiffusion(nn.Module):
         if collect_eps:
             return loop.x, eps_log
         return loop.x
+
+    def _ensemble_condition(self, x_in):
+        """Hook of ``super_resolution_ensemble``: (condition tensor for the plan, field added to every member at the end or None).
+        ResDiff / PhyDiff: the condition is x_in['SR'] and the sampler returns image + SR."""
+        sr = x_in["SR"].to(device=self.betas.device, dtype=torch.float32)
+        return sr, sr
+
+    @torch.no_grad()
+    def super_resolution_ensemble(self, x_in, n_members, seed=None, member_offset=0, max_images=64):
+        """``n_members`` samples per condition: (n_members, B, C, H, W) fp32.  Member k is global member member_offset + k, whose
+        noise is Philox key ``member_key(seed, member_offset + k)``: it equals ``p_sample_loop`` on the B conditions with that seed,
+        independently of the chunking and of ``member_offset``.  Members run in chunks of R = max(1, max_images // B) whole members;
+        a chunk is one reverse loop over R * B images whose condition-only work runs once on the B conditions
+        (``UNetPlan.set_condition(cond, repeats=R)``)."""
+        if not self.conditional:
+            raise NotImplementedError("unconditional sampling is not part of the accelerated path")
+        n_members = int(n_members)
+        if n_members < 1:
+            raise ValueError("n_members must be >= 1")
+        dev = self.betas.device
+        shape = tuple(x_in["SR"].shape)
+        B = shape[0]
+        base = int(seed) if seed is not None else (int(self.sample_seed) if self.sample_seed is not None
+                                                   else int(torch.randint(0, 2 ** 62, (1,)).item()))
+        cond, add = self._ensemble_condition(x_in)
+        out = torch.empty((n_members,) + shape, device=dev, dtype=torch.float32)
+        for first, r in ensemble_chunks(n_members, B, max_images, member_offset):
+            plan = self._plan(r * B, dev)
+            plan.set_condition(cond, repeats=r)
+            keys = torch.tensor([member_key(base, first + k) for k in range(r)], dtype=torch.int64).to(dev)
+            img = self._reverse_loop(plan, (r * B,) + shape[1:], member_keys=keys)
+            k0 = first - member_offset
+            dst = out[k0:k0 + r]
+            dst.copy_(img.view((r,) + shape))
+            if add is not None:
+                dst.add_(add.unsqueeze(0))
+        return out
 
     @torch.no_grad()
     def sample(self, batch_size=1, continous=False):
@@ -218,7 +276,7 @@ class ReverseLoop:
     captured CUDA graph of one step.  ``step()`` launches one step eagerly, ``capture()`` records the same launches
     into a graph, ``replay()`` replays it -- the step index lives on the device, so every replay advances the chain."""
 
-    def __init__(self, diffusion, plan, shape, noise_chain=None, seed=None):
+    def __init__(self, diffusion, plan, shape, noise_chain=None, seed=None, member_keys=None):
         self.diffusion, self.plan = diffusion, plan
         dev = plan.eng.device
         T = diffusion.num_timesteps
@@ -227,6 +285,15 @@ class ReverseLoop:
         self.x = torch.empty(shape, device=dev, dtype=torch.float32)
         # an explicit seed is still made rank-distinct: sharded ranks pass the same value (bench.py, sample.py)
         self.seed = diffusion._next_seed() if seed is None else rank_stream_seed(int(seed))
+        self.members = None
+        if member_keys is not None:
+            # ensemble batch: R equal member slices, each keyed by its own entry of the (constant, graph-safe) device key table
+            keys = member_keys.to(device=dev, dtype=torch.int64).contiguous()
+            n = 1
+            for d in shape:
+                n *= int(d)
+            assert n % keys.numel() == 0
+            self.members = (keys, n // keys.numel())
         if noise_chain is not None:
             self.z = noise_chain.to(device=dev, dtype=torch.float32).contiguous()
             assert self.z.shape[0] == T + 1 and tuple(self.z.shape[1:]) == tuple(shape)
@@ -234,7 +301,11 @@ class ReverseLoop:
             self.z_stride = self.x.numel()
         else:
             self.z, self.z_stride = None, 0
-            nat.call("wsr_randn", self.x.data_ptr(), self.x.numel(), self.seed, 0xFFFFFFFF, plan.eng.stream)
+            if self.members is None:
+                nat.call("wsr_randn", self.x.data_ptr(), self.x.numel(), self.seed, 0xFFFFFFFF, plan.eng.stream)
+            else:
+                nat.call("wsr_randn_members", self.x.data_ptr(), self.x.numel(), self.members[0].data_ptr(), self.members[1],
+                         0xFFFFFFFF, plan.eng.stream)
         self.t_dev = torch.tensor([T - 1], dtype=torch.int32, device=dev)
         self.graph = None
 
@@ -242,7 +313,7 @@ class ReverseLoop:
         self.t_dev.fill_(self.diffusion.num_timesteps - 1 if t is None else int(t))
 
     def step(self):
-        self.diffusion._step(self.plan, self.x, self.t_dev, self.tab, self.z, self.z_stride, self.seed)
+        self.diffusion._step(self.plan, self.x, self.t_dev, self.tab, self.z, self.z_stride, self.seed, members=self.members)
 
     def capture(self):
         torch.cuda.synchronize(self.plan.eng.device)

@@ -117,6 +117,14 @@ class DDPM(BaseModel):
             self.SR = self.SR.unsqueeze(0) if len(self.SR.size()) == 3 else self.SR
         self.netG.train()
 
+    def generate_ensemble(self, n_members, seed=None, member_offset=0):
+        """self.ENS = (n_members, B, C, H, W): members member_offset .. member_offset + n_members - 1 of the ensemble of ``seed``
+        for the fed batch (GaussianDiffusion.super_resolution_ensemble).  SR is left untouched."""
+        self.netG.eval()
+        with torch.no_grad():
+            self.ENS = self._net().super_resolution_ensemble(self.data, n_members, seed=seed, member_offset=member_offset)
+        self.netG.train()
+
     def sample(self, batch_size=1, continous=False):
         self.netG.eval()
         with torch.no_grad():

@@ -29,6 +29,10 @@ class SR3Diffusion(GaussianDiffusion):
     def super_resolution(self, x_in, continous=False):
         return self.p_sample_loop(x_in["SR"], continous)
 
+    def _ensemble_condition(self, x_in):
+        """SR3 returns the final image itself: nothing is added back."""
+        return x_in["SR"].to(device=self.betas.device, dtype=torch.float32), None
+
     def p_losses(self, x_in, noise=None):
         """reference :101-137: x_start = HR, one t per batch, per-sample continuous level, sum-reduced loss."""
         hr, sr = x_in['HR'], x_in['SR']

@@ -56,6 +56,11 @@ class SRDiffDiffusion(GaussianDiffusion):
     def super_resolution(self, x_in, continous=False):
         return self.p_sample_loop(x_in, continous)
 
+    def _ensemble_condition(self, x_in):
+        """The RRDB encoder runs once on the B LR fields; every member adds back the bicubic SR."""
+        dev = self.betas.device
+        return self._condition(x_in['LR'].to(dev)), x_in['SR'].to(device=dev, dtype=torch.float32)
+
     @torch.no_grad()
     def p_sample(self, x, t, clip_denoised=True, condition_x=None):
         """condition_x: the list of 18 RRDB feature maps (reference :133-159)."""

@@ -2,11 +2,18 @@
 
     python sample.py -c CONFIG.json -p MODEL_PATH -o OUT_DIR -gpu 0 [-n N]
     torchrun --nproc-per-node 8 sample.py -c CONFIG.json -o OUT_DIR -gpu 0,1,2,3,4,5,6,7     # batch-sharded
+    python sample.py -c CONFIG.json -o OUT_DIR --ensemble 16 [--seed S]                      # 16 members per condition
 
 Builds the model through the reference's registry path (Config -> create_model -> DDPM -> define_diffusion),
 ``prepare_to_eval``, ``feed_data``, ``generate_sr``; writes the super-resolved fields as ``sr.npy`` (the reference's
 cartopy plots, training/visualization.py, are outside the accelerated path).  ``-p`` may be omitted to sample from
-random-init weights (smoke / benchmarking)."""
+random-init weights (smoke / benchmarking).
+
+``--ensemble N`` samples N members per condition instead (``DDPM.generate_ensemble``) and writes ``ensemble.npy`` (N, B, C, H, W),
+``ensemble_mean.npy`` and ``ensemble_spread.npy`` (unbiased), their ``*_physical.npy`` versions with a store, and, when the batch
+carries HR, ``ensemble_scores.json`` (training.metrics.EnsembleScores; physical units with a store).  Under torchrun the MEMBERS are
+sharded (rank r runs a contiguous member range) and rank 0 gathers them; the condition batch is not split.  ``--seed S`` fixes the
+Philox seed (member m uses member_key(S, m); member 0 is the plain run with seed S)."""
 import argparse
 import os
 import sys
@@ -29,6 +36,8 @@ def main(argv=None):
     ap.add_argument("-t", "--image_types", nargs="+", default=["SR"], choices=["HR", "SR", "LR", "INTERPOLATED", "DELTA", "AE"])
     ap.add_argument("-m", "--color_map", type=str, default="coolwarm", choices=["coolwarm", "heat_muted"])
     ap.add_argument("-d", "--date", type=str, default=None)
+    ap.add_argument("--ensemble", type=int, default=None, help="members per condition (ensemble sampling)")
+    ap.add_argument("--seed", type=int, default=None, help="Philox seed of the sampler")
     args = ap.parse_args(argv)
 
     Config = wsr.sub("configs.config").Config
@@ -66,6 +75,13 @@ def main(argv=None):
         batch, months = handler.get_data_by_date(args.date)
     else:
         batch, months = next(iter(data.batches_from_opt(opt, "val")))
+    if args.seed is not None:
+        model._net().sample_seed = args.seed
+    if args.ensemble is not None:
+        _ensemble(args, model, batch, months, handler, par, rank, world)
+        if world > 1:
+            torch.distributed.destroy_process_group()
+        return
     n_total = batch["SR"].shape[0]
     if world > 1:
         batch = par.shard_batch(batch, rank, world)
@@ -83,6 +99,44 @@ def main(argv=None):
             np.save(os.path.join(args.output_path, "sr_physical.npy"), phys["SR"].float().cpu().numpy())
     if world > 1:
         torch.distributed.destroy_process_group()
+
+
+def _ensemble(args, model, batch, months, handler, par, rank, world):
+    n = int(args.ensemble)
+    if n < 1:
+        raise SystemExit("--ensemble needs at least one member")
+    lo, hi = par.shard_bounds(n, rank, world)
+    model.feed_data((batch, months))
+    model.generate_ensemble(hi - lo, seed=args.seed, member_offset=lo)
+    ens = model.ENS
+    if world > 1:
+        ens = par.gather_batch(ens, n)
+    if rank != 0:
+        return
+    import json
+    out = args.output_path
+    os.makedirs(out, exist_ok=True)
+    spread = ens.std(0, unbiased=True) if n > 1 else torch.zeros_like(ens[0])
+    arrays = {"ensemble": ens, "ensemble_mean": ens.mean(0), "ensemble_spread": spread}
+    hr = batch.get("HR") if isinstance(batch, dict) else None
+    target = None if hr is None else hr.to(device=ens.device, dtype=torch.float32)
+    if handler is not None:
+        tr = handler.get_data_transformer()
+        ms = months[:ens.shape[1]] if len(months) >= ens.shape[1] else months
+        phys = torch.stack([tr.inverse_transform({"SR": m}, ms)["SR"].float() for m in ens], 0)
+        arrays.update({"ensemble_physical": phys, "ensemble_mean_physical": phys.mean(0),
+                       "ensemble_spread_physical": phys.std(0, unbiased=True) if n > 1 else torch.zeros_like(phys[0])})
+        if target is not None:
+            target = tr.inverse_transform({"HR": target}, ms)["HR"].float()
+            ens = phys
+    for name, a in arrays.items():
+        np.save(os.path.join(out, name + ".npy"), a.float().cpu().numpy())
+    print("saved %s %s" % (os.path.join(out, "ensemble.npy"), tuple(arrays["ensemble"].shape)))
+    if target is not None and n > 1:
+        scores = wsr.sub("training.metrics").EnsembleScores(ens.device)
+        scores.update(ens, target)
+        with open(os.path.join(out, "ensemble_scores.json"), "w") as fh:
+            json.dump(scores.compute(), fh, indent=1)
 
 
 if __name__ == "__main__":

@@ -128,3 +128,75 @@ class ValidationMetrics:
         for metric, value in self.metrics.items():
             message = f"{message}  |  {metric:s}: {float(value):.5f}"
         return message
+
+
+class EnsembleScores:
+    """Probabilistic scores of ensembles against their targets: per-plane double accumulators and rank histograms on the device,
+    filled by one ``wsr_ensemble_stats`` launch per ``update``; the host synchronises only in ``compute``.
+
+    ``update(ensemble, target, scale=None)``: ensemble (N, B, C, H, W), target (B, C, H, W); ``scale`` = std per variable (C values) or
+    per plane (B * C values) puts every score in physical units (the inverse StandardScaling; the means cancel in differences).
+    ``compute()`` returns, per variable (lists of C values) and over all variables ("overall"): CRPS (standard, 1/(2N^2) pairwise
+    term) and fair CRPS (1/(2N(N-1))), the RMSE of the ensemble mean, the mean spread sqrt(mean unbiased variance), the spread-skill
+    ratio sqrt((N+1)/N) * spread / RMSE and the rank histogram normalised to sum 1 (rank = members strictly below the target)."""
+
+    def __init__(self, device=None):
+        self.device = torch.device(device if device is not None else "cuda")
+        if self.device.type != "cuda":
+            raise nat.WsrError("metric accumulators run on the CUDA path only (got device %s)" % self.device)
+        self.reset()
+
+    def reset(self):
+        self.N = self.C = None
+        self.acc = self.hist = None
+        self.pixels = 0              # pixels per variable seen so far
+
+    def update(self, ensemble, target, scale=None):
+        ens = ensemble.to(device=self.device, dtype=torch.float32).contiguous()
+        tgt = target.to(device=self.device, dtype=torch.float32).contiguous()
+        N, B, C, H, W = ens.shape
+        assert tuple(tgt.shape) == (B, C, H, W), (tuple(ens.shape), tuple(tgt.shape))
+        if self.N is None:
+            self.N, self.C = N, C
+            self.acc = torch.zeros((C, 5), dtype=torch.float64, device=self.device)
+            self.hist = torch.zeros((C, N + 1), dtype=torch.int64, device=self.device)
+        assert (N, C) == (self.N, self.C), "every update of one EnsembleScores needs the same member and variable count"
+        planes = B * C
+        sp = 0
+        if scale is not None:
+            sc = scale.to(device=self.device, dtype=torch.float32).reshape(-1)
+            if sc.numel() == C:
+                sc = sc.repeat(B)
+            assert sc.numel() == planes
+            sc = sc.contiguous()
+            sp = sc.data_ptr()
+        acc = torch.zeros((planes, 5), dtype=torch.float64, device=self.device)
+        hist = torch.zeros((planes, N + 1), dtype=torch.int64, device=self.device)
+        nat.call("wsr_ensemble_stats", ens.data_ptr(), N, planes * H * W, tgt.data_ptr(), planes, H * W, sp, 0, 0, acc.data_ptr(),
+                 hist.data_ptr(), torch.cuda.current_stream(self.device).cuda_stream)
+        self.acc += acc.view(B, C, 5).sum(0)
+        self.hist += hist.view(B, C, N + 1).sum(0)
+        self.pixels += B * H * W
+        self._keep = (ens, tgt, sc if scale is not None else None, acc, hist)
+
+    def compute(self):
+        if self.N is None or self.pixels == 0:
+            return {}
+        N = self.N
+        acc = self.acc.cpu().double()
+        hist = self.hist.cpu().double()
+
+        def scores(a, h, n):
+            crps = a[0] / n - a[1] / (2.0 * N * N * n)
+            fair = a[0] / n - a[1] / (2.0 * N * (N - 1) * n)
+            rmse = float(torch.sqrt(a[2] / n))
+            spread = float(torch.sqrt(a[3] / n))
+            return {"crps": float(crps), "crps_fair": float(fair), "rmse": rmse, "spread": spread,
+                    "spread_skill": (((N + 1) / N) ** 0.5) * spread / rmse if rmse > 0 else float("inf"),
+                    "rank_hist": (h / h.sum()).tolist()}
+
+        per = [scores(acc[c], hist[c], self.pixels) for c in range(self.C)]
+        out = {k: [p[k] for p in per] for k in per[0]}
+        out["overall"] = scores(acc.sum(0), hist.sum(0), self.pixels * self.C)
+        out["members"] = N
+        return out

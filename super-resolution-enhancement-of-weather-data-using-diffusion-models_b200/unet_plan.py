@@ -366,12 +366,23 @@ class UNetPlan:
     # ------------------------------------------------------------------------------------------------------------------
     # condition-only and level-only precompute
     # ------------------------------------------------------------------------------------------------------------------
-    def set_condition(self, cond):
-        """resdiff: cond = x_in['SR'] (B,C,H,W).  srdiff: cond = cat(feas[2::3], 1) (B,384,H/4,W/4)."""
-        e, B = self.eng, self.B
+    def set_condition(self, cond, repeats=1):
+        """resdiff: cond = x_in['SR'] (B,C,H,W).  srdiff: cond = cat(feas[2::3], 1) (B,384,H/4,W/4).
+        repeats = R > 1 (ensembles): cond holds B / R conditions; the condition-only work runs once on them and its outputs are copied
+        into the other R - 1 member slices of the batch, so every member sees exactly what a run on the B / R conditions alone sees
+        (for resdiff the FD splitter's 4-D FFT couples the batch: each member gets the spectrum of its own B / R group)."""
+        e = self.eng
+        repeats = int(repeats)
+        if repeats < 1 or self.B % repeats or cond.shape[0] * repeats != self.B:
+            raise ValueError("set_condition: %d conditions x %d repeats != plan batch %d" % (cond.shape[0], repeats, self.B))
+        B = self.B // repeats
         st = e.stream
+
+        def head(a):
+            # the first B images of an activation buffer (Act is image-major, so this is a prefix of the same buffer)
+            return Act(a.buf, B, a.H, a.W, a.C, a.ld, a.coff, a.dt)
         if self.kind == "resdiff":
-            self.cond.copy_(cond.to(torch.float32))
+            self.cond[:B].copy_(cond.to(torch.float32))
             nat.call("wsr_fd_precompute", self.cond.data_ptr(), B, self.C_img, self.H, self.W, self.fd_s0.data_ptr(),
                      self.fd_s2.data_ptr(), self.fd_h0.data_ptr(), self.fd_h2.data_ptr(), self.fd_ctw.data_ptr(),
                      self.fd_ctb.data_ptr(), self.fd_ctw.shape[0], self.lf.data_ptr(), self.hf.data_ptr(),
@@ -385,18 +396,19 @@ class UNetPlan:
                 assert (ca.h, ca.w) == (self.H >> (j + 1), self.W >> (j + 1))
                 nat.call("wsr_nchw_to_nhwc", self.haar_out.data_ptr() + 4 * off, B, self.C_img, ca.h, ca.w, ca.qimg.ptr,
                          nat.F32, ca.qimg.ld, st)
-                e.conv(ca.qimg, ca.wq, ca.q, bias=False, force_simt=True)
+                e.conv(head(ca.qimg), ca.wq, head(ca.q), bias=False, force_simt=True)
                 off += n
+            shared = [self.cond, self.lf, self.hf] + [ca.q.buf for ca in self.hfca]
         elif self.kind == "phydiff":
             # condition-only work of phydiff/unet.py:262-314, done once per batch: stencil channels of the reflect-padded
             # condition, the 3-band Haar queries and their 1x1 projections; cond and the stencils are written straight into
             # their channel slices of the stem input [cond | x_t | Kx Ky Kxy]
             C = self.C_img
             stem = self.downs[0]
-            self.cond.copy_(cond.to(torch.float32))
+            self.cond[:B].copy_(cond.to(torch.float32))
             nat.call("wsr_phy_stencils", self.cond.data_ptr(), B, C, self.H, self.W, self.stencils.data_ptr(), st)
-            e.nchw_to_act(self.cond, stem.xin.slice(0, C))
-            e.nchw_to_act(self.stencils, stem.xin.slice(2 * C, 3))
+            e.nchw_to_act(self.cond[:B], head(stem.xin.slice(0, C)))
+            e.nchw_to_act(self.stencils[:B], head(stem.xin.slice(2 * C, 3)))
             nat.call("wsr_haar_detail_bands", self.cond.data_ptr(), B, C, self.H, self.W, 4, self.haar_out.data_ptr(),
                      self.haar_work.data_ptr(), st)
             off = 0
@@ -406,17 +418,23 @@ class UNetPlan:
                 assert (ca.h, ca.w) == (self.H >> (j + 1), self.W >> (j + 1))
                 nat.call("wsr_nchw_to_nhwc", self.haar_out.data_ptr() + 4 * off, B, 3 * C, ca.h, ca.w, ca.qimg.ptr,
                          nat.F32, ca.qimg.ld, st)
-                e.conv(ca.qimg, ca.wq, ca.q, bias=False, force_simt=True)
+                e.conv(head(ca.qimg), ca.wq, head(ca.q), bias=False, force_simt=True)
                 off += n
+            shared = [stem.xin.buf] + [ca.q.buf for ca in self.hfca]     # stem input: its x_t slice is rewritten every step
         elif self.kind == "sr3":
-            self.cond.copy_(cond.to(torch.float32))
-            e.nchw_to_act(self.cond, self.downs[0].xin.slice(0, self.C_img))
+            self.cond[:B].copy_(cond.to(torch.float32))
+            e.nchw_to_act(self.cond[:B], head(self.downs[0].xin.slice(0, self.C_img)))
+            shared = [self.downs[0].xin.buf]
         else:
             src = cond.to(torch.float32).contiguous()
-            e.nchw_to_act(src, self.cond_feat)
+            e.nchw_to_act(src, head(self.cond_feat))
             nat.call("wsr_conv_transpose_k8s4", self.cond_feat.ptr, self.cond_feat.dt, B, self.cond_feat.H, self.cond_feat.W,
                      self.cond_feat.C, self.cond_feat.ld, self.cp_w.data_ptr(), self.cp_b.data_ptr(), self.cond_up.C,
                      self.cond_up.ptr, self.cond_up.dt, self.cond_up.ld, st)
+            shared = [self.cond_up.buf]
+        for t in shared if repeats > 1 else ():
+            for r in range(1, repeats):
+                t[r * B:(r + 1) * B].copy_(t[:B])          # contiguous device-to-device copies
 
     def _embed(self, levels, n_rows, temb, proj):
         st = self.eng.stream
@@ -573,16 +591,22 @@ class UNetPlan:
                                     and bool(nat.call("wsr_head_sampler_supported", self.final_cin, self.C_img, self.groups)))
         return ok
 
-    def head_sampler_step(self, feat, x_state, tab, T, t_dev, z, z_stride, seed, clip):
-        """eps_hat = final_conv(feat) and x_state <- reverse-step update, one launch; eps_hat is also left in ``self.eps``."""
+    def head_sampler_step(self, feat, x_state, tab, T, t_dev, z, z_stride, seed, clip, members=None):
+        """eps_hat = final_conv(feat) and x_state <- reverse-step update, one launch; eps_hat is also left in ``self.eps``.
+        members: None, or (device key table, elements per member) for member-keyed noise (wsr_final_conv_sampler_step_members)."""
         e = self.eng
         assert feat.stats_ptr and feat.C == self.final_cin and feat.dt == nat.BF16
         npix = self.B * self.H * self.W
-        e.call("wsr_final_conv_sampler_step", feat.ptr, feat.ld, self.B, self.H, self.W, feat.C, feat.stats_ptr, feat.st_ld,
-               self.gf.data_ptr(), self.bf_.data_ptr(), self.groups, 1e-5, self.final_hw.data_ptr(), self.final.bias.data_ptr(),
-               self.C_img, self.eps.data_ptr(), x_state.data_ptr(), 0 if z is None else z.data_ptr(), z_stride, seed, tab.data_ptr(), T,
-               t_dev.data_ptr(), 1 if clip else 0, e.stream, tag="head_sampler",
-               flops=2 * npix * 9 * feat.C * self.C_img, nbytes=npix * (feat.C * 2 + self.C_img * (16 if z is not None else 12)))
+        head = (feat.ptr, feat.ld, self.B, self.H, self.W, feat.C, feat.stats_ptr, feat.st_ld, self.gf.data_ptr(), self.bf_.data_ptr(),
+                self.groups, 1e-5, self.final_hw.data_ptr(), self.final.bias.data_ptr(), self.C_img, self.eps.data_ptr(),
+                x_state.data_ptr(), 0 if z is None else z.data_ptr(), z_stride)
+        tail = (tab.data_ptr(), T, t_dev.data_ptr(), 1 if clip else 0, e.stream)
+        cost = dict(tag="head_sampler", flops=2 * npix * 9 * feat.C * self.C_img,
+                    nbytes=npix * (feat.C * 2 + self.C_img * (16 if z is not None else 12)))
+        if members is None:
+            e.call("wsr_final_conv_sampler_step", *head, seed, *tail, **cost)
+        else:
+            e.call("wsr_final_conv_sampler_step_members", *head, members[0].data_ptr(), members[1], *tail, **cost)
 
     def run(self, x_t, head=True):
         """One denoiser call on the current condition / level projection.  x_t: fp32 NCHW device tensor (B,C,H,W).
