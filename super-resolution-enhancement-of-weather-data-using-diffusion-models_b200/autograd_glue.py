@@ -17,28 +17,16 @@ weights_epoch = 0          # bumped by every optimizer step that writes paramete
 
 class DenoiseFn(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, anchor, net, x, time, cond=None):
-        """cond: SRDiff with a trainable encoder -- the condition cat(feas[2::3]) as a tensor ARGUMENT, so that autograd routes
-        its gradient (``UNetTrainPlan.cond_grad``) back into the encoder's backward pass."""
-        ctx.has_cond = cond is not None
-        if isinstance(x, (tuple, list)):
-            # SRDiff: x = (18 RRDB feature maps, x_t); the condition is cat(feas[2::3]) (srdiff/unet.py:117-118)
-            feas, x_t = x
-            b = x_t.shape[0]
-            pl = net.train_plan(b, x_t.device)
-            pl.train_mode = bool(net.training)
-            pl.want_cond_grad = cond is not None
-            pl.set_condition(cond.detach() if cond is not None else torch.cat(list(feas[2::3]), dim=1))
-            pl.set_levels(time.reshape(b))
-            eps = pl.denoise(x_t)
-            ctx.pl, ctx.net = pl, net
-            return eps
-        b, c = x.shape[0], net.image_channels
-        pl = net.train_plan(b, x.device)
+    def forward(ctx, anchor, net, cond, x_t, time):
+        """cond, x_t: the split of the UNet's input (``PlannedUNet._split``).  A condition that requires grad -- SRDiff with a
+        trainable encoder, cat(feas[2::3]) -- gets its gradient (``UNetTrainPlan.cond_grad``) back into the encoder's backward pass."""
+        b = x_t.shape[0]
+        pl = net.train_plan(b, x_t.device)
         pl.train_mode = bool(net.training)
-        pl.set_condition(x[:, :c])
+        pl.want_cond_grad = ctx.needs_input_grad[2]
+        pl.set_condition(cond.detach())
         pl.set_levels(time.reshape(b))
-        eps = pl.denoise(x[:, c:])
+        eps = pl.denoise(x_t)
         ctx.pl, ctx.net = pl, net
         return eps
 
@@ -59,7 +47,7 @@ class DenoiseFn(torch.autograd.Function):
                 p.grad = g
             else:
                 p.grad.add_(g)
-        return None, None, None, None, (pl.cond_grad() if (ctx.has_cond and ctx.needs_input_grad[4]) else None)
+        return None, None, (pl.cond_grad() if ctx.needs_input_grad[2] else None), None, None
 
 
 class NoiseLossFn(torch.autograd.Function):

@@ -550,7 +550,6 @@ class Engine:
                       1.0 / math.sqrt(Cc), self.stream, flops=4 * B * Nq * Nk * Cc,
                       tag="attn_small_tc" if not self.prof_detail else "attn_small_tc N%d d%d" % (Nk, Cc))
             return o
-        es = q.buf.element_size()
         s_dt = nat.BF16 if scores.dtype == torch.bfloat16 else nat.F32
         p_dt = nat.BF16 if probs.dtype == torch.bfloat16 else nat.F32
         self.gemm(q.ptr, q.dt, (Nq * q.ld, q.ld, 1), k.ptr, k.dt, (Nk * k.ld, k.ld, 1),
@@ -558,5 +557,4 @@ class Engine:
         self.softmax(scores, s_dt, B * Nq, Nk, 1.0 / math.sqrt(Cc), probs, p_dt)
         self.gemm(probs.data_ptr(), p_dt, (Nq * Nk, Nk, 1), vT.data_ptr(), self.dt, (Cc * Nk, Nk, 1),
                   o.ptr, o.dt, (Nq * o.ld, o.ld, 1), B, Nq, Cc, Nk)
-        del es
         return o

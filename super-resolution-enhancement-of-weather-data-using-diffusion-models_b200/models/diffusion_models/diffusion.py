@@ -6,8 +6,6 @@ attributes (``num_timesteps``, ``sqrt_alphas_cumprod_prev`` as a host numpy arra
 wsr_noise_loss); the reverse loop keeps the step counter on the device and replays one captured CUDA graph per step
 instead of ~610 eager launches plus a host->device copy (reference diffusion.py:159-160).
 """
-from abc import abstractmethod
-
 import numpy as np
 import torch
 from torch import nn
@@ -49,6 +47,10 @@ def ensemble_chunks(n_members, batch, max_images=64, member_offset=0):
 
 
 class GaussianDiffusion(nn.Module):
+    # ResDiff, PhyDiff, SRDiff: the forward process runs on HR - SR (q_sample around SR) and the sampler returns image + SR.
+    # SR3 sets False: the target is HR itself and nothing is added back.
+    residual = True
+
     def __init__(self, denoise_fn, channels=1, loss_type='l1', conditional=True, schedule_opt=None, image_height=128,
                  image_width=256, pretrained_model_path=None, lock_weights=True):
         super().__init__()
@@ -195,11 +197,31 @@ class GaussianDiffusion(nn.Module):
             return loop.x, eps_log
         return loop.x
 
-    def _ensemble_condition(self, x_in):
-        """Hook of ``super_resolution_ensemble``: (condition tensor for the plan, field added to every member at the end or None).
-        ResDiff / PhyDiff: the condition is x_in['SR'] and the sampler returns image + SR."""
-        sr = x_in["SR"].to(device=self.betas.device, dtype=torch.float32)
-        return sr, sr
+    def _loop_input(self, x_in):
+        """super_resolution's dict -> p_sample_loop's input: the condition x_in['SR']."""
+        return x_in["SR"]
+
+    def _loop_condition(self, x):
+        """p_sample_loop's input -> (condition tensor for the plan, field added to the sampled image or None).  Here x is the
+        condition itself, which is added back when the process is ``residual``."""
+        cond = x.to(device=self.betas.device, dtype=torch.float32)
+        return cond, (cond if self.residual else None)
+
+    @torch.no_grad()
+    def p_sample_loop(self, x_in, continous=False, noise_chain=None, seed=None):
+        """The conditional reverse loop (reference :58-94): x_in is ``_loop_input``'s form of the batch."""
+        if not self.conditional:
+            raise NotImplementedError("unconditional sampling is not part of the accelerated path")
+        cond, add = self._loop_condition(x_in)
+        shape = tuple((cond if add is None else add).shape)       # the image's: the added field's, or (SR3) the condition's
+        plan = self._plan(shape[0], self.betas.device)
+        plan.set_condition(cond)
+        img = self._reverse_loop(plan, shape, noise_chain=noise_chain, seed=seed)
+        return img if add is None else img + add
+
+    @torch.no_grad()
+    def super_resolution(self, x_in, continous=False):
+        return self.p_sample_loop(self._loop_input(x_in), continous)
 
     @torch.no_grad()
     def super_resolution_ensemble(self, x_in, n_members, seed=None, member_offset=0, max_images=64):
@@ -218,7 +240,7 @@ class GaussianDiffusion(nn.Module):
         B = shape[0]
         base = int(seed) if seed is not None else (int(self.sample_seed) if self.sample_seed is not None
                                                    else int(torch.randint(0, 2 ** 62, (1,)).item()))
-        cond, add = self._ensemble_condition(x_in)
+        cond, add = self._loop_condition(self._loop_input(x_in))
         out = torch.empty((n_members,) + shape, device=dev, dtype=torch.float32)
         for first, r in ensemble_chunks(n_members, B, max_images, member_offset):
             plan = self._plan(r * B, dev)
@@ -236,17 +258,32 @@ class GaussianDiffusion(nn.Module):
     def sample(self, batch_size=1, continous=False):
         return self.p_sample_loop((batch_size, self.channels, self.image_height, self.image_height), continous)
 
-    def q_sample(self, x_start, continuous_sqrt_alpha_cumprod, noise=None):
-        """reference :209-228.  x_start (B,C,H,W), continuous_sqrt_alpha_cumprod (B,1,1,1)."""
+    def q_sample(self, x_start, continuous_sqrt_alpha_cumprod, noise=None, offset=None):
+        """reference :209-228.  x_start (B,C,H,W), continuous_sqrt_alpha_cumprod (B,1,1,1).  offset: x_t is centred on
+        ``offset + a * x_start`` (the residual processes' SR; None = 0)."""
         noise = default(noise, lambda: torch.randn_like(x_start))
         x0 = x_start.to(torch.float32).contiguous()
         a = continuous_sqrt_alpha_cumprod.reshape(-1).to(torch.float32).contiguous()
         nz = noise.to(torch.float32).contiguous()
-        zero = torch.zeros_like(x0)
+        off = torch.zeros_like(x0) if offset is None else offset.to(torch.float32).contiguous()
         out = torch.empty_like(x0)
-        nat.call("wsr_q_sample", x0.data_ptr(), zero.data_ptr(), nz.data_ptr(), a.data_ptr(), x0.shape[0],
+        nat.call("wsr_q_sample", x0.data_ptr(), off.data_ptr(), nz.data_ptr(), a.data_ptr(), x0.shape[0],
                  x0[0].numel(), out.data_ptr(), torch.cuda.current_stream(x0.device).cuda_stream)
         return out
+
+    def _draw_levels(self, b, device):
+        """ONE t per batch, then b continuous noise levels in [sqrt(abar[t-1]), sqrt(abar[t])), from numpy's global RNG in the
+        reference's order: randint, then uniform (reference :116-121)."""
+        t = np.random.randint(1, self.num_timesteps + 1)
+        return torch.FloatTensor(np.random.uniform(self.sqrt_alphas_cumprod_prev[t - 1],
+                                                   self.sqrt_alphas_cumprod_prev[t], size=b)).to(device)
+
+    def _loss(self, noise, eps):
+        """The noise loss, through the autograd node when eps carries a gradient."""
+        if eps.requires_grad:
+            from ...autograd_glue import NoiseLossFn
+            return NoiseLossFn.apply(noise, eps, self.loss_type == 'l2')
+        return self._noise_loss(noise, eps)
 
     def _noise_loss(self, noise, eps):
         """Sum-reduced L1/L2 (reference :98-110) computed by wsr_noise_loss; returns a 0-dim fp32 tensor."""
@@ -258,17 +295,19 @@ class GaussianDiffusion(nn.Module):
     def forward(self, x, *args, **kwargs):
         return self.p_losses(x, *args, **kwargs)
 
-    @abstractmethod
-    def p_sample_loop(self, x_in, continous=False) -> torch.Tensor:
-        pass
-
-    @abstractmethod
-    def super_resolution(self, x_in, continous=False) -> torch.Tensor:
-        pass
-
-    @abstractmethod
-    def p_losses(self, x_in, noise=None) -> torch.Tensor:
-        pass
+    def p_losses(self, x_in, noise=None):
+        """reference :111-152: one t per batch and per-sample continuous level (``_draw_levels``), q_sample of HR around SR
+        (``residual``) or 0, the denoiser on cat([SR, x_t]), sum-reduced loss."""
+        sr, hr = x_in['SR'], x_in['HR']
+        b = sr.shape[0]
+        level = self._draw_levels(b, sr.device)
+        noise = default(noise, lambda: torch.randn_like(sr)).to(torch.float32).contiguous()
+        hr32, sr32 = hr.to(torch.float32).contiguous(), sr.to(torch.float32).contiguous()
+        x_noisy = self.q_sample(hr32, level, noise, offset=sr32 if self.residual else None)
+        if not self.conditional:
+            raise NotImplementedError("unconditional training is not part of the accelerated path")
+        eps = self.denoise_fn(torch.cat([sr32, x_noisy], dim=1), level.view(b, -1))
+        return self._loss(noise, eps)
 
 
 class ReverseLoop:

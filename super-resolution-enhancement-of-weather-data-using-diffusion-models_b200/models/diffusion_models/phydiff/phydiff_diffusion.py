@@ -1,12 +1,7 @@
 """PhyDiffDiffusion -- drop-in for the reference's phydiff/phydiff_diffusion.py:9-139: ResDiff's process (residual target
 HR - SR, sampler returns image + condition) around the PhyDiff UNet; the moment loss of the reference is commented out there
 (:134-137) and therefore absent here too."""
-import numpy as np
-import torch
-
-from .... import _native as nat
 from ..diffusion import GaussianDiffusion
-from ..nn_modules.functional_layers import default
 
 
 class PhyDiffDiffusion(GaussianDiffusion):
@@ -15,39 +10,3 @@ class PhyDiffDiffusion(GaussianDiffusion):
         super().__init__(denoise_fn=denoise_fn, channels=channels, loss_type=loss_type, conditional=conditional,
                          schedule_opt=schedule_opt, image_height=image_height, image_width=image_width,
                          pretrained_model_path=pretrained_model_path, lock_weights=lock_weights)
-
-    @torch.no_grad()
-    def p_sample_loop(self, x_in, continous=False, noise_chain=None, seed=None):
-        """reference :49-82 (conditional branch): returns the final image + the condition."""
-        if not self.conditional:
-            raise NotImplementedError("unconditional sampling is not part of the accelerated path")
-        cond = x_in
-        plan = self._plan(cond.shape[0], self.betas.device)
-        plan.set_condition(cond.to(self.betas.device))
-        img = self._reverse_loop(plan, tuple(cond.shape), noise_chain=noise_chain, seed=seed)
-        return img + cond.to(device=img.device, dtype=torch.float32)
-
-    @torch.no_grad()
-    def super_resolution(self, x_in, continous=False):
-        return self.p_sample_loop(x_in["SR"], continous)
-
-    def p_losses(self, x_in, noise=None):
-        """reference :98-139."""
-        sr, hr = x_in['SR'], x_in['HR']
-        b = sr.shape[0]
-        dev = sr.device
-        t = np.random.randint(1, self.num_timesteps + 1)
-        level = torch.FloatTensor(np.random.uniform(self.sqrt_alphas_cumprod_prev[t - 1],
-                                                    self.sqrt_alphas_cumprod_prev[t], size=b)).to(dev)
-        noise = default(noise, lambda: torch.randn_like(sr)).to(torch.float32).contiguous()
-        hr32, sr32 = hr.to(torch.float32).contiguous(), sr.to(torch.float32).contiguous()
-        x_noisy = torch.empty_like(sr32)
-        nat.call("wsr_q_sample", hr32.data_ptr(), sr32.data_ptr(), noise.data_ptr(), level.data_ptr(), b,
-                 sr32[0].numel(), x_noisy.data_ptr(), torch.cuda.current_stream(dev).cuda_stream)
-        if not self.conditional:
-            raise NotImplementedError("unconditional training is not part of the accelerated path")
-        eps = self.denoise_fn(torch.cat([sr32, x_noisy], dim=1), level.view(b, -1))
-        if eps.requires_grad:
-            from ....autograd_glue import NoiseLossFn
-            return NoiseLossFn.apply(noise, eps, self.loss_type == 'l2')
-        return self._noise_loss(noise, eps)

@@ -4,12 +4,10 @@ The condition is whatever tensor is under ``x_in['SR']`` (bicubic x4 of LR in th
 dataset_builder.py:374-380); the SimpleCNN prior is loaded under ``self.cnn`` for checkpoint compatibility but, as in
 the reference, never called on this path (SURVEY.md 0.1).
 """
-import numpy as np
 import torch
 
 from ...simple_cnn.Simple_CNN import SimpleCNN
 from ..diffusion import GaussianDiffusion
-from ..nn_modules.functional_layers import default
 
 
 class ResDiffDiffusion(GaussianDiffusion):
@@ -26,44 +24,3 @@ class ResDiffDiffusion(GaussianDiffusion):
             if lock_weights:
                 for p in self.cnn.parameters():
                     p.requires_grad_(False)
-
-    @torch.no_grad()
-    def p_sample_loop(self, x_in, continous=False, noise_chain=None, seed=None):
-        """reference :58-94.  Conditional: x_in is the condition (B,C,H,W); returns final image + condition."""
-        if not self.conditional:
-            raise NotImplementedError("unconditional sampling is not part of the accelerated path")
-        cond = x_in
-        plan = self._plan(cond.shape[0], self.betas.device)
-        plan.set_condition(cond.to(self.betas.device))
-        img = self._reverse_loop(plan, tuple(cond.shape), noise_chain=noise_chain, seed=seed)
-        return img + cond.to(device=img.device, dtype=torch.float32)
-
-    @torch.no_grad()
-    def super_resolution(self, x_in, continous=False):
-        return self.p_sample_loop(x_in["SR"], continous)
-
-    def p_losses(self, x_in, noise=None):
-        """reference :111-152: residual target HR-SR, ONE t per batch and per-sample continuous noise level from numpy's
-        global RNG (same call order: randint, then uniform), q_sample, denoiser, sum-reduced loss."""
-        sr = x_in['SR']
-        hr = x_in['HR']
-        b = sr.shape[0]
-        t = np.random.randint(1, self.num_timesteps + 1)
-        level = torch.FloatTensor(np.random.uniform(self.sqrt_alphas_cumprod_prev[t - 1],
-                                                    self.sqrt_alphas_cumprod_prev[t], size=b)).to(sr.device)
-        noise = default(noise, lambda: torch.randn_like(sr))
-        noise = noise.to(torch.float32).contiguous()
-        dev = sr.device
-        hr32, sr32 = hr.to(torch.float32).contiguous(), sr.to(torch.float32).contiguous()
-        x_noisy = torch.empty_like(sr32)
-        from .... import _native as nat
-        nat.call("wsr_q_sample", hr32.data_ptr(), sr32.data_ptr(), noise.data_ptr(), level.data_ptr(), b,
-                 sr32[0].numel(), x_noisy.data_ptr(), torch.cuda.current_stream(dev).cuda_stream)
-        if not self.conditional:
-            raise NotImplementedError("unconditional training is not part of the accelerated path")
-        eps = self.denoise_fn(torch.cat([sr32, x_noisy], dim=1), level.view(b, -1))
-        self._last_eps = eps
-        if eps.requires_grad:
-            from ....autograd_glue import NoiseLossFn
-            return NoiseLossFn.apply(noise, eps, self.loss_type == 'l2')
-        return self._noise_loss(noise, eps)

@@ -56,34 +56,24 @@ def build_unet_body(net, in_channel, out_channel, inner_channel, norm_groups, ch
     net.final_conv = Block(width, default(out_channel, in_channel), groups=norm_groups)
 
 
-class UNet(nn.Module):
-    def __init__(self, in_channel=9, out_channel=3, inner_channel=32, norm_groups=32, channel_mults=(1, 2, 4, 8, 8),
-                 attn_res=(8,), res_blocks=3, dropout=0, with_noise_level_emb=True, image_width=128, image_height=128,
-                 image_channels=3, precision="bf16"):
+def noise_level_mlp(inner_channel, act):
+    """PositionalEncoding -> Linear -> act -> Linear: the noise-level embedding of every UNet of the family."""
+    return nn.Sequential(
+        PositionalEncoding(inner_channel),
+        nn.Linear(inner_channel, inner_channel * 4),
+        act,
+        nn.Linear(inner_channel * 4, inner_channel),
+    )
+
+
+class PlannedUNet(nn.Module):
+    """The engine glue shared by the four UNets: plan caches and ``forward`` through ``UNetPlan`` / ``UNetTrainPlan``.
+    Subclasses build their modules and say how ``forward``'s input splits into (condition, x_t) (``_split``)."""
+
+    def __init__(self):
         super().__init__()
-        if not with_noise_level_emb:
-            raise NotImplementedError("with_noise_level_emb=False is never used on the reference's path")
-        self.noise_level_mlp = nn.Sequential(
-            PositionalEncoding(inner_channel),
-            nn.Linear(inner_channel, inner_channel * 4),
-            Swish(),
-            nn.Linear(inner_channel * 4, inner_channel),
-        )
-        self.image_channels = image_channels
-        self.fd_spliter = FD_Info_Spliter(dim=inner_channel, in_channels=image_channels, out_channels=out_channel,
-                                          image_height=image_height, image_width=image_width)
-        self.image_height, self.image_width = image_height, image_width
-        self.inner_channel, self.norm_groups, self.dropout = inner_channel, norm_groups, dropout
-        self.J = 4
-        self.hf_ca_list = nn.ModuleList(
-            [HF_guided_CA(inner_channel * (2 ** i), image_channels=image_channels) for i in range(self.J)])
-        build_unet_body(self, in_channel, out_channel, inner_channel, norm_groups, channel_mults, attn_res, res_blocks,
-                        dropout, inner_channel, image_height)
-        self.precision = precision
-        self.time_act = "swish"
         self._plans = {}
 
-    # ---- engine glue ------------------------------------------------------------------------------------------------
     def plan(self, batch, device=None, precision=None, strict_tc=False):
         """The compiled launch schedule for a given local batch size (cached)."""
         device = device or next(self.parameters()).device
@@ -110,23 +100,48 @@ class UNet(nn.Module):
         self._plans = {}           # .to() / .cuda() re-allocate the parameters: drop plans that point at the old storage
         return super()._apply(fn, *args, **kwargs)
 
-    def forward(self, x, time):
-        b = x.shape[0]
+    def _split(self, x):
+        """forward's input -> (condition, x_t): x = cat([condition, x_t], 1) (ResDiff, PhyDiff, SR3)."""
         c = self.image_channels
         if x.shape[1] != 2 * c:
             raise AssertionError("expected cat([condition, x_t]) with %d channels, got %d" % (2 * c, x.shape[1]))
+        return x[:, :c], x[:, c:]
+
+    def forward(self, x, time):
+        cond, x_t = self._split(x)
+        b = x_t.shape[0]
         if torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters()):
             # training step: the autograd node runs the hand-written backward pass (unet_train.py)
             from ....autograd_glue import DenoiseFn
             anchor = next(p for p in self.parameters() if p.requires_grad)
-            return DenoiseFn.apply(anchor, self, x, time)
+            return DenoiseFn.apply(anchor, self, cond, x_t, time)
         if self.training and self.dropout:
-            pl = self.train_plan(b, x.device)
+            pl = self.train_plan(b, x_t.device)
             pl.train_mode = True
-            pl.set_condition(x[:, :c])
-            pl.set_levels(time.reshape(b))
-            return pl.denoise(x[:, c:])
-        pl = self.plan(b, x.device)
-        pl.set_condition(x[:, :c])
+        else:
+            pl = self.plan(b, x_t.device)
+        pl.set_condition(cond)
         pl.set_levels(time.reshape(b))
-        return pl.denoise(x[:, c:])
+        return pl.denoise(x_t)
+
+
+class UNet(PlannedUNet):
+    def __init__(self, in_channel=9, out_channel=3, inner_channel=32, norm_groups=32, channel_mults=(1, 2, 4, 8, 8),
+                 attn_res=(8,), res_blocks=3, dropout=0, with_noise_level_emb=True, image_width=128, image_height=128,
+                 image_channels=3, precision="bf16"):
+        super().__init__()
+        if not with_noise_level_emb:
+            raise NotImplementedError("with_noise_level_emb=False is never used on the reference's path")
+        self.noise_level_mlp = noise_level_mlp(inner_channel, Swish())
+        self.image_channels = image_channels
+        self.fd_spliter = FD_Info_Spliter(dim=inner_channel, in_channels=image_channels, out_channels=out_channel,
+                                          image_height=image_height, image_width=image_width)
+        self.image_height, self.image_width = image_height, image_width
+        self.inner_channel, self.norm_groups, self.dropout = inner_channel, norm_groups, dropout
+        self.J = 4
+        self.hf_ca_list = nn.ModuleList(
+            [HF_guided_CA(inner_channel * (2 ** i), image_channels=image_channels) for i in range(self.J)])
+        build_unet_body(self, in_channel, out_channel, inner_channel, norm_groups, channel_mults, attn_res, res_blocks,
+                        dropout, inner_channel, image_height)
+        self.precision = precision
+        self.time_act = "swish"

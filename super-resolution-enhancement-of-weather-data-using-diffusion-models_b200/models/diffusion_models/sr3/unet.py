@@ -4,15 +4,13 @@ The plain conditional UNet of the family: ``forward(x, time)`` with ``x = cat([c
 the stem convolution; no FD splitter, no HF-guided cross attention, ONE mid block without attention (:77-81).  Same
 constructor signature and state_dict keys (347 tensors for the canonical config); runs through ``UNetPlan`` (kind 'sr3').
 """
-import torch
 from torch import nn
 
-from ....unet_plan import UNetPlan
-from ..nn_modules.functional_layers import PositionalEncoding, Swish
-from ..resdiff.unet import build_unet_body
+from ..nn_modules.functional_layers import Swish
+from ..resdiff.unet import PlannedUNet, build_unet_body, noise_level_mlp
 
 
-class UNet(nn.Module):
+class UNet(PlannedUNet):
     def __init__(self, in_channel=6, out_channel=3, inner_channel=32, norm_groups=32, channel_mults=(1, 2, 4, 8, 8),
                  attn_res=(8,), res_blocks=3, dropout=0, with_noise_level_emb=True, image_width=128, image_height=128,
                  image_channels=3, precision="bf16"):
@@ -21,12 +19,7 @@ class UNet(nn.Module):
             raise NotImplementedError("with_noise_level_emb=False is never used on the reference's path")
         if in_channel != 2 * image_channels:
             raise AssertionError("SR3 consumes cat([condition, x_t]): in_channel must be 2 * image_channels")
-        self.noise_level_mlp = nn.Sequential(
-            PositionalEncoding(inner_channel),
-            nn.Linear(inner_channel, inner_channel * 4),
-            Swish(),
-            nn.Linear(inner_channel * 4, inner_channel),
-        )
+        self.noise_level_mlp = noise_level_mlp(inner_channel, Swish())
         self.image_channels = image_channels
         self.image_height, self.image_width = image_height, image_width
         self.inner_channel, self.norm_groups, self.dropout = inner_channel, norm_groups, dropout
@@ -34,52 +27,3 @@ class UNet(nn.Module):
                         dropout, inner_channel, image_height, mid_attn=(False,))
         self.precision = precision
         self.time_act = "swish"
-        self._plans = {}
-
-    # ---- engine glue ------------------------------------------------------------------------------------------------
-    def plan(self, batch, device=None, precision=None, strict_tc=False):
-        """The compiled launch schedule for a given local batch size (cached)."""
-        device = device or next(self.parameters()).device
-        key = (batch, str(device), precision or self.precision, strict_tc)
-        pl = self._plans.get(key)
-        if pl is None:
-            pl = UNetPlan(self, batch, device, precision or self.precision, strict_tc=strict_tc)
-            self._plans[key] = pl
-        pl.refresh_weights()
-        return pl
-
-    def train_plan(self, batch, device=None, precision=None):
-        """Forward + backward schedule (``UNetTrainPlan``) for a given local batch size (cached)."""
-        from ....unet_train import UNetTrainPlan
-        device = device or next(self.parameters()).device
-        key = ("train", batch, str(device), precision or self.precision)
-        pl = self._plans.get(key)
-        if pl is None:
-            pl = UNetTrainPlan(self, batch, device, precision or self.precision)
-            self._plans[key] = pl
-        return pl
-
-    def _apply(self, fn, *args, **kwargs):
-        self._plans = {}           # .to() / .cuda() re-allocate the parameters: drop plans that point at the old storage
-        return super()._apply(fn, *args, **kwargs)
-
-    def forward(self, x, time):
-        b = x.shape[0]
-        c = self.image_channels
-        if x.shape[1] != 2 * c:
-            raise AssertionError("expected cat([condition, x_t]) with %d channels, got %d" % (2 * c, x.shape[1]))
-        if torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters()):
-            # training step: the autograd node runs the hand-written backward pass (unet_train.py)
-            from ....autograd_glue import DenoiseFn
-            anchor = next(p for p in self.parameters() if p.requires_grad)
-            return DenoiseFn.apply(anchor, self, x, time)
-        if self.training and self.dropout:
-            pl = self.train_plan(b, x.device)
-            pl.train_mode = True
-            pl.set_condition(x[:, :c])
-            pl.set_levels(time.reshape(b))
-            return pl.denoise(x[:, c:])
-        pl = self.plan(b, x.device)
-        pl.set_condition(x[:, :c])
-        pl.set_levels(time.reshape(b))
-        return pl.denoise(x[:, c:])

@@ -1,10 +1,8 @@
 """SRDiffDiffusion -- drop-in for the reference's srdiff/srdiff_diffusion.py:9-219: RRDB encoder once per batch, then T reverse
 steps of the SRDiff UNet conditioned on 6 of its 18 feature maps; training with a frozen (``lock_weights=True``) or a jointly trained
 encoder."""
-import numpy as np
 import torch
 
-from .... import _native as nat
 from ...rrdb_encoder.RRDBNet import RRDBNet
 from ..diffusion import GaussianDiffusion
 from ..nn_modules.functional_layers import default
@@ -39,25 +37,12 @@ class SRDiffDiffusion(GaussianDiffusion):
         pl, feas = self.rrdb_encoder.features_device(lr)
         return torch.cat([f.to_nchw(pl.eng) for f in feas[2::3]], dim=1)
 
-    @torch.no_grad()
-    def p_sample_loop(self, x_in, continous=False, noise_chain=None, seed=None):
-        """reference :77-117.  x_in: dict with 'SR' (bicubic) and 'LR'."""
-        if not self.conditional:
-            raise NotImplementedError("unconditional sampling is not part of the accelerated path")
-        dev = self.betas.device
-        sr_up = x_in['SR'].to(dev)
-        cond = self._condition(x_in['LR'].to(dev))
-        plan = self._plan(sr_up.shape[0], dev)
-        plan.set_condition(cond)
-        img = self._reverse_loop(plan, tuple(sr_up.shape), noise_chain=noise_chain, seed=seed)
-        return img + sr_up.to(torch.float32)
+    def _loop_input(self, x_in):
+        """p_sample_loop takes the whole dict (reference :77-117): 'LR' feeds the encoder, 'SR' is added back."""
+        return x_in
 
-    @torch.no_grad()
-    def super_resolution(self, x_in, continous=False):
-        return self.p_sample_loop(x_in, continous)
-
-    def _ensemble_condition(self, x_in):
-        """The RRDB encoder runs once on the B LR fields; every member adds back the bicubic SR."""
+    def _loop_condition(self, x_in):
+        """The RRDB encoder runs once on the B LR fields; the bicubic SR is added back."""
         dev = self.betas.device
         return self._condition(x_in['LR'].to(dev)), x_in['SR'].to(device=dev, dtype=torch.float32)
 
@@ -79,20 +64,11 @@ class SRDiffDiffusion(GaussianDiffusion):
             rrdb_sr, feas = self.rrdb_encoder.forward_joint(lr.to(dev))
         else:
             rrdb_sr, feas = self.rrdb_encoder(lr, True)
-        t = np.random.randint(1, self.num_timesteps + 1)
-        level = torch.FloatTensor(np.random.uniform(self.sqrt_alphas_cumprod_prev[t - 1],
-                                                    self.sqrt_alphas_cumprod_prev[t], size=b)).to(dev)
+        level = self._draw_levels(b, dev)
         noise = default(noise, lambda: torch.randn_like(sr_up)).to(torch.float32).contiguous()
         hr32, sr32 = hr.to(torch.float32).contiguous(), sr_up.to(torch.float32).contiguous()
-        x_noisy = torch.empty_like(sr32)
-        nat.call("wsr_q_sample", hr32.data_ptr(), sr32.data_ptr(), noise.data_ptr(), level.data_ptr(), b,
-                 sr32[0].numel(), x_noisy.data_ptr(), torch.cuda.current_stream(dev).cuda_stream)
-        eps = self.denoise_fn((feas, x_noisy), level.view(b, -1))
-        if eps.requires_grad:
-            from ....autograd_glue import NoiseLossFn
-            loss = NoiseLossFn.apply(noise, eps, self.loss_type == 'l2')
-        else:
-            loss = self._noise_loss(noise, eps)
+        x_noisy = self.q_sample(hr32, level, noise, offset=sr32)
+        loss = self._loss(noise, self.denoise_fn((feas, x_noisy), level.view(b, -1)))
         if self.rrdb_encoder is not None and not self.lock_weights:
             return loss + torch.nn.functional.l1_loss(rrdb_sr, hr.to(torch.float32))          # reference :212-214
         return loss

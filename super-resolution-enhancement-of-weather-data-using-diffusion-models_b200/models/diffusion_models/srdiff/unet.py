@@ -4,12 +4,11 @@ projected by ConvTranspose2d(384->64, k8, s4, p2) (hoisted: condition-only) and 
 import torch
 from torch import nn
 
-from ....unet_plan import UNetPlan
-from ..nn_modules.functional_layers import Mish, PositionalEncoding
-from ..resdiff.unet import build_unet_body
+from ..nn_modules.functional_layers import Mish
+from ..resdiff.unet import PlannedUNet, build_unet_body, noise_level_mlp
 
 
-class UNet(nn.Module):
+class UNet(PlannedUNet):
     def __init__(self, in_channel=9, out_channel=3, inner_channel=32, norm_groups=32, channel_mults=(1, 2, 4, 8, 8),
                  attn_res=(8,), res_blocks=3, dropout=0, with_noise_level_emb=True, image_width=128, image_height=128,
                  image_channels=1, precision="bf16"):
@@ -19,12 +18,7 @@ class UNet(nn.Module):
         self.hidden_size = 64
         self.num_block = 17
         self.cond_proj = nn.ConvTranspose2d(self.hidden_size * ((self.num_block + 1) // 3), self.hidden_size, 8, 4, 2)
-        self.noise_level_mlp = nn.Sequential(
-            PositionalEncoding(inner_channel),
-            nn.Linear(inner_channel, inner_channel * 4),
-            Mish(),
-            nn.Linear(inner_channel * 4, inner_channel),
-        )
+        self.noise_level_mlp = noise_level_mlp(inner_channel, Mish())
         self.image_channels = image_channels
         self.image_height, self.image_width = image_height, image_width
         self.inner_channel, self.norm_groups, self.dropout = inner_channel, norm_groups, dropout
@@ -32,47 +26,9 @@ class UNet(nn.Module):
                         dropout, inner_channel, image_height)
         self.precision = precision
         self.time_act = "mish"
-        self._plans = {}
 
-    def plan(self, batch, device=None, precision=None, strict_tc=False):
-        device = device or next(self.parameters()).device
-        key = (batch, str(device), precision or self.precision, strict_tc)
-        pl = self._plans.get(key)
-        if pl is None:
-            pl = UNetPlan(self, batch, device, precision or self.precision, strict_tc=strict_tc)
-            self._plans[key] = pl
-        pl.refresh_weights()
-        return pl
-
-    def train_plan(self, batch, device=None, precision=None):
-        """Forward + backward schedule (``UNetTrainPlan``) for a given local batch size (cached)."""
-        from ....unet_train import UNetTrainPlan
-        device = device or next(self.parameters()).device
-        key = ("train", batch, str(device), precision or self.precision)
-        pl = self._plans.get(key)
-        if pl is None:
-            pl = UNetTrainPlan(self, batch, device, precision or self.precision)
-            self._plans[key] = pl
-        return pl
-
-    def _apply(self, fn, *args, **kwargs):
-        self._plans = {}           # .to() / .cuda() re-allocate the parameters: drop plans that point at the old storage
-        return super()._apply(fn, *args, **kwargs)
-
-    def forward(self, x, time):
+    def _split(self, x):
+        """x = (rrdb_features, x_t): the condition is cat(features[2::3], 1), or -- joint training with a trainable encoder --
+        that concatenation already made by ``RRDBNet.forward_joint`` as one differentiable tensor."""
         feas, x_t = x
-        b = x_t.shape[0]
-        if torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters()):
-            from ....autograd_glue import DenoiseFn
-            anchor = next(p for p in self.parameters() if p.requires_grad)
-            if torch.is_tensor(feas):          # joint training: the condition cat(feas[2::3]) as ONE differentiable tensor
-                return DenoiseFn.apply(anchor, self, ([], x_t), time, feas)
-            return DenoiseFn.apply(anchor, self, (list(feas), x_t), time)
-        if self.training and self.dropout:
-            pl = self.train_plan(b, x_t.device)
-            pl.train_mode = True
-        else:
-            pl = self.plan(b, x_t.device)
-        pl.set_condition(torch.cat(list(feas[2::3]), dim=1))
-        pl.set_levels(time.reshape(b))
-        return pl.denoise(x_t)
+        return (feas if torch.is_tensor(feas) else torch.cat(list(feas[2::3]), dim=1)), x_t

@@ -31,6 +31,11 @@ def _is_res(m):
 
 
 class UNetPlan:
+    # True for the train plan, whose forward is followed by the hand-written backward pass: every activation that pass reads stays
+    # materialised (no GroupNorm fused into the consuming convolution, q | k and V^T kept apart), and, because its forward is replayed
+    # from a recorded launch list that holds no stream events, there is no fused head and no HF-CA side stream.
+    feeds_backward = False
+
     def __init__(self, net, batch, device, precision="bf16", strict_tc=False):
         self.net = net
         self.B = int(batch)
@@ -54,7 +59,7 @@ class UNetPlan:
         # the N = 64 layers are bound by the tensor core's own shared-memory operand fetch, and the transform's traffic on the same
         # banks slows both.  So only layers with at least 128 output channels fuse (_res_block); fusing every eligible layer measured
         # slower at every batch size (DESIGN.md section 8).
-        self.fuse_gn = getattr(self, "fuse_gn", True) and self.eng.mode == "bf16"
+        self.fuse_gn = not self.feeds_backward and self.eng.mode == "bf16"
         self._structure()
         self._buffers()
         self.refresh_weights()
@@ -139,7 +144,7 @@ class UNetPlan:
                 r.nbuf = e.new_act(B, r.h, r.w, r.cout)
                 # sampling plans at the low-resolution levels: ONE q | k | v projection, V consumed as pixels x channels by the fused
                 # attention kernel (no V^T GEMM); the train plan keeps q | k + V^T (its backward pass reads them)
-                r.v_nhwc = self._plain_plan() and bf and e.small_attention_takes_nhwc_v(n, n, r.cout)
+                r.v_nhwc = not self.feeds_backward and bf and e.small_attention_takes_nhwc_v(n, n, r.cout)
                 if r.v_nhwc:
                     r.qkv = e.new_act(B, r.h, r.w, 3 * r.cout)
                     r.qk, r.vT = r.qkv.slice(0, 2 * r.cout), None
@@ -167,7 +172,7 @@ class UNetPlan:
                     n = r.h * r.w
                     ca = _L(mod=self.net.hf_ca_list[hf_i], c=r.cout, h=r.h, w=r.w, x=r.y, y=feat_dst[i], level=hf_i)
                     ca.nbuf = e.new_act(B, r.h, r.w, r.cout)
-                    ca.v_nhwc = self._plain_plan() and bf and e.small_attention_takes_nhwc_v(n, n, r.cout)
+                    ca.v_nhwc = not self.feeds_backward and bf and e.small_attention_takes_nhwc_v(n, n, r.cout)
                     if ca.v_nhwc:
                         ca.kv = e.new_act(B, r.h, r.w, 2 * r.cout)           # one k | v projection
                         ca.kbuf, ca.vT = ca.kv.slice(0, r.cout), None
@@ -191,7 +196,6 @@ class UNetPlan:
         res_scratch(self.mids[-1], up_res[0].cat.slice(0, up_res[0].cx))
         # up path: each layer writes into the x slot of the next res block's concat buffer
         for k, r in enumerate(self.ups):
-            nxt = next((q for q in self.ups[k + 1:] if q.kind == "res"), None) if k + 1 < len(self.ups) else None
             following = self.ups[k + 1] if k + 1 < len(self.ups) else None
             if following is not None and following.kind == "res":
                 dst = following.cat.slice(0, following.cx)
@@ -201,8 +205,6 @@ class UNetPlan:
                 res_scratch(r, dst)
             else:
                 r.y = dst
-            del nxt
-        # fix-up: an Upsample layer is fed by the res block before it (plain buffer) and feeds the next res block
         # head
         self.final_a = e.new_act(B, self.H, self.W, self.final_cin)
         self.eps_nhwc = e.new_act(B, self.H, self.W, self.C_img, dt=nat.F32)
@@ -309,8 +311,8 @@ class UNetPlan:
             self.gf, self.bf_ = e.f32(fc[0].weight), e.f32(fc[0].bias)
             self.final = e.pack_conv(fc[3].weight, fc[3].bias, rows=64 if e.mode == "bf16" else None)
             # fp32 [9][Cout][Cin] copy of the head's weights for the fused head + reverse-step kernel (wsr_final_conv_sampler_step)
-            self.final_f32 = self._pack_f32_conv(fc[3].weight) if (e.mode == "bf16" and type(self) is UNetPlan) else None
-            if (type(self) is UNetPlan and self.final_f32 is not None
+            self.final_f32 = self._pack_f32_conv(fc[3].weight) if (e.mode == "bf16" and not self.feeds_backward) else None
+            if (self.final_f32 is not None
                     and nat.call("wsr_head_sampler_supported", self.final_cin, self.C_img, self.groups)):
                 # ldmatrix-ready bf16 blocks of the head's weights for wsr_final_conv_sampler_step
                 key = ("headw", fc[3].weight.data_ptr())
@@ -527,17 +529,13 @@ class UNetPlan:
         e.gemm(wv.data_ptr(), e.dt, (0, cc, 1), nact.ptr, nact.dt, (n * nact.ld, nact.ld, 1),
                vT.data_ptr(), e.dt, (cc * n, n, 1), self.B, cc, n, cc)
 
-    def _plain_plan(self):
-        """The sampling / inference plan (not the train plan, whose backward pass reads q | k and V^T separately)."""
-        return type(self) is UNetPlan
-
     def _side_stream(self):
         """The HF-guided cross-attention branches (resdiff/unet.py:156-163: they only produce the SKIP tensors; the main path continues
         with the un-attended x) run on a second stream, forked after each Downsample and joined before the up path: the N = 8192 /
         2048 attention launches then overlap the deep levels of the down path, whose kernels leave most SMs idle at small batch.
         Works eagerly and inside a captured CUDA graph (event fork / join).  Only when every branch launch is a fused kernel -- the
         unfused fallback shares the score scratch with the main path's self-attention -- and not while per-launch timing is on."""
-        if not self.has_hfca or self.eng.prof is not None:
+        if self.feeds_backward or not self.has_hfca or self.eng.prof is not None:
             return None
         ok = getattr(self, "_side_ok", None)
         if ok is None:
@@ -587,7 +585,7 @@ class UNetPlan:
         (wsr_final_conv_sampler_step): bf16 sampling plan, head input produced by a convolution that emitted its statistics."""
         ok = getattr(self, "_fuse_head", None)
         if ok is None:
-            ok = self._fuse_head = (type(self) is UNetPlan and self.eng.mode == "bf16" and self.eng.use_tc
+            ok = self._fuse_head = (not self.feeds_backward and self.eng.mode == "bf16" and self.eng.use_tc
                                     and bool(nat.call("wsr_head_sampler_supported", self.final_cin, self.C_img, self.groups)))
         return ok
 
@@ -611,7 +609,8 @@ class UNetPlan:
     def run(self, x_t, head=True):
         """One denoiser call on the current condition / level projection.  x_t: fp32 NCHW device tensor (B,C,H,W).
         Leaves eps_hat in ``self.eps`` (fp32 NCHW).  head=False: stop before ``final_conv`` and return its (raw) input Act --
-        the caller runs the head fused with the sampler update (``head_sampler_step``)."""
+        the caller runs the head fused with the sampler update (``head_sampler_step``).  Records which buffer fed each layer
+        (``_down_inputs``, ``_mid_inputs``, ``_up_inputs``, ``_x_last``): the train plan's backward walks them in reverse."""
         e, B = self.eng, self.B
         st = e.stream
         e.call("wsr_fill_zero", self.stats.data_ptr(), self.stats.numel() * 8, st)
@@ -619,7 +618,9 @@ class UNetPlan:
         stem = self.downs[0]
         self._stem_input(x_t)
         x = e.conv(stem.xin, stem.conv, stem.y)
+        self._down_inputs, self._mid_inputs, self._up_inputs = {}, {}, {}
         for i, r in enumerate(self.downs[1:], start=1):
+            self._down_inputs[i] = x
             extra = self.cond_up if (self.kind == "srdiff" and i == 2) else None
             if r.kind == "res":
                 x = self._res_block(r, x, extra_res=extra)
@@ -636,17 +637,20 @@ class UNetPlan:
                         side.wait_event(ev)
                         with torch.cuda.stream(side):
                             self._hf_ca(r.ca)
-        for r in self.mids:
+        for i, r in enumerate(self.mids):
+            self._mid_inputs[i] = x
             x = self._res_block(r, x)
         if side is not None:
             ev = torch.cuda.Event()
             ev.record(side)
             main.wait_event(ev)            # join: the up path consumes the skips written by the branch
-        for r in self.ups:
+        for k, r in enumerate(self.ups):
             if r.kind == "res":
                 x = self._res_block(r, r.cat)
             else:
+                self._up_inputs[k] = x
                 x = e.conv(x, r.conv, r.y, upsample=True)
+        self._x_last = x
         if not head:
             return x
         self._head(x)

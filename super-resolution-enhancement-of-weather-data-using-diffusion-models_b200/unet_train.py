@@ -25,12 +25,13 @@ import torch
 
 from . import _native as nat
 from . import taps as T
-from . import taps as taps_mod
 from .engine import Act
 from .unet_plan import UNetPlan, _L
 
 
 class UNetTrainPlan(UNetPlan):
+    feeds_backward = True
+
     def __init__(self, net, batch, device, precision="bf16", strict_tc=False):
         self.drop_p = float(getattr(net, "dropout", 0.0) or 0.0)
         self.drop_seed = 0
@@ -46,9 +47,7 @@ class UNetTrainPlan(UNetPlan):
         self.replay_enabled = True
         self._jobtab = None            # (device WsrPackJob table, njobs, total units, parameter-address signature)
         self.batched_refresh = True     # False: re-pack weights tensor by tensor (the reference the tests compare with)
-        self.fuse_gn = False           # the backward pass reads the normalised activations (a1, a2): keep them materialised
         super().__init__(net, batch, device, precision, strict_tc)
-        self.eng.no_fused_attention = False
         self._grad_layout()
         self._grad_buffers()
 
@@ -605,7 +604,7 @@ class UNetTrainPlan(UNetPlan):
         cf = self.cond_feat
         if getattr(self, "_dcond", None) is None:
             self._dcond = e.new_act(self.B, cf.H, cf.W, cf.C)
-        for q, tp in enumerate(taps_mod.conv_transpose_k8s4_wgrad_taps(cf.H, cf.W)):
+        for q, tp in enumerate(T.conv_transpose_k8s4_wgrad_taps(cf.H, cf.W)):
             e.conv(gy, pc, self._dcond, taps=tp, bias=False, res=self._dcond if q else None, force_simt=True)
 
     def cond_grad(self):
@@ -751,10 +750,11 @@ class UNetTrainPlan(UNetPlan):
         return self.gflat
 
     # ------------------------------------------------------------------------------------------------------------------
-    # forward with the producer / consumer bookkeeping the backward pass needs
+    # forward: UNetPlan.run, recorded once and then replayed
     # ------------------------------------------------------------------------------------------------------------------
     def run(self, x_t):
-        """UNetPlan.run plus a record of which buffer fed each layer (the backward pass walks it in reverse)."""
+        """UNetPlan.run after a weight refresh and a fresh dropout seed; from the second identical call on, a replay of its
+        recorded launch list."""
         e = self.eng
         self.refresh_weights()
         if self.drop_p > 0.0 and self.train_mode:
@@ -769,44 +769,9 @@ class UNetTrainPlan(UNetPlan):
         if record:
             e.rec = []
         try:
-            self._run_body(x_t)
+            super().run(x_t)
         finally:
             lst, e.rec = e.rec, None
         if record:
             self._lists["fwd"], self._lists["fwd_key"] = lst, key
-        return self.eps
-
-    def _run_body(self, x_t):
-        e, B = self.eng, self.B
-        st = e.stream
-        e.call("wsr_fill_zero", self.stats.data_ptr(), self.stats.numel() * 8, st)
-        stem = self.downs[0]
-        self._stem_input(x_t)
-        x = e.conv(stem.xin, stem.conv, stem.y)
-        self._down_inputs = {}
-        for i, r in enumerate(self.downs[1:], start=1):
-            self._down_inputs[i] = x
-            extra = self.cond_up if (self.kind == "srdiff" and i == 2) else None
-            if r.kind == "res":
-                x = self._res_block(r, x, extra_res=extra)
-            else:
-                x = e.conv(x, r.conv, r.y, stride=2, res=extra)
-                if self.has_hfca:
-                    self._hf_ca(r.ca)
-        self._mid_inputs = {}
-        for i, r in enumerate(self.mids):
-            self._mid_inputs[i] = x
-            x = self._res_block(r, x)
-        self._up_inputs = {}
-        for k, r in enumerate(self.ups):
-            if r.kind == "res":
-                x = self._res_block(r, r.cat)
-            else:
-                self._up_inputs[k] = x
-                x = e.conv(x, r.conv, r.y, upsample=True)
-        self._x_last = x
-        self._head(x)
-        if self.C_img != 1:
-            e.call("wsr_nhwc_to_nchw", self.eps_nhwc.ptr, nat.F32, self.eps_nhwc.ld, B, self.C_img, self.H, self.W,
-                   self.eps.data_ptr(), st)
         return self.eps
