@@ -420,6 +420,17 @@ int wsr_final_conv_sampler_step_members(const void* x, int x_ld, int B, int H, i
                                         const float* bias, int Cout, float* eps_out, float* x_state, const float* z,
                                         int64_t z_step_stride, const uint64_t* member_keys, int64_t member_elems, const float* tables,
                                         int T, const int* t_dev, int clip, void* stream);
+/* Multistep (DPM-Solver++(2M)) variants of wsr_sampler_step and wsr_final_conv_sampler_step.  tables: float [5][S] =
+ * (c_recip, c_recipm1, c_x0, c_x, c_prev), row = *t_dev:
+ *   x0 = clamp(c_recip*x - c_recipm1*eps, -1, 1); x_out = c_x0*x0 + c_x*x + c_prev*x0_hist; x0_hist = x0
+ * x0_hist: fp32, same shape as x, the clamped x0 of the previous step; it is NOT read when the row's c_prev == 0 (first and final
+ * steps), so it needs no initialisation.  No noise.  A null x0_hist, tables or (fused) x_state returns WSR_E_INVALID. */
+int wsr_sampler_step_multistep(const float* x, const void* eps, int eps_dtype, float* x0_hist, const float* tables, int S,
+                               const int* t_dev, int clip, float* x_out, int64_t n, void* stream);
+int wsr_final_conv_sampler_step_multistep(const void* x, int x_ld, int B, int H, int W, int Cin, const double* stats, int stats_ld,
+                                          const float* gamma, const float* beta, int groups, float gn_eps, const void* w,
+                                          const float* bias, int Cout, float* eps_out, float* x_state, float* x0_hist,
+                                          const float* tables, int S, const int* t_dev, int clip, void* stream);
 int wsr_head_sampler_supported(int Cin, int Cout, int groups);
 int wsr_pack_head_weight(const float* w_tap_cout_cin, int Cout, int Cin, void* dst, void* stream);
 /* out[b][:] = table[r][:] for b < B, r = *row_index (one row of the per-time-step projection table broadcast to the

@@ -141,6 +141,8 @@ SIGNATURES = {
     "wsr_sampler_step_members": [_P, _P, _I, _P, _L, _P, _L, _P, _I, _P, _I, _P, _L, _P],
     "wsr_final_conv_sampler_step_members": [_P, _I, _I, _I, _I, _I, _P, _I, _P, _P, _I, _F, _P, _P, _I, _P, _P, _P, _L, _P, _L, _P, _I, _P,
                                             _I, _P],
+    "wsr_sampler_step_multistep": [_P, _P, _I, _P, _P, _I, _P, _I, _P, _L, _P],
+    "wsr_final_conv_sampler_step_multistep": [_P, _I, _I, _I, _I, _I, _P, _I, _P, _P, _I, _F, _P, _P, _I, _P, _P, _P, _P, _I, _P, _I, _P],
     "wsr_head_sampler_supported": [_I, _I, _I],
     "wsr_pack_head_weight": [_P, _I, _I, _P, _P],
     "wsr_broadcast_row": [_P, _I, _P, _I, _P, _P],

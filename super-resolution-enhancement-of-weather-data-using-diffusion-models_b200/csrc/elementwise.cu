@@ -515,19 +515,23 @@ __device__ __forceinline__ uint64_t noise_key(uint64_t seed, const uint64_t* __r
   }
 }
 
-template <bool MK>
+// MS = false: the DDPM / DDIM step, tables (c_recip, c_recipm1, coef1, coef2, logvar), noise from the chain z or Philox.
+// MS = true: the multistep (DPM-Solver++(2M)) step, tables (c_recip, c_recipm1, c_x0, c_x, c_prev): x_out = c_x0 x0 + c_x x + c_prev hist,
+// then hist <- x0 (clamped); no noise.  hist is not read when c_prev == 0 (first and final steps), so its initial contents never matter.
+template <bool MK, bool MS>
 __global__ void sampler_step_kernel(const float* x, const void* eps, int edt, const float* __restrict__ z, int64_t z_stride,
-                                    uint64_t seed, const uint64_t* __restrict__ member_keys, int64_t member_groups,
+                                    uint64_t seed, const uint64_t* __restrict__ member_keys, int64_t member_groups, float* __restrict__ hist,
                                     const float* __restrict__ tab, int T, const int* __restrict__ t_dev, int clip, float* xo, int64_t n) {
   const int t = *t_dev;
-  if (z) z += (int64_t)(T - t) * z_stride;
+  if (!MS && z) z += (int64_t)(T - t) * z_stride;
   const float c_recip = tab[t], c_recipm1 = tab[T + t], coef1 = tab[2 * T + t], coef2 = tab[3 * T + t];
-  const float sigma = t > 0 ? __expf(0.5f * tab[4 * T + t]) : 0.f;
+  const float sigma = !MS && t > 0 ? __expf(0.5f * tab[4 * T + t]) : 0.f;
+  const float c_prev = MS ? tab[4 * T + t] : 0.f;
   int64_t g = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;   // group of 4 elements
   int64_t i0 = g * 4;
   if (i0 >= n) return;
   float zz[4] = {0.f, 0.f, 0.f, 0.f};
-  if (t > 0) {
+  if (!MS && t > 0) {
     if (z) {
 #pragma unroll
       for (int j = 0; j < 4; ++j) if (i0 + j < n) zz[j] = z[i0 + j];
@@ -544,7 +548,14 @@ __global__ void sampler_step_kernel(const float* x, const void* eps, int edt, co
     float xv = x[i];
     float x0 = c_recip * xv - c_recipm1 * ld_dt(eps, i, edt);
     if (clip) x0 = fminf(1.f, fmaxf(-1.f, x0));
-    xo[i] = coef1 * x0 + coef2 * xv + sigma * zz[j];
+    if constexpr (MS) {
+      float o = coef1 * x0 + coef2 * xv;
+      if (c_prev != 0.f) o += c_prev * hist[i];
+      hist[i] = x0;
+      xo[i] = o;
+    } else {
+      xo[i] = coef1 * x0 + coef2 * xv + sigma * zz[j];
+    }
   }
 }
 
@@ -839,8 +850,8 @@ extern "C" int wsr_sampler_step(const float* x, const void* eps, int eps_dtype, 
                                 uint64_t seed, const float* tables, int T, const int* t_dev, int clip, float* x_out,
                                 int64_t n, void* stream) {
   WSR_REQUIRE(x && eps && tables && t_dev && x_out && valid_dtype(eps_dtype) && T > 0 && n > 0, WSR_E_INVALID, "sampler_step: bad argument");
-  sampler_step_kernel<false><<<blocks_for((n + 3) / 4, 256), 256, 0, (cudaStream_t)stream>>>(x, eps, eps_dtype, z, z_step_stride, seed, nullptr, 1,
-                                                                                              tables, T, t_dev, clip, x_out, n);
+  sampler_step_kernel<false, false><<<blocks_for((n + 3) / 4, 256), 256, 0, (cudaStream_t)stream>>>(x, eps, eps_dtype, z, z_step_stride, seed, nullptr, 1,
+                                                                                                     nullptr, tables, T, t_dev, clip, x_out, n);
   WSR_LAUNCH_OK();
   return WSR_OK;
 }
@@ -852,8 +863,18 @@ extern "C" int wsr_sampler_step_members(const float* x, const void* eps, int eps
               "sampler_step_members: bad argument");
   WSR_REQUIRE(member_elems > 0 && member_elems % 4 == 0, WSR_E_INVALID, "sampler_step_members: member_elems=%lld is not a positive multiple of 4",
               (long long)member_elems);
-  sampler_step_kernel<true><<<blocks_for((n + 3) / 4, 256), 256, 0, (cudaStream_t)stream>>>(x, eps, eps_dtype, z, z_step_stride, 0, member_keys,
-                                                                                             member_elems / 4, tables, T, t_dev, clip, x_out, n);
+  sampler_step_kernel<true, false><<<blocks_for((n + 3) / 4, 256), 256, 0, (cudaStream_t)stream>>>(x, eps, eps_dtype, z, z_step_stride, 0, member_keys,
+                                                                                                    member_elems / 4, nullptr, tables, T, t_dev, clip, x_out, n);
+  WSR_LAUNCH_OK();
+  return WSR_OK;
+}
+
+extern "C" int wsr_sampler_step_multistep(const float* x, const void* eps, int eps_dtype, float* x0_hist, const float* tables, int S,
+                                          const int* t_dev, int clip, float* x_out, int64_t n, void* stream) {
+  WSR_REQUIRE(x && eps && x0_hist && tables && t_dev && x_out && valid_dtype(eps_dtype) && S > 0 && n > 0, WSR_E_INVALID,
+              "sampler_step_multistep: bad argument");
+  sampler_step_kernel<false, true><<<blocks_for((n + 3) / 4, 256), 256, 0, (cudaStream_t)stream>>>(x, eps, eps_dtype, nullptr, 0, 0, nullptr, 1,
+                                                                                                    x0_hist, tables, S, t_dev, clip, x_out, n);
   WSR_LAUNCH_OK();
   return WSR_OK;
 }

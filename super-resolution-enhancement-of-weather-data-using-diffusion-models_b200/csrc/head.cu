@@ -29,6 +29,7 @@ struct HeadParams {
   float* xs;                               // fp32 NCHW state x_t -> x_{t-1} in place, or null (convolution only)
   const float* z; long long z_stride; unsigned long long seed; const float* tab; int T; const int* t_dev; int clip;
   const unsigned long long* member_keys; long long member_groups;   // ensemble batch (MK): per-member Philox keys, member elements / 4
+  float* hist;                             // multistep (MS): fp32 NCHW x0 of the previous step, read when c_prev != 0, then overwritten
 };
 
 __device__ __forceinline__ void head_randn4(uint64_t seed, uint32_t tag, uint64_t grp, float (&z)[4]) {
@@ -47,7 +48,8 @@ __device__ __forceinline__ void head_randn4(uint64_t seed, uint32_t tag, uint64_
 
 // shared memory: tile [Cin/64 planes][6 rows][130 cols][64 ch] bf16 | weights bf16 as ldmatrix-ready 8x8 blocks
 // [plane][tap][16-channel step][k half][n = 8 output channels (zero above Cout)][8 channels] | scale[Cin] shift[Cin] | group moments
-template <int COUT, bool MK>
+// MS: the epilogue is the multistep update of wsr_sampler_step_multistep (tables (c_recip, c_recipm1, c_x0, c_x, c_prev), no noise)
+template <int COUT, bool MK, bool MS>
 __global__ void __launch_bounds__(kHeadThreads) head_sampler_kernel(const HeadParams p) {
   extern __shared__ __align__(16) uint8_t hsm[];
   constexpr int TR = kHeadRows + 2, TC = kHeadCols + 2;
@@ -208,11 +210,16 @@ __global__ void __launch_bounds__(kHeadThreads) head_sampler_kernel(const HeadPa
   int t = 0;
   float c_recip = 0.f, c_recipm1 = 0.f, coef1 = 0.f, coef2 = 0.f, sigma = 0.f;
   const float* zt = nullptr;
+  float c_prev = 0.f;
   if (p.xs) {
     t = *p.t_dev;
     c_recip = p.tab[t]; c_recipm1 = p.tab[p.T + t]; coef1 = p.tab[2 * p.T + t]; coef2 = p.tab[3 * p.T + t];
-    sigma = t > 0 ? __expf(0.5f * p.tab[4 * p.T + t]) : 0.f;
-    if (p.z) zt = p.z + (long long)(p.T - t) * p.z_stride;
+    if constexpr (MS) {
+      c_prev = p.tab[4 * p.T + t];
+    } else {
+      sigma = t > 0 ? __expf(0.5f * p.tab[4 * p.T + t]) : 0.f;
+      if (p.z) zt = p.z + (long long)(p.T - t) * p.z_stride;
+    }
   }
 #pragma unroll
   for (int px = 0; px < 2; ++px) {
@@ -223,7 +230,15 @@ __global__ void __launch_bounds__(kHeadThreads) head_sampler_kernel(const HeadPa
       const long long i = (((long long)n * COUT + co) * p.H + gy) * p.W + gx;
       const float e = outv[px][co];
       if (p.eps_out) p.eps_out[i] = e;
-      if (p.xs) {
+      if (MS && p.xs) {
+        const float xv = p.xs[i];
+        float x0v = c_recip * xv - c_recipm1 * e;
+        if (p.clip) x0v = fminf(1.f, fmaxf(-1.f, x0v));
+        float o = coef1 * x0v + coef2 * xv;
+        if (c_prev != 0.f) o += c_prev * p.hist[i];
+        p.hist[i] = x0v;
+        p.xs[i] = o;
+      } else if (p.xs) {
         float zz = 0.f;
         if (t > 0) {
           if (zt) zz = zt[i];
@@ -262,16 +277,16 @@ static size_t head_smem_bytes(int Cin, int Cout, int groups) {
   return (size_t)(Cin / 64) * (kHeadRows + 2) * (kHeadCols + 2) * 128 + (size_t)(Cin / 64) * 9 * 4 * 2 * 128 + (size_t)(2 * Cin + 2 * groups) * 4;
 }
 
-template <int COUT, bool MK>
+template <int COUT, bool MK, bool MS>
 static int launch_head(const HeadParams& p, cudaStream_t st) {
   const size_t smem = head_smem_bytes(p.Cin, COUT, p.groups);
   static size_t attr = 0;
   if (smem > attr) {
-    WSR_CUDA_OK(cudaFuncSetAttribute(head_sampler_kernel<COUT, MK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    WSR_CUDA_OK(cudaFuncSetAttribute(head_sampler_kernel<COUT, MK, MS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     attr = smem;
   }
   const int tiles = ((p.W + kHeadCols - 1) / kHeadCols) * ((p.H + kHeadRows - 1) / kHeadRows);
-  WSR_CUDA_OK(launch_pdl(head_sampler_kernel<COUT, MK>, dim3(tiles, p.B), dim3(kHeadThreads), smem, st, p));
+  WSR_CUDA_OK(launch_pdl(head_sampler_kernel<COUT, MK, MS>, dim3(tiles, p.B), dim3(kHeadThreads), smem, st, p));
   return WSR_OK;
 }
 
@@ -295,8 +310,8 @@ extern "C" int wsr_pack_head_weight(const float* w, int Cout, int Cin, void* dst
 static int head_sampler_step(const void* x, int x_ld, int B, int H, int W, int Cin, const double* stats, int stats_ld,
                              const float* gamma, const float* beta, int groups, float gn_eps, const void* w, const float* bias, int Cout,
                              float* eps_out, float* x_state, const float* z, int64_t z_step_stride, uint64_t seed,
-                             const uint64_t* member_keys, int64_t member_elems, const float* tables, int T, const int* t_dev, int clip,
-                             void* stream) {
+                             const uint64_t* member_keys, int64_t member_elems, float* hist, const float* tables, int T, const int* t_dev,
+                             int clip, void* stream) {
   WSR_REQUIRE(x && stats && gamma && beta && w, WSR_E_INVALID, "final_conv_sampler_step: null pointer");
   WSR_REQUIRE(B > 0 && B <= 65535 && H > 0 && W > 0, WSR_E_INVALID, "final_conv_sampler_step: bad shape");
   WSR_REQUIRE(wsr_head_sampler_supported(Cin, Cout, groups), WSR_E_UNSUPPORTED,
@@ -310,21 +325,29 @@ static int head_sampler_step(const void* x, int x_ld, int B, int H, int W, int C
   p.stats = stats; p.stats_ld = stats_ld; p.gamma = gamma; p.beta = beta; p.groups = groups; p.gn_eps = gn_eps;
   p.w = (const uint4*)w; p.bias = bias; p.eps_out = eps_out; p.xs = x_state; p.z = z; p.z_stride = z_step_stride; p.seed = seed;
   p.tab = tables; p.T = T; p.t_dev = t_dev; p.clip = clip;
-  p.member_keys = (const unsigned long long*)member_keys; p.member_groups = member_elems / 4;
+  p.member_keys = (const unsigned long long*)member_keys; p.member_groups = member_elems / 4; p.hist = hist;
   cudaStream_t st = (cudaStream_t)stream;
+  if (hist) {
+    switch (Cout) {
+      case 1: return launch_head<1, false, true>(p, st);
+      case 2: return launch_head<2, false, true>(p, st);
+      case 3: return launch_head<3, false, true>(p, st);
+      default: return launch_head<4, false, true>(p, st);
+    }
+  }
   if (member_keys) {
     switch (Cout) {
-      case 1: return launch_head<1, true>(p, st);
-      case 2: return launch_head<2, true>(p, st);
-      case 3: return launch_head<3, true>(p, st);
-      default: return launch_head<4, true>(p, st);
+      case 1: return launch_head<1, true, false>(p, st);
+      case 2: return launch_head<2, true, false>(p, st);
+      case 3: return launch_head<3, true, false>(p, st);
+      default: return launch_head<4, true, false>(p, st);
     }
   }
   switch (Cout) {
-    case 1: return launch_head<1, false>(p, st);
-    case 2: return launch_head<2, false>(p, st);
-    case 3: return launch_head<3, false>(p, st);
-    default: return launch_head<4, false>(p, st);
+    case 1: return launch_head<1, false, false>(p, st);
+    case 2: return launch_head<2, false, false>(p, st);
+    case 3: return launch_head<3, false, false>(p, st);
+    default: return launch_head<4, false, false>(p, st);
   }
 }
 
@@ -334,7 +357,7 @@ extern "C" int wsr_final_conv_sampler_step(const void* x, int x_ld, int B, int H
                                            int64_t z_step_stride, uint64_t seed, const float* tables, int T, const int* t_dev,
                                            int clip, void* stream) {
   return head_sampler_step(x, x_ld, B, H, W, Cin, stats, stats_ld, gamma, beta, groups, gn_eps, w, bias, Cout, eps_out, x_state, z,
-                           z_step_stride, seed, nullptr, 0, tables, T, t_dev, clip, stream);
+                           z_step_stride, seed, nullptr, 0, nullptr, tables, T, t_dev, clip, stream);
 }
 
 extern "C" int wsr_final_conv_sampler_step_members(const void* x, int x_ld, int B, int H, int W, int Cin, const double* stats,
@@ -347,5 +370,14 @@ extern "C" int wsr_final_conv_sampler_step_members(const void* x, int x_ld, int 
   WSR_REQUIRE(member_elems > 0 && member_elems % 4 == 0, WSR_E_INVALID,
               "final_conv_sampler_step_members: member_elems=%lld is not a positive multiple of 4", (long long)member_elems);
   return head_sampler_step(x, x_ld, B, H, W, Cin, stats, stats_ld, gamma, beta, groups, gn_eps, w, bias, Cout, eps_out, x_state, z,
-                           z_step_stride, 0, member_keys, member_elems, tables, T, t_dev, clip, stream);
+                           z_step_stride, 0, member_keys, member_elems, nullptr, tables, T, t_dev, clip, stream);
+}
+
+extern "C" int wsr_final_conv_sampler_step_multistep(const void* x, int x_ld, int B, int H, int W, int Cin, const double* stats,
+                                                     int stats_ld, const float* gamma, const float* beta, int groups, float gn_eps,
+                                                     const void* w, const float* bias, int Cout, float* eps_out, float* x_state,
+                                                     float* x0_hist, const float* tables, int S, const int* t_dev, int clip, void* stream) {
+  WSR_REQUIRE(x_state && x0_hist && tables, WSR_E_INVALID, "final_conv_sampler_step_multistep: null state, history or tables");
+  return head_sampler_step(x, x_ld, B, H, W, Cin, stats, stats_ld, gamma, beta, groups, gn_eps, w, bias, Cout, eps_out, x_state, nullptr,
+                           0, 0, nullptr, 0, x0_hist, tables, S, t_dev, clip, stream);
 }

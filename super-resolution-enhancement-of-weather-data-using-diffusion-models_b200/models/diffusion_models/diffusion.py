@@ -11,6 +11,7 @@ import torch
 from torch import nn
 
 from ... import _native as nat
+from . import samplers
 from .nn_modules.functional_layers import default
 from .sheduler import make_beta_schedule
 
@@ -63,6 +64,8 @@ class GaussianDiffusion(nn.Module):
         self.use_cuda_graph = True
         self.sample_seed = None          # None -> derive from torch's global generator at every loop
         self._sampler_tables = None
+        self.sampler = ("ddpm", None, None)   # set_sampler's (name, steps, eta)
+        self._fewer_step_tables = None
 
     # ---- schedule (reference :49-96) --------------------------------------------------------------------------------
     def set_new_noise_schedule(self, schedule_opt, device):
@@ -93,14 +96,41 @@ class GaussianDiffusion(nn.Module):
         for name, arr in tables.items():
             self.register_buffer(name, torch.tensor(arr, dtype=torch.float32, device=device))
         self._sampler_tables = None
+        self._fewer_step_tables = None
 
-    def _tables_dev(self):
+    def set_sampler(self, name="ddpm", steps=None, eta=None):
+        """Select the reverse loop's sampler (samplers.py): 'ddpm' (the reference's ancestral loop over all T steps, the default),
+        'ddim' (``steps`` of the T timesteps, ``eta`` in [0, inf), default 0; eta = 1 is the respaced ancestral sampler) or 'dpmpp2m'
+        (DPM-Solver++(2M), deterministic).  steps=None is every timestep.  ``super_resolution``, ``p_sample_loop``,
+        ``super_resolution_ensemble`` and ``begin_loop`` follow it; ``p_sample`` stays the DDPM step."""
+        T = getattr(self, "num_timesteps", None)
+        if T is None:
+            raise ValueError("set_sampler needs the noise schedule (set_new_noise_schedule) first")
+        samplers.check(name, steps, eta, T)
+        self.sampler = (name, steps, eta)
+        self._fewer_step_tables = None
+
+    def _ddpm_tables_dev(self):
         """[5][T] fp32 table consumed by wsr_sampler_step + the T noise levels sqrt(abar_prev[t+1]) (:159-160)."""
         if self._sampler_tables is None or self._sampler_tables[0].device != self.betas.device:
             tab = torch.stack([getattr(self, n) for n in _TABLE_ORDER], 0).contiguous()
             levels = torch.tensor(self.sqrt_alphas_cumprod_prev[1:].astype(np.float32), device=self.betas.device)
             self._sampler_tables = (tab, levels)
         return self._sampler_tables
+
+    def _tables_dev(self):
+        """The selected sampler's [5][S] fp32 table and its S noise levels, rows in device-counter order (samplers.py)."""
+        name, steps, eta = self.sampler
+        if name == "ddpm":
+            return self._ddpm_tables_dev()
+        if self._fewer_step_tables is None or self._fewer_step_tables[0].device != self.betas.device:
+            # the schedule may have changed since set_sampler: re-validate against the current T
+            name, S, eta = samplers.check(name, steps, eta, self.num_timesteps)
+            abar = np.square(self.sqrt_alphas_cumprod_prev[1:])
+            tab, levels = samplers.tables(name, abar, S, eta)
+            self._fewer_step_tables = (torch.tensor(tab, dtype=torch.float32, device=self.betas.device),
+                                       torch.tensor(levels, dtype=torch.float32, device=self.betas.device))
+        return self._fewer_step_tables
 
     def set_loss(self, device):
         if self.loss_type not in ('l1', 'l2'):
@@ -136,32 +166,38 @@ class GaussianDiffusion(nn.Module):
             raise NotImplementedError("unconditional sampling is not part of the accelerated path")
         plan = self._plan(x.shape[0], x.device)
         self._set_condition(plan, condition_x)
-        tab, levels = self._tables_dev()
+        tab, levels = self._ddpm_tables_dev()
         plan.set_level_table(levels)
         t_dev = torch.tensor([int(t)], dtype=torch.int32, device=x.device)
         xb = x.to(torch.float32).contiguous().clone()
         self._step(plan, xb, t_dev, tab, None, 0, self._next_seed(), clip_denoised)
         return xb
 
-    def _step(self, plan, x, t_dev, tab, z, z_stride, seed, clip=True, members=None):
-        """members: None, or (device int64 key table, elements per member) -- an ensemble batch with member-keyed noise."""
+    def _step(self, plan, x, t_dev, tab, z, z_stride, seed, clip=True, members=None, hist=None):
+        """members: None, or (device int64 key table, elements per member) -- an ensemble batch with member-keyed noise.
+        hist: None (DDPM / DDIM tables), or the fp32 x0 history of a multistep (DPM-Solver++(2M)) table; the step then draws no noise.
+        The table's row count is the loop length (T for DDPM, S for the fewer-step samplers)."""
         st = plan.eng.stream
+        S = tab.shape[1]
         plan.select_level_row(t_dev)
         if plan.can_fuse_head():
             # head (GroupNorm + Swish + conv3x3) and the reverse-step update in one HBM-bound kernel
             feat = plan.run(x, head=False)
-            plan.head_sampler_step(feat, x, tab, self.num_timesteps, t_dev, z, z_stride, seed, clip, members=members)
+            plan.head_sampler_step(feat, x, tab, S, t_dev, z, z_stride, seed, clip, members=members, hist=hist)
             plan.eng.call("wsr_step_counter_add", t_dev.data_ptr(), -1, st)
             return
         plan.run(x)
         zp = 0 if z is None else z.data_ptr()
-        if members is None:
+        if hist is not None:
+            plan.eng.call("wsr_sampler_step_multistep", x.data_ptr(), plan.eps.data_ptr(), nat.F32, hist.data_ptr(), tab.data_ptr(), S,
+                          t_dev.data_ptr(), 1 if clip else 0, x.data_ptr(), x.numel(), st, nbytes=x.numel() * 20)
+        elif members is None:
             plan.eng.call("wsr_sampler_step", x.data_ptr(), plan.eps.data_ptr(), nat.F32, zp, z_stride, seed, tab.data_ptr(),
-                          self.num_timesteps, t_dev.data_ptr(), 1 if clip else 0, x.data_ptr(), x.numel(), st,
+                          S, t_dev.data_ptr(), 1 if clip else 0, x.data_ptr(), x.numel(), st,
                           nbytes=x.numel() * (16 if z is not None else 12))
         else:
             plan.eng.call("wsr_sampler_step_members", x.data_ptr(), plan.eps.data_ptr(), nat.F32, zp, z_stride, members[0].data_ptr(),
-                          members[1], tab.data_ptr(), self.num_timesteps, t_dev.data_ptr(), 1 if clip else 0, x.data_ptr(), x.numel(),
+                          members[1], tab.data_ptr(), S, t_dev.data_ptr(), 1 if clip else 0, x.data_ptr(), x.numel(),
                           st, nbytes=x.numel() * (16 if z is not None else 12))
         plan.eng.call("wsr_step_counter_add", t_dev.data_ptr(), -1, st)
 
@@ -172,12 +208,12 @@ class GaussianDiffusion(nn.Module):
 
     @torch.no_grad()
     def _reverse_loop(self, plan, shape, noise_chain=None, seed=None, steps=None, collect_eps=False, member_keys=None):
-        """T reverse steps on the plan's current condition.  noise_chain: optional injected noise [T+1, *shape]
-        (index 0 = initial image, index T-t = noise of step t) for parity runs; otherwise Philox noise from ``seed``, or, with
-        ``member_keys`` (R Philox keys), from key member_keys[m] for the m-th of R equal member slices of the batch.
-        Returns the final x_0 (fp32 NCHW)."""
+        """S reverse steps of the selected sampler (S = T for DDPM) on the plan's current condition.  noise_chain: optional injected
+        noise [S+1, *shape] (index 0 = initial image, index S-t = noise of the step at counter t) for parity runs; otherwise Philox
+        noise from ``seed``, or, with ``member_keys`` (R Philox keys), from key member_keys[m] for the m-th of R equal member slices of
+        the batch.  Returns the final x_0 (fp32 NCHW)."""
         loop = self.begin_loop(plan, shape, noise_chain, seed, member_keys)
-        n_steps = self.num_timesteps if steps is None else min(int(steps), self.num_timesteps)
+        n_steps = loop.S if steps is None else min(int(steps), loop.S)
         eps_log = []
         # first step eagerly (lazy initialisation of kernel attributes happens here), the rest as graph replays
         loop.step()
@@ -311,17 +347,19 @@ class GaussianDiffusion(nn.Module):
 
 
 class ReverseLoop:
-    """State of one reverse (p_sample) loop: the image x (updated in place), the device-side step counter and the
-    captured CUDA graph of one step.  ``step()`` launches one step eagerly, ``capture()`` records the same launches
-    into a graph, ``replay()`` replays it -- the step index lives on the device, so every replay advances the chain."""
+    """State of one reverse loop of the diffusion's sampler: the image x (updated in place), the device-side step counter
+    (S-1 -> 0, S = T for DDPM), the x0 history of a multistep sampler and the captured CUDA graph of one step.  ``step()``
+    launches one step eagerly, ``capture()`` records the same launches into a graph, ``replay()`` replays it -- the step index
+    and the history live on the device, so every replay advances the chain."""
 
     def __init__(self, diffusion, plan, shape, noise_chain=None, seed=None, member_keys=None):
         self.diffusion, self.plan = diffusion, plan
         dev = plan.eng.device
-        T = diffusion.num_timesteps
         self.tab, levels = diffusion._tables_dev()
+        self.S = S = self.tab.shape[1]
         plan.set_level_table(levels)
         self.x = torch.empty(shape, device=dev, dtype=torch.float32)
+        self.hist = torch.zeros(shape, device=dev, dtype=torch.float32) if diffusion.sampler[0] == "dpmpp2m" else None
         # an explicit seed is still made rank-distinct: sharded ranks pass the same value (bench.py, sample.py)
         self.seed = diffusion._next_seed() if seed is None else rank_stream_seed(int(seed))
         self.members = None
@@ -335,7 +373,7 @@ class ReverseLoop:
             self.members = (keys, n // keys.numel())
         if noise_chain is not None:
             self.z = noise_chain.to(device=dev, dtype=torch.float32).contiguous()
-            assert self.z.shape[0] == T + 1 and tuple(self.z.shape[1:]) == tuple(shape)
+            assert self.z.shape[0] == S + 1 and tuple(self.z.shape[1:]) == tuple(shape)
             self.x.copy_(self.z[0])
             self.z_stride = self.x.numel()
         else:
@@ -345,14 +383,14 @@ class ReverseLoop:
             else:
                 nat.call("wsr_randn_members", self.x.data_ptr(), self.x.numel(), self.members[0].data_ptr(), self.members[1],
                          0xFFFFFFFF, plan.eng.stream)
-        self.t_dev = torch.tensor([T - 1], dtype=torch.int32, device=dev)
+        self.t_dev = torch.tensor([S - 1], dtype=torch.int32, device=dev)
         self.graph = None
 
     def reset_counter(self, t=None):
-        self.t_dev.fill_(self.diffusion.num_timesteps - 1 if t is None else int(t))
+        self.t_dev.fill_(self.S - 1 if t is None else int(t))
 
     def step(self):
-        self.diffusion._step(self.plan, self.x, self.t_dev, self.tab, self.z, self.z_stride, self.seed, members=self.members)
+        self.diffusion._step(self.plan, self.x, self.t_dev, self.tab, self.z, self.z_stride, self.seed, members=self.members, hist=self.hist)
 
     def capture(self):
         torch.cuda.synchronize(self.plan.eng.device)

@@ -3,6 +3,7 @@
     python sample.py -c CONFIG.json -p MODEL_PATH -o OUT_DIR -gpu 0 [-n N]
     torchrun --nproc-per-node 8 sample.py -c CONFIG.json -o OUT_DIR -gpu 0,1,2,3,4,5,6,7     # batch-sharded
     python sample.py -c CONFIG.json -o OUT_DIR --ensemble 16 [--seed S]                      # 16 members per condition
+    python sample.py -c CONFIG.json -o OUT_DIR --sampler dpmpp2m --steps 20                  # 20 network calls instead of T
 
 Builds the model through the reference's registry path (Config -> create_model -> DDPM -> define_diffusion),
 ``prepare_to_eval``, ``feed_data``, ``generate_sr``; writes the super-resolved fields as ``sr.npy`` (the reference's
@@ -13,7 +14,10 @@ random-init weights (smoke / benchmarking).
 ``ensemble_mean.npy`` and ``ensemble_spread.npy`` (unbiased), their ``*_physical.npy`` versions with a store, and, when the batch
 carries HR, ``ensemble_scores.json`` (training.metrics.EnsembleScores; physical units with a store).  Under torchrun the MEMBERS are
 sharded (rank r runs a contiguous member range) and rank 0 gathers them; the condition batch is not split.  ``--seed S`` fixes the
-Philox seed (member m uses member_key(S, m); member 0 is the plain run with seed S)."""
+Philox seed (member m uses member_key(S, m); member 0 is the plain run with seed S).
+
+``--sampler {ddpm,ddim,dpmpp2m} --steps S --eta E`` selects the reverse loop (GaussianDiffusion.set_sampler): the reference's DDPM over
+all T steps (default), DDIM(eta) or DPM-Solver++(2M) over S of the T trained timesteps.  It applies to plain, sharded and ensemble runs."""
 import argparse
 import os
 import sys
@@ -26,7 +30,7 @@ sys.path.insert(0, os.path.dirname(_HERE))
 import wsr  # noqa: E402
 
 
-def main(argv=None):
+def parse_args(argv=None):
     ap = argparse.ArgumentParser()
     ap.add_argument("-c", "--config", type=str, required=True, help="JSON file for configuration")
     ap.add_argument("-p", "--model_path", type=str, default=None, help="Path to trained model")
@@ -38,7 +42,22 @@ def main(argv=None):
     ap.add_argument("-d", "--date", type=str, default=None)
     ap.add_argument("--ensemble", type=int, default=None, help="members per condition (ensemble sampling)")
     ap.add_argument("--seed", type=int, default=None, help="Philox seed of the sampler")
-    args = ap.parse_args(argv)
+    ap.add_argument("--sampler", type=str, default=None, choices=["ddpm", "ddim", "dpmpp2m"],
+                    help="reverse-loop sampler (default ddpm: every timestep of the schedule)")
+    ap.add_argument("--steps", type=int, default=None, help="network calls of a ddim / dpmpp2m loop (default: every timestep)")
+    ap.add_argument("--eta", type=float, default=None, help="DDIM noise scale (default 0: deterministic; 1: respaced ancestral)")
+    return ap.parse_args(argv)
+
+
+def sampler_options(args):
+    """set_sampler's keyword arguments from the command line, or None when no sampler flag was given (the default DDPM loop)."""
+    if args.sampler is None and args.steps is None and args.eta is None:
+        return None
+    return dict(name=args.sampler or "ddpm", steps=args.steps, eta=args.eta)
+
+
+def main(argv=None):
+    args = parse_args(argv)
 
     Config = wsr.sub("configs.config").Config
     create_model = wsr.sub("models.base_model").create_model
@@ -77,6 +96,12 @@ def main(argv=None):
         batch, months = next(iter(data.batches_from_opt(opt, "val")))
     if args.seed is not None:
         model._net().sample_seed = args.seed
+    opts = sampler_options(args)
+    if opts is not None:
+        try:
+            model._net().set_sampler(**opts)
+        except ValueError as e:
+            raise SystemExit("sample.py: %s" % e)
     if args.ensemble is not None:
         _ensemble(args, model, batch, months, handler, par, rank, world)
         if world > 1:

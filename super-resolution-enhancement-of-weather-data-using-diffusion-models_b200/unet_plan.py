@@ -589,9 +589,10 @@ class UNetPlan:
                                     and bool(nat.call("wsr_head_sampler_supported", self.final_cin, self.C_img, self.groups)))
         return ok
 
-    def head_sampler_step(self, feat, x_state, tab, T, t_dev, z, z_stride, seed, clip, members=None):
+    def head_sampler_step(self, feat, x_state, tab, T, t_dev, z, z_stride, seed, clip, members=None, hist=None):
         """eps_hat = final_conv(feat) and x_state <- reverse-step update, one launch; eps_hat is also left in ``self.eps``.
-        members: None, or (device key table, elements per member) for member-keyed noise (wsr_final_conv_sampler_step_members)."""
+        members: None, or (device key table, elements per member) for member-keyed noise (wsr_final_conv_sampler_step_members).
+        hist: None, or the fp32 x0 history of a multistep table (wsr_final_conv_sampler_step_multistep; z, seed and members unused)."""
         e = self.eng
         assert feat.stats_ptr and feat.C == self.final_cin and feat.dt == nat.BF16
         npix = self.B * self.H * self.W
@@ -601,7 +602,10 @@ class UNetPlan:
         tail = (tab.data_ptr(), T, t_dev.data_ptr(), 1 if clip else 0, e.stream)
         cost = dict(tag="head_sampler", flops=2 * npix * 9 * feat.C * self.C_img,
                     nbytes=npix * (feat.C * 2 + self.C_img * (16 if z is not None else 12)))
-        if members is None:
+        if hist is not None:
+            cost["nbytes"] = npix * (feat.C * 2 + self.C_img * 20)
+            e.call("wsr_final_conv_sampler_step_multistep", *head[:-2], hist.data_ptr(), *tail, **cost)
+        elif members is None:
             e.call("wsr_final_conv_sampler_step", *head, seed, *tail, **cost)
         else:
             e.call("wsr_final_conv_sampler_step_members", *head, members[0].data_ptr(), members[1], *tail, **cost)
