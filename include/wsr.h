@@ -454,6 +454,13 @@ int wsr_noise_loss(const float* noise, const float* eps, int64_t n, int l2, doub
  * 1 - beta is rounded to fp32 exactly as torch does. */
 int wsr_adam_step(float* p, const float* g, float* m, float* v, int64_t n, double lr, double beta1, double beta2, double eps,
                   double weight_decay, int step, void* stream);
+/* wsr_adam_step (p, m, v bit-identical) that also updates an exponential moving average of the parameters from the new value
+ * p' it has just computed: ema = ema * d + (1 - d) * p', three separately rounded fp32 operations like torch's expression with a
+ * Python-float d; d == 0 is an exact copy ema = p' (whatever ema held, NaN included).  The library is built with
+ * --use_fast_math, so a denormal result is flushed to zero where torch would keep it.  WSR_E_INVALID, nothing written, for a
+ * null pointer, n <= 0, step <= 0, ema_decay outside [0, 1), or an ema range that overlaps p, g, m or v. */
+int wsr_adam_step_ema(float* p, const float* g, float* m, float* v, float* ema, int64_t n, double lr, double beta1, double beta2,
+                      double eps, double weight_decay, int step, double ema_decay, void* stream);
 
 #ifdef __cplusplus
 }

@@ -169,6 +169,7 @@ SIGNATURES = {
     "wsr_fd_backward_workspace_bytes": [_I, _I, _I, _I],
     "wsr_fd_backward": [_P, _I, _I, _I, _I, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P],
     "wsr_adam_step": [_P, _P, _P, _P, _L, C.c_double, C.c_double, C.c_double, C.c_double, C.c_double, _I, _P],
+    "wsr_adam_step_ema": [_P, _P, _P, _P, _P, _L, C.c_double, C.c_double, C.c_double, C.c_double, C.c_double, _I, C.c_double, _P],
 }
 _RESTYPE = {"wsr_fd_precompute_workspace_bytes": C.c_int64, "wsr_fd_backward_workspace_bytes": C.c_int64}
 # functions whose return value is data, not a status

@@ -6,13 +6,15 @@ runs unchanged on the CUDA path.
                 parameter gradient as ``p.grad`` (a view into the plan's flat gradient buffer).
 ``NoiseLossFn`` sum-reduced L1 / L2 between the injected noise and eps_hat (diffusion.py:98-110) via ``wsr_noise_loss``.
 ``FusedAdam``   torch.optim.Adam-compatible optimizer (same state_dict layout) whose update is ``wsr_adam_step``: one
-                launch over the flat parameter buffer when the parameters were flattened by the train plan.
+                launch over the flat parameter buffer when the parameters were flattened by the train plan.  Optionally keeps
+                an EMA of the weights, updated in the same launch (``wsr_adam_step_ema``).
 """
 import torch
 
 from . import _native as nat
 
 weights_epoch = 0          # bumped by every optimizer step that writes parameters through raw pointers
+weights_swapped = False    # True inside DDPM.ema_weights(): a training forward there is refused (see its docstring)
 
 
 class DenoiseFn(torch.autograd.Function):
@@ -20,6 +22,9 @@ class DenoiseFn(torch.autograd.Function):
     def forward(ctx, anchor, net, cond, x_t, time):
         """cond, x_t: the split of the UNet's input (``PlannedUNet._split``).  A condition that requires grad -- SRDiff with a
         trainable encoder, cat(feas[2::3]) -- gets its gradient (``UNetTrainPlan.cond_grad``) back into the encoder's backward pass."""
+        if weights_swapped:
+            raise RuntimeError("training forward inside DDPM.ema_weights(): the train plan would keep EMA-derived level projections "
+                               "and condition weights for the first training forward after the swap back")
         b = x_t.shape[0]
         pl = net.train_plan(b, x_t.device)
         pl.train_mode = bool(net.training)
@@ -68,29 +73,75 @@ class NoiseLossFn(torch.autograd.Function):
         return None, grad * go.to(grad.dtype), None
 
 
+def check_ema_schedule(sched):
+    """``train.ema_scheduler`` of a config -> (step_start_ema, update_ema_every, ema_decay); ValueError when a key is missing or
+    out of range."""
+    if not isinstance(sched, dict):
+        raise ValueError("EMA needs train.ema_scheduler {step_start_ema, update_ema_every, ema_decay} in the config")
+    missing = [k for k in ("step_start_ema", "update_ema_every", "ema_decay") if sched.get(k) is None]
+    if missing:
+        raise ValueError("train.ema_scheduler lacks %s" % ", ".join(missing))
+    start, every, decay = int(sched["step_start_ema"]), int(sched["update_ema_every"]), float(sched["ema_decay"])
+    if every < 1:
+        raise ValueError("train.ema_scheduler.update_ema_every must be >= 1 (got %d)" % every)
+    if start < 0:
+        raise ValueError("train.ema_scheduler.step_start_ema must be >= 0 (got %d)" % start)
+    if not 0.0 <= decay < 1.0:
+        raise ValueError("train.ema_scheduler.ema_decay must be in [0, 1) (got %r)" % decay)
+    return start, every, decay
+
+
+def ema_action(step, start, every):
+    """What the s-th optimizer step (s = 1, 2, ...) does to the EMA, with k = s - 1: 'skip' when k % every != 0, else 'copy'
+    (ema = p) while k < start, else 'blend' (ema = ema * d + (1 - d) * p)."""
+    k = step - 1
+    if k % every != 0:
+        return "skip"
+    return "copy" if k < start else "blend"
+
+
 class FusedAdam(torch.optim.Optimizer):
     """Adam with torch.optim.Adam's arithmetic and state layout (``step``, ``exp_avg``, ``exp_avg_sq`` per parameter);
-    amsgrad / maximize / capturable are not supported (the reference uses none of them)."""
+    amsgrad / maximize / capturable are not supported (the reference uses none of them).
 
-    def __init__(self, params, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, weight_decay=0.0):
+    ``ema=(step_start_ema, update_ema_every, ema_decay)`` also keeps an exponential moving average of every parameter it steps
+    (``ema_action``), updated inside the Adam launch by ``wsr_adam_step_ema``.  The averages live in ``self.ema`` (parameter ->
+    tensor), outside ``state_dict()``, which stays torch.optim.Adam's."""
+
+    def __init__(self, params, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, weight_decay=0.0, ema=None):
         super().__init__(params, dict(lr=lr, betas=betas, eps=eps, weight_decay=weight_decay))
         self._flat = None
+        self.ema, self.ema_schedule = None, None
+        if ema is not None:
+            self.enable_ema(ema)
+
+    @torch.no_grad()
+    def enable_ema(self, schedule):
+        """Start the EMA from the current parameter values."""
+        start, every, decay = schedule
+        self.ema_schedule = (int(start), int(every), float(decay))
+        self.ema = {p: p.detach().clone() for group in self.param_groups for p in group["params"] if p.requires_grad}
+        if self._flat is not None:
+            self.attach_flat(self._flat["plan"])
 
     def attach_flat(self, plan):
         """Use the train plan's flat parameter / gradient buffers: one kernel launch per step.  Existing per-parameter state
         (a loaded checkpoint, or steps already taken one by one) is COPIED into the flat moment buffers, so attaching before or
-        after ``load_state_dict`` keeps the optimizer state."""
+        after ``load_state_dict`` keeps the optimizer state.  The same holds for the EMA."""
         pflat = plan.flatten_parameters()
         m, v = torch.zeros_like(pflat), torch.zeros_like(pflat)
+        e = pflat.clone() if self.ema is not None else None
         step = 0
         for p in plan.param_order:
+            off = plan._goff[id(p)]
             st = self.state.get(p)
             if st:
-                off = plan._goff[id(p)]
                 m[off:off + p.numel()].copy_(st["exp_avg"].reshape(-1))
                 v[off:off + p.numel()].copy_(st["exp_avg_sq"].reshape(-1))
                 step = max(step, int(float(st["step"])))
-        self._flat = dict(plan=plan, p=pflat, m=m, v=v, step=step)
+            if e is not None and p in self.ema:
+                e[off:off + p.numel()].copy_(self.ema[p].reshape(-1))
+        self._flat = dict(plan=plan, p=pflat, m=m, v=v, ema=e, step=step)
         step_t = torch.tensor(float(step))
         for p in plan.param_order:
             off = plan._goff[id(p)]
@@ -98,6 +149,8 @@ class FusedAdam(torch.optim.Optimizer):
             st["step"] = step_t
             st["exp_avg"] = m[off:off + p.numel()].view(p.shape)
             st["exp_avg_sq"] = v[off:off + p.numel()].view(p.shape)
+            if e is not None and p in self.ema:
+                self.ema[p] = e[off:off + p.numel()].view(p.shape)
 
     def load_state_dict(self, state_dict):
         """torch.optim.Optimizer.load_state_dict replaces the state tensors: the per-parameter ``step`` counters are moved back to
@@ -130,10 +183,7 @@ class FusedAdam(torch.optim.Optimizer):
             f, group = self._flat, self.param_groups[0]
             plan = f["plan"]
             f["step"] += 1
-            b1, b2 = group["betas"]
-            nat.call("wsr_adam_step", f["p"].data_ptr(), plan.gflat.data_ptr(), f["m"].data_ptr(), f["v"].data_ptr(), f["p"].numel(),
-                     float(group["lr"]), float(b1), float(b2), float(group["eps"]), float(group["weight_decay"]), int(f["step"]),
-                     torch.cuda.current_stream(f["p"].device).cuda_stream)
+            self._launch(f["p"], plan.gflat, f["m"], f["v"], f["ema"], f["step"], group)
             step_t = torch.tensor(float(f["step"]))
             for p in plan.param_order:
                 self.state[p]["step"] = step_t
@@ -150,7 +200,6 @@ class FusedAdam(torch.optim.Optimizer):
         return loss
 
     def _step_each(self, params, group):
-        b1, b2 = group["betas"]
         for p in params:
             if p.grad is None:
                 continue
@@ -163,6 +212,18 @@ class FusedAdam(torch.optim.Optimizer):
                 st["exp_avg"] = torch.zeros_like(p, memory_format=torch.preserve_format)
                 st["exp_avg_sq"] = torch.zeros_like(p, memory_format=torch.preserve_format)
             st["step"] = st["step"] + 1
-            nat.call("wsr_adam_step", p.data_ptr(), g.data_ptr(), st["exp_avg"].data_ptr(), st["exp_avg_sq"].data_ptr(), p.numel(),
-                     float(group["lr"]), float(b1), float(b2), float(group["eps"]), float(group["weight_decay"]),
-                     int(st["step"].item()), torch.cuda.current_stream(p.device).cuda_stream)
+            self._launch(p, g, st["exp_avg"], st["exp_avg_sq"], None if self.ema is None else self.ema.get(p),
+                         int(st["step"].item()), group)
+
+    def _launch(self, p, g, m, v, ema, step, group):
+        """One Adam update; with EMA, the fused variant on the steps where the schedule writes the EMA (d = 0 copies)."""
+        b1, b2 = group["betas"]
+        args = (float(group["lr"]), float(b1), float(b2), float(group["eps"]), float(group["weight_decay"]), int(step))
+        stream = torch.cuda.current_stream(p.device).cuda_stream
+        action = "skip" if ema is None else ema_action(step, *self.ema_schedule[:2])
+        if action == "skip":
+            nat.call("wsr_adam_step", p.data_ptr(), g.data_ptr(), m.data_ptr(), v.data_ptr(), p.numel(), *args, stream)
+        else:
+            decay = 0.0 if action == "copy" else self.ema_schedule[2]
+            nat.call("wsr_adam_step_ema", p.data_ptr(), g.data_ptr(), m.data_ptr(), v.data_ptr(), ema.data_ptr(), p.numel(), *args,
+                     decay, stream)

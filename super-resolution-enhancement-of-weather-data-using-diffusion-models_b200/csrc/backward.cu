@@ -574,19 +574,26 @@ __global__ void __launch_bounds__(256) fd_gate_bwd_kernel(const void* dxin, int 
 
 // ------------------------------------------------------------------------------------------------------------------
 // Adam (torch.optim.Adam semantics, models/diffusion_models/model.py:43-44: lr, betas (0.9, 0.999), eps 1e-8, wd 0)
+// With EMA the updated parameter, still in a register, also moves the exponential moving average:
+// ema = ema * d + (1 - d) * p_new as three separately rounded fp32 operations (torch's expression with a Python-float d;
+// __fmul_rn / __fadd_rn keep the compiler from contracting them into an FMA), or ema = p_new exactly when d == 0.
 // ------------------------------------------------------------------------------------------------------------------
+template <bool EMA>
 __global__ void adam_step_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m, float* __restrict__ v,
                                  int64_t n, float lr, float b1, float b2, float omb1, float omb2, float eps, float wd, float bc1,
-                                 float bc2_sqrt) {
+                                 float bc2_sqrt, float* __restrict__ ema, float ema_d, float ema_omd) {
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
     float gi = g[i];
     const float pi = p[i];
+    const float ei = EMA ? ema[i] : 0.f;             // issued with the other loads, not after the stores
     if (wd != 0.f) gi = fmaf(wd, pi, gi);
     const float mi = b1 * m[i] + omb1 * gi;          // 1 - beta rounded from double, as torch does
     const float vi = b2 * v[i] + omb2 * gi * gi;
     m[i] = mi; v[i] = vi;
     const float denom = sqrtf(vi) / bc2_sqrt + eps;
-    p[i] = pi - (lr / bc1) * (mi / denom);
+    const float pn = pi - (lr / bc1) * (mi / denom);
+    p[i] = pn;
+    if constexpr (EMA) ema[i] = ema_d == 0.f ? pn : __fadd_rn(__fmul_rn(ei, ema_d), __fmul_rn(ema_omd, pn));
   }
 }
 
@@ -774,9 +781,30 @@ extern "C" int wsr_adam_step(float* p, const float* g, float* m, float* v, int64
   const double bc2 = 1.0 - pow(beta2, (double)step);
   unsigned blocks = (unsigned)((n + 255) / 256);
   if (blocks > 2368) blocks = 2368;
-  adam_step_kernel<<<blocks, 256, 0, (cudaStream_t)stream>>>(p, g, m, v, n, (float)lr, (float)beta1, (float)beta2, (float)(1.0 - beta1),
-                                                             (float)(1.0 - beta2), (float)eps, (float)weight_decay, (float)bc1,
-                                                             (float)sqrt(bc2));
+  adam_step_kernel<false><<<blocks, 256, 0, (cudaStream_t)stream>>>(p, g, m, v, n, (float)lr, (float)beta1, (float)beta2,
+                                                                    (float)(1.0 - beta1), (float)(1.0 - beta2), (float)eps,
+                                                                    (float)weight_decay, (float)bc1, (float)sqrt(bc2), nullptr, 0.f,
+                                                                    0.f);
+  WSR_LAUNCH_OK();
+  return WSR_OK;
+}
+
+static bool ranges_overlap(const float* a, const float* b, int64_t n) { return a < b + n && b < a + n; }
+
+extern "C" int wsr_adam_step_ema(float* p, const float* g, float* m, float* v, float* ema, int64_t n, double lr, double beta1,
+                                 double beta2, double eps, double weight_decay, int step, double ema_decay, void* stream) {
+  WSR_REQUIRE(p && g && m && v && ema && n > 0 && step > 0, WSR_E_INVALID, "adam_step_ema: bad argument");
+  WSR_REQUIRE(ema_decay >= 0.0 && ema_decay < 1.0, WSR_E_INVALID, "adam_step_ema: ema_decay %g outside [0, 1)", ema_decay);
+  WSR_REQUIRE(!ranges_overlap(ema, p, n) && !ranges_overlap(ema, g, n) && !ranges_overlap(ema, m, n) && !ranges_overlap(ema, v, n),
+              WSR_E_INVALID, "adam_step_ema: ema overlaps p, g, m or v");
+  const double bc1 = 1.0 - pow(beta1, (double)step);
+  const double bc2 = 1.0 - pow(beta2, (double)step);
+  unsigned blocks = (unsigned)((n + 255) / 256);
+  if (blocks > 2368) blocks = 2368;
+  adam_step_kernel<true><<<blocks, 256, 0, (cudaStream_t)stream>>>(p, g, m, v, n, (float)lr, (float)beta1, (float)beta2,
+                                                                   (float)(1.0 - beta1), (float)(1.0 - beta2), (float)eps,
+                                                                   (float)weight_decay, (float)bc1, (float)sqrt(bc2), ema,
+                                                                   (float)ema_decay, (float)(1.0 - ema_decay));
   WSR_LAUNCH_OK();
   return WSR_OK;
 }

@@ -1,5 +1,7 @@
 """DDPM facade -- drop-in for the reference's models/diffusion_models/model.py:13-252 (same methods, same checkpoint
-file names and contents: ``I{iter}_E{epoch}_gen.pth`` = netG.state_dict() on CPU, ``..._opt.pth`` = optimizer state)."""
+file names and contents: ``I{iter}_E{epoch}_gen.pth`` = netG.state_dict() on CPU, ``..._opt.pth`` = optimizer state).
+With ``enable_ema`` a third file, ``..._ema.pth``, holds the same state_dict with the stepped parameters replaced by their EMA."""
+import contextlib
 import logging
 import os
 from collections import OrderedDict
@@ -170,14 +172,19 @@ class DDPM(BaseModel):
         state = {k: v.cpu() for k, v in self._net().state_dict().items()}
         torch.save(state, gen_path)
         torch.save({'epoch': epoch, 'iter': iter_step, 'scheduler': None, 'optimizer': self.optG.state_dict()}, opt_path)
+        if self.optG.ema is not None:
+            ema_path = os.path.join(self.opt['path']['checkpoint'], 'I{}_E{}_ema.pth'.format(iter_step, epoch))
+            torch.save(self.ema_state_dict(), ema_path)
         logger.info('Saved model in [{:s}] ...'.format(gen_path))
 
-    def load_network(self):
-        load_path = self.opt['path']['resume_state']
+    def load_network(self, load_path=None, weights='gen'):
+        """Load ``{load_path}_{weights}.pth`` (default: ``path.resume_state`` and the gen file; ``weights='ema'`` reads the EMA
+        file, which has the gen file's keys and shapes) and, in the train phase, the optimizer state."""
+        load_path = load_path or self.opt['path']['resume_state']
         if load_path is None:
             return
-        logger.info('Loading pretrained model for G [{:s}] ...'.format(load_path))
-        self._net().load_state_dict(torch.load('{}_gen.pth'.format(load_path), map_location=self.device),
+        logger.info('Loading pretrained model for G [{:s}_{:s}.pth] ...'.format(load_path, weights))
+        self._net().load_state_dict(torch.load('{}_{}.pth'.format(load_path, weights), map_location=self.device),
                                     strict=(not self.opt['model']['finetune_norm']))
         if self.opt['phase'] == 'train':
             # optimizer state: moments go to the device with load_state_dict; the per-parameter step counters stay on the host
@@ -185,6 +192,76 @@ class DDPM(BaseModel):
             self.optG.load_state_dict(o['optimizer'])
             self.begin_step = o['iter']
             self.begin_epoch = o['epoch']
+
+    def enable_ema(self, schedule):
+        """Keep an EMA of the parameters the optimizer steps, ``schedule`` = (step_start_ema, update_ema_every, ema_decay)
+        (autograd_glue.ema_action).  It starts from the current weights; when resuming, from ``{resume_state}_ema.pth`` if
+        that file exists."""
+        self.optG.enable_ema(schedule)
+        load_path = self.opt['path']['resume_state']
+        if load_path is None:
+            return
+        ema_path = '{}_ema.pth'.format(load_path)
+        if not os.path.exists(ema_path):
+            logger.info('No EMA weights at [{:s}]: the EMA starts from the loaded weights'.format(ema_path))
+            return
+        state = torch.load(ema_path, map_location=self.device)
+        expect = self._net().state_dict()
+        if set(state) != set(expect) or any(state[k].shape != expect[k].shape for k in expect):
+            raise RuntimeError('{:s} does not match the keys and shapes of the model'.format(ema_path))
+        with torch.no_grad():
+            for name, p in self._net().named_parameters(remove_duplicate=False):
+                if p in self.optG.ema:
+                    self.optG.ema[p].copy_(state[name])
+        logger.info('Loaded EMA weights [{:s}] ...'.format(ema_path))
+
+    def ema_state_dict(self):
+        """netG.state_dict() on CPU with every parameter the optimizer steps replaced by its EMA (frozen parameters and
+        buffers as they are): loads with ``load_state_dict(strict=True)`` wherever the gen file does."""
+        state = {k: v.cpu() for k, v in self._net().state_dict().items()}
+        for name, p in self._net().named_parameters(remove_duplicate=False):
+            if p in self.optG.ema:
+                state[name] = self.optG.ema[p].detach().cpu().clone()
+        return state
+
+    @contextlib.contextmanager
+    def ema_weights(self):
+        """Run the body with the EMA values in the live parameters, then put the trained values back bit for bit.  The flat
+        parameter buffer of the train plan is swapped as one block, the other stepped parameters (a jointly trained encoder)
+        one by one with an in-place copy that bumps their ``_version``, which is what the encoder plan's packs are keyed on;
+        the only temporary is one copy of the swapped parameters.  ``weights_epoch`` is bumped both ways so that the packed
+        bf16 weights of the denoiser plans are rebuilt from the values in place.
+
+        For validation and sampling only: a training forward (``DenoiseFn``) inside the block raises.  The train plan runs
+        ``set_levels`` / ``set_condition`` before its weight refresh, so they use the level projections and condition weights
+        of the PREVIOUS refresh; a training forward on the EMA would leave the first training forward after the swap back on
+        EMA-derived state."""
+        from ... import autograd_glue
+        opt = self.optG
+        if opt.ema is None:
+            raise RuntimeError('ema_weights() needs enable_ema()')
+        if autograd_glue.weights_swapped:
+            raise RuntimeError('ema_weights() does not nest')
+        pairs, in_flat = [], set()
+        f = opt._flat
+        if f is not None and f['ema'] is not None and f['plan'].parameters_are_flat():
+            pairs.append((f['p'], f['ema']))
+            in_flat = {id(p) for p in f['plan'].param_order}
+        pairs += [(p, e) for p, e in opt.ema.items() if id(p) not in in_flat]
+        with torch.no_grad():
+            saved = [live.clone() for live, _ in pairs]
+            for live, e in pairs:
+                live.copy_(e)
+        autograd_glue.weights_epoch += 1
+        autograd_glue.weights_swapped = True
+        try:
+            yield
+        finally:
+            with torch.no_grad():
+                for (live, _), s in zip(pairs, saved):
+                    live.copy_(s)
+            autograd_glue.weights_epoch += 1
+            autograd_glue.weights_swapped = False
 
     def prepare_to_train(self) -> None:
         self.set_new_noise_schedule(self.opt['model']['beta_schedule']['train'], schedule_phase='train')

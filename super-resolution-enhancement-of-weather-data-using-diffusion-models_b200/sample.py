@@ -17,7 +17,10 @@ sharded (rank r runs a contiguous member range) and rank 0 gathers them; the con
 Philox seed (member m uses member_key(S, m); member 0 is the plain run with seed S).
 
 ``--sampler {ddpm,ddim,dpmpp2m} --steps S --eta E`` selects the reverse loop (GaussianDiffusion.set_sampler): the reference's DDPM over
-all T steps (default), DDIM(eta) or DPM-Solver++(2M) over S of the T trained timesteps.  It applies to plain, sharded and ensemble runs."""
+all T steps (default), DDIM(eta) or DPM-Solver++(2M) over S of the T trained timesteps.  It applies to plain, sharded and ensemble runs.
+
+``--ema`` samples from the EMA weights ``{MODEL_PATH}_ema.pth`` written by ``train.py --ema`` instead of ``{MODEL_PATH}_gen.pth``; it needs
+``-p`` and combines with every other option, since it only changes the weights."""
 import argparse
 import os
 import sys
@@ -46,7 +49,11 @@ def parse_args(argv=None):
                     help="reverse-loop sampler (default ddpm: every timestep of the schedule)")
     ap.add_argument("--steps", type=int, default=None, help="network calls of a ddim / dpmpp2m loop (default: every timestep)")
     ap.add_argument("--eta", type=float, default=None, help="DDIM noise scale (default 0: deterministic; 1: respaced ancestral)")
-    return ap.parse_args(argv)
+    ap.add_argument("--ema", action="store_true", help="load MODEL_PATH_ema.pth (EMA weights) instead of MODEL_PATH_gen.pth")
+    args = ap.parse_args(argv)
+    if args.ema and not args.model_path:
+        ap.error("--ema needs -p MODEL_PATH")
+    return args
 
 
 def sampler_options(args):
@@ -71,13 +78,19 @@ def main(argv=None):
         torch.distributed.init_process_group("nccl")
     opt = Config(args, experiment=False).params
     opt["phase"] = "val"
-    if args.model_path:
+    if args.ema:
+        if not os.path.exists(args.model_path + "_ema.pth"):
+            raise SystemExit("sample.py --ema: no EMA weights at %s_ema.pth" % args.model_path)
+        opt["path"]["resume_state"] = None                 # the EMA file is loaded in place of the gen file
+    elif args.model_path:
         opt["path"]["resume_state"] = args.model_path
     elif opt["path"].get("resume_state") and not os.path.exists(str(opt["path"]["resume_state"]) + "_gen.pth"):
         opt["path"]["resume_state"] = None                # config points at the authors' machine: random-init weights
     if opt["model"].get("pretrained_model", {}).get("model_path") and not os.path.exists(opt["model"]["pretrained_model"]["model_path"]):
         opt["model"]["pretrained_model"]["model_path"] = None
     model = create_model(opt, None)
+    if args.ema:
+        model.load_network(args.model_path, weights="ema")
     model.prepare_to_eval()
     handler = None
     if data.is_store(str(opt["data"].get("dataroot", ""))):

@@ -3,7 +3,12 @@
 ``-p val`` runs the validation loop (generate_sr per batch, MSE / RMSE / MAE / MR on device accumulators) on the CUDA path.
 ``-p train`` builds the optimiser and runs ``optimize_parameters`` (forward, hand-written backward, fused Adam).  Under
 ``torchrun`` (one process per GPU) the batch is sharded across ranks and the gradients are all-reduced in buckets
-overlapped with the backward pass (parallel.FlatGradReducer); weights start identical on every rank (same seed)."""
+overlapped with the backward pass (parallel.FlatGradReducer); weights start identical on every rank (same seed).
+
+``--ema`` keeps an exponential moving average of the weights on the schedule of the config's ``train.ema_scheduler``
+(autograd_glue.ema_action), updated inside the Adam launch, saved as ``I{iter}_E{epoch}_ema.pth`` beside the gen / opt files at
+every checkpoint, and used for the in-loop validation.  ``-p val --ema`` validates ``{resume_state}_ema.pth`` instead of the gen
+file.  Every rank keeps its own EMA (the replicas are identical after the all-reduce); rank 0 writes the file."""
 import argparse
 import logging
 import os
@@ -21,6 +26,7 @@ def main(argv=None):
     ap.add_argument("-c", "--config", type=str, help="JSON file for configuration")
     ap.add_argument("-p", "--phase", type=str, choices=["train", "val"], default="train")
     ap.add_argument("-gpu", "--gpu_ids", type=str, default=None)
+    ap.add_argument("--ema", action="store_true", help="train / validate EMA weights (config train.ema_scheduler)")
     args = ap.parse_args(argv)
     logging.basicConfig(level=logging.INFO)
     log = logging.getLogger("base")
@@ -38,6 +44,17 @@ def main(argv=None):
         dist.init_process_group("nccl")
         args.gpu_ids = os.environ.get("LOCAL_RANK", "0")
     opt = Config(args, experiment=True).params
+    ema_schedule, ema_path = None, None
+    if args.ema and args.phase == "train":
+        try:
+            ema_schedule = wsr.sub("autograd_glue").check_ema_schedule(opt["train"].get("ema_scheduler"))
+        except ValueError as e:
+            raise SystemExit("train.py --ema: %s" % e)
+    if args.ema and args.phase == "val":
+        ema_path = opt["path"].get("resume_state")
+        if not ema_path or not os.path.exists(str(ema_path) + "_ema.pth"):
+            raise SystemExit("train.py -p val --ema: no EMA weights at %s_ema.pth (path.resume_state)" % ema_path)
+        opt["path"]["resume_state"] = None                 # the EMA file is loaded in place of the gen file
     for key in ("resume_state",):
         if opt["path"].get(key) and not os.path.exists(str(opt["path"][key]) + "_gen.pth"):
             opt["path"][key] = None
@@ -45,6 +62,10 @@ def main(argv=None):
     if pm.get("model_path") and not os.path.exists(pm["model_path"]):
         pm["model_path"] = None
     model = create_model(opt, None)
+    if ema_path is not None:
+        model.load_network(ema_path, weights="ema")
+    if ema_schedule is not None:
+        model.enable_ema(ema_schedule)
     if world > 1:
         # weights were initialised under seed 0 on every rank (identical replicas); from here on each rank must draw its OWN
         # timestep, noise levels, noise and dropout masks (the reference's single process draws them once for the whole batch)
@@ -78,7 +99,12 @@ def main(argv=None):
                 # train.py:79-117: the first validation batch only, the whole loader every full_val_freq iterations
                 model.prepare_to_eval()
                 full = bool(full_val_freq) and curr_iter % full_val_freq == 0
-                validate(model, opt, data, log, max_batches=None if full else 1)
+                if ema_schedule is None:
+                    validate(model, opt, data, log, max_batches=None if full else 1)
+                else:
+                    log.info("validation with the EMA weights")
+                    with model.ema_weights():
+                        validate(model, opt, data, log, max_batches=None if full else 1)
                 model.prepare_to_train()
             if curr_iter % opt["train"]["save_checkpoint_freq"] == 0 and rank == 0:
                 model.save_network(curr_epoch, curr_iter)
