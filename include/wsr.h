@@ -369,6 +369,16 @@ int wsr_error_sums(const float* pred, const float* target, int planes, int64_t h
  * below it -- members equal to the target count as not below.  scale folds the inverse StandardScaling in, as in wsr_error_sums. */
 int wsr_ensemble_stats(const float* ens, int N, int64_t member_stride, const float* target, int planes, int64_t hw, const float* scale,
                        float* mean, float* spread, double* acc, unsigned long long* rank_hist, void* stream);
+/* Zonal power spectra and row error sums (training.metrics.FieldScores).  pred, target: fp32 (planes, H, W), W along longitude
+ * (periodic).  Physical field x = scale[p] * in + shift[p] (scale NULL: 1, shift NULL: 0), error d = scale[p] * (pred - target).  Per
+ * (plane p, row r), with X_k = sum_n x_n exp(-2 pi i k n / W) and c_0 = c_{W/2} = 1, c_k = 2 otherwise, the one-sided power
+ * P_k = c_k |X_k|^2 / W^2, k = 0 .. W/2 (so sum_k P_k = mean_n x_n^2), is ADDED (doubles) to acc[(p*H + r)*S + j], S = 3*(W/2+1) + 3:
+ *   j = k: P of pred      j = (W/2+1) + k: P of target      j = 2*(W/2+1) + k: P of d      j = 3*(W/2+1) + {0,1,2}: sum |d|, sum d^2, sum d
+ * A NULL target touches only the pred slots.  Direct DFT in double; one CTA per (plane, row), no atomics (repeated calls are
+ * bit-identical).  Nothing is written, and WSR_E_INVALID / WSR_E_UNSUPPORTED returned, for a NULL pred or acc, planes or H below 1,
+ * or W odd, below 4 or above 2048. */
+int wsr_zonal_spectra(const float* pred, const float* target, int planes, int H, int W, const float* scale, const float* shift, double* acc,
+                      void* stream);
 
 /* Prior pre-training (SURVEY.md 8f N4).  image_compare_loss of models/simple_cnn/loss.py:60-76: alpha * fft_mse_loss +
  * beta * dwt_mse_loss (4 Haar levels) between x and y, fp32 NCHW planes with H, W multiples of 16.  *loss += value (double);

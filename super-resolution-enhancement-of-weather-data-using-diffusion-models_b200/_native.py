@@ -133,6 +133,7 @@ SIGNATURES = {
     "wsr_standard_scale": [_P, _I, _L, _P, _P, _I, _P, _P],
     "wsr_error_sums": [_P, _P, _I, _L, _P, _P, _P],
     "wsr_ensemble_stats": [_P, _I, _L, _P, _I, _L, _P, _P, _P, _P, _P, _P],
+    "wsr_zonal_spectra": [_P, _P, _I, _I, _I, _P, _P, _P, _P],
     "wsr_image_compare_loss": [_P, _P, _I, _I, _I, _F, _F, _P, _P, _P],
     "wsr_relu_mask": [_P, _P, _L, _P],
     "wsr_lrelu_mask": [_P, _I, _I, _P, _I, _I, _L, _I, _F, _P],

@@ -14,7 +14,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 PKG = os.path.dirname(HERE)
 OUT_DIR = os.path.join(PKG, "_lib")
 LIB = os.path.join(OUT_DIR, "libwsr.so")
-SOURCES = ["common.cu", "elementwise.cu", "simt.cu", "fd.cu", "gemm_tc.cu", "attn_tc.cu", "attn_small_tc.cu", "head.cu", "backward.cu", "wgrad_tc.cu", "edge.cu", "pretrain.cu", "ensemble.cu"]
+SOURCES = ["common.cu", "elementwise.cu", "simt.cu", "fd.cu", "gemm_tc.cu", "attn_tc.cu", "attn_small_tc.cu", "head.cu", "backward.cu", "wgrad_tc.cu", "edge.cu", "pretrain.cu", "ensemble.cu", "spectra.cu"]
 HEADERS = ["common.cuh", "tc_common.cuh", "philox.cuh", os.path.join("..", "..", "include", "wsr.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "--use_fast_math",
               "-Xcompiler", "-fPIC"]

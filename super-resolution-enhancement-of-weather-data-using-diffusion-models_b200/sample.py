@@ -19,6 +19,11 @@ Philox seed (member m uses member_key(S, m); member 0 is the plain run with seed
 ``--sampler {ddpm,ddim,dpmpp2m} --steps S --eta E`` selects the reverse loop (GaussianDiffusion.set_sampler): the reference's DDPM over
 all T steps (default), DDIM(eta) or DPM-Solver++(2M) over S of the T trained timesteps.  It applies to plain, sharded and ensemble runs.
 
+``--scores`` writes ``scores.json`` beside ``sr.npy`` (training.metrics.FieldScores against the batch's HR: zonal power spectra per
+latitude band, cos(latitude)-weighted and unweighted errors; physical units with a store): sections ``model`` and ``bicubic`` (the
+condition ``SR``, the reference's INTERPOLATED), or with ``--ensemble`` ``members`` (all N x B member fields), ``ensemble_mean`` and
+``bicubic``.  It is computed on rank 0 after the gather; a batch without HR is an error.
+
 ``--ema`` samples from the EMA weights ``{MODEL_PATH}_ema.pth`` written by ``train.py --ema`` instead of ``{MODEL_PATH}_gen.pth``; it needs
 ``-p`` and combines with every other option, since it only changes the weights."""
 import argparse
@@ -50,6 +55,7 @@ def parse_args(argv=None):
     ap.add_argument("--steps", type=int, default=None, help="network calls of a ddim / dpmpp2m loop (default: every timestep)")
     ap.add_argument("--eta", type=float, default=None, help="DDIM noise scale (default 0: deterministic; 1: respaced ancestral)")
     ap.add_argument("--ema", action="store_true", help="load MODEL_PATH_ema.pth (EMA weights) instead of MODEL_PATH_gen.pth")
+    ap.add_argument("--scores", action="store_true", help="write scores.json: spectra and latitude-weighted errors against HR")
     args = ap.parse_args(argv)
     if args.ema and not args.model_path:
         ap.error("--ema needs -p MODEL_PATH")
@@ -107,6 +113,8 @@ def main(argv=None):
         batch, months = handler.get_data_by_date(args.date)
     else:
         batch, months = next(iter(data.batches_from_opt(opt, "val")))
+    if args.scores and not (isinstance(batch, dict) and batch.get("HR") is not None):
+        raise SystemExit("sample.py --scores: the batch carries no HR field to score against")
     if args.seed is not None:
         model._net().sample_seed = args.seed
     opts = sampler_options(args)
@@ -116,11 +124,12 @@ def main(argv=None):
         except ValueError as e:
             raise SystemExit("sample.py: %s" % e)
     if args.ensemble is not None:
-        _ensemble(args, model, batch, months, handler, par, rank, world)
+        _ensemble(args, opt, model, batch, months, handler, par, rank, world)
         if world > 1:
             torch.distributed.destroy_process_group()
         return
     n_total = batch["SR"].shape[0]
+    full = batch
     if world > 1:
         batch = par.shard_batch(batch, rank, world)
     model.feed_data((batch, months))
@@ -135,11 +144,13 @@ def main(argv=None):
         if handler is not None:
             phys = handler.get_data_transformer().inverse_transform({"SR": sr}, months[:sr.shape[0]] if len(months) >= sr.shape[0] else months)
             np.save(os.path.join(args.output_path, "sr_physical.npy"), phys["SR"].float().cpu().numpy())
+        if args.scores:
+            _field_scores(args, opt, full, months, handler, {"model": [sr]})
     if world > 1:
         torch.distributed.destroy_process_group()
 
 
-def _ensemble(args, model, batch, months, handler, par, rank, world):
+def _ensemble(args, opt, model, batch, months, handler, par, rank, world):
     n = int(args.ensemble)
     if n < 1:
         raise SystemExit("--ensemble needs at least one member")
@@ -151,6 +162,7 @@ def _ensemble(args, model, batch, months, handler, par, rank, world):
         ens = par.gather_batch(ens, n)
     if rank != 0:
         return
+    model_ens = ens                                        # standardised units (ens becomes physical below with a store)
     import json
     out = args.output_path
     os.makedirs(out, exist_ok=True)
@@ -170,11 +182,36 @@ def _ensemble(args, model, batch, months, handler, par, rank, world):
     for name, a in arrays.items():
         np.save(os.path.join(out, name + ".npy"), a.float().cpu().numpy())
     print("saved %s %s" % (os.path.join(out, "ensemble.npy"), tuple(arrays["ensemble"].shape)))
+    if args.scores:
+        _field_scores(args, opt, batch, months, handler, {"members": list(model_ens), "ensemble_mean": [model_ens.mean(0)]})
     if target is not None and n > 1:
         scores = wsr.sub("training.metrics").EnsembleScores(ens.device)
         scores.update(ens, target)
         with open(os.path.join(out, "ensemble_scores.json"), "w") as fh:
             json.dump(scores.compute(), fh, indent=1)
+
+
+def _field_scores(args, opt, batch, months, handler, outputs):
+    """scores.json in the output directory: one FieldScores per entry of ``outputs`` (name -> list of (B, C, H, W) standardised fields,
+    each scored against the batch's HR), plus the bicubic condition; physical units with a store."""
+    metrics = wsr.sub("training.metrics")
+    hr = batch["HR"]
+    B, C, H, W = hr.shape
+    mean = std = None
+    if handler is not None:
+        mean, std = handler.get_data_transformer().batch_statistics("hr", months[:B] if len(months) >= B else months)
+    d = opt["data"]
+    lat, lat_source = metrics.field_latitudes(d.get("dataroot"), (d.get("variables") or [None])[0], H)
+    lr_width = batch["LR"].shape[-1] if batch.get("LR") is not None else None
+    dev = outputs[next(iter(outputs))][0].device
+    sections = {}
+    for name, fields in list(outputs.items()) + [("bicubic", [batch["SR"]])]:
+        sections[name] = metrics.FieldScores(dev, lat, lr_width)
+        for f in fields:
+            sections[name].update(f, hr, std, mean)
+    path = os.path.join(args.output_path, "scores.json")
+    metrics.write_field_scores(path, sections, "physical" if handler is not None else "standardised", lat_source, d.get("variables"))
+    print("saved %s" % path)
 
 
 if __name__ == "__main__":

@@ -8,7 +8,13 @@ overlapped with the backward pass (parallel.FlatGradReducer); weights start iden
 ``--ema`` keeps an exponential moving average of the weights on the schedule of the config's ``train.ema_scheduler``
 (autograd_glue.ema_action), updated inside the Adam launch, saved as ``I{iter}_E{epoch}_ema.pth`` beside the gen / opt files at
 every checkpoint, and used for the in-loop validation.  ``-p val --ema`` validates ``{resume_state}_ema.pth`` instead of the gen
-file.  Every rank keeps its own EMA (the replicas are identical after the all-reduce); rank 0 writes the file."""
+file.  Every rank keeps its own EMA (the replicas are identical after the all-reduce); rank 0 writes the file.
+
+``-p val --scores FILE`` also scores the whole validation loader with training.metrics.FieldScores (zonal power spectra per latitude
+band, cos(latitude)-weighted and unweighted errors) for the model output and, as the baseline, the bicubic condition ``SR``, both
+against HR, and writes them to FILE as JSON (sections ``model`` and ``bicubic``).  With a store the scores are in physical units (the
+fitted mean and std of each sample's month); otherwise they are in standardised units (``units`` says which).  Under torchrun rank 0
+writes the file."""
 import argparse
 import logging
 import os
@@ -21,13 +27,22 @@ sys.path.insert(0, os.path.dirname(_HERE))
 import wsr  # noqa: E402
 
 
-def main(argv=None):
+def parse_args(argv=None):
     ap = argparse.ArgumentParser()
     ap.add_argument("-c", "--config", type=str, help="JSON file for configuration")
     ap.add_argument("-p", "--phase", type=str, choices=["train", "val"], default="train")
     ap.add_argument("-gpu", "--gpu_ids", type=str, default=None)
     ap.add_argument("--ema", action="store_true", help="train / validate EMA weights (config train.ema_scheduler)")
+    ap.add_argument("--scores", type=str, default=None, metavar="FILE",
+                    help="-p val: write spectral and latitude-weighted scores of the model and the bicubic baseline to FILE (JSON)")
     args = ap.parse_args(argv)
+    if args.scores and args.phase != "val":
+        ap.error("--scores needs -p val")
+    return args
+
+
+def main(argv=None):
+    args = parse_args(argv)
     logging.basicConfig(level=logging.INFO)
     log = logging.getLogger("base")
 
@@ -71,7 +86,7 @@ def main(argv=None):
         # timestep, noise levels, noise and dropout masks (the reference's single process draws them once for the whole batch)
         random.seed(rank); np.random.seed(rank); torch.manual_seed(rank); torch.cuda.manual_seed(rank)
     if args.phase == "val":
-        return validate(model, opt, data, log)
+        return validate(model, opt, data, log, scores_path=args.scores)
     # reference train.py:55-123: resume from the loaded iteration / epoch, stop at n_iter, validate every val_freq iterations,
     # checkpoints named by the REAL epoch and iteration
     curr_iter, curr_epoch = int(model.get_loaded_iter() or 0), int(model.get_loaded_epoch() or 0)
@@ -114,16 +129,18 @@ def main(argv=None):
     return curr_iter, curr_epoch
 
 
-def validate(model, opt, data, log, max_batches=None):
+def validate(model, opt, data, log, max_batches=None, scores_path=None):
     """reference train.py:132-196 (validate): generate_sr per batch, inverse transform, metric accumulators -- here the
     accumulators live on the device (training/metrics.py) and the inverse StandardScaling is folded into the same pass
-    as a per-(sample, variable) scale, so nothing is copied to the host until the final compute."""
+    as a per-(sample, variable) scale, so nothing is copied to the host until the final compute.  ``scores_path``: also
+    accumulate FieldScores of the model output and of the bicubic condition and write them there (rank 0)."""
     model.prepare_to_eval()
     metrics = wsr.sub("training.metrics")
     vm = metrics.ValidationMetrics(metrics.create_metric_dict(model.device))
     vm_k = metrics.ValidationMetrics(metrics.create_metric_dict(model.device))
     sigma_k = float(opt["data"].get("sigma_kelvin", 21.26))          # WeatherBench t2m std (synthetic data has no fitted transform)
     handler = data.store_handler(opt)                                # the reference's on-disk store, when dataroot is one
+    fields, lat_source = None, None
     for i, (batch, months) in enumerate(data.batches_from_opt(opt, "val")):
         if max_batches is not None and i >= max_batches:
             break
@@ -131,18 +148,31 @@ def validate(model, opt, data, log, max_batches=None):
         model.generate_sr(False)
         sr, hr = model.SR, model.data["HR"]
         vm.update(sr, hr)
+        mean = std = None
         if handler is not None:
             # physical units = fitted std of each sample's month and variable (train.py:96-99 inverse_transform, folded in)
-            _, std = handler.get_data_transformer().batch_statistics("hr", months)
+            mean, std = handler.get_data_transformer().batch_statistics("hr", months)
             vm_k.update(sr, hr, scale=std.reshape(-1))
         else:
             vm_k.update(sr, hr, scale=torch.full((sr.shape[0] * sr.shape[1],), sigma_k))
+        if scores_path:
+            if fields is None:
+                variable = (opt["data"].get("variables") or [None])[0]
+                lat, lat_source = metrics.field_latitudes(opt["data"].get("dataroot"), variable, hr.shape[2])
+                lr_width = model.data["LR"].shape[-1] if "LR" in model.data else None
+                fields = {name: metrics.FieldScores(model.device, lat, lr_width) for name in ("model", "bicubic")}
+            fields["model"].update(sr, hr, std, mean)
+            fields["bicubic"].update(model.data["SR"], hr, std, mean)      # the bicubic condition (the reference's INTERPOLATED)
     vm.compute_metrics(); vm_k.compute_metrics()
     log.info("validation (standardised units)%s", vm.metrics2str())
     if handler is not None:
         log.info("validation (physical units, fitted statistics)%s", vm_k.metrics2str())
     else:
         log.info("validation (x sigma = %.2f K)%s", sigma_k, vm_k.metrics2str())
+    if fields is not None and int(os.environ.get("RANK", "0")) == 0:
+        metrics.write_field_scores(scores_path, fields, "physical" if handler is not None else "standardised", lat_source,
+                                   opt["data"].get("variables"))
+        log.info("spectral and latitude-weighted scores written to %s", scores_path)
     return vm.metrics2dict(), vm_k.metrics2dict()
 
 
